@@ -13,7 +13,7 @@ One "step" = one pass of the hot path over the whole batch.  Printed JSON line:
   roofline  the dominant kernel (count_kernel) against the measured HBM copy peak
   cpu_baseline  the oracle port timed on this box's host cores on a bounded sample
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 """
 import argparse
 import json
@@ -50,7 +50,15 @@ def parse_args():
                     help="also time the other BASELINE configs (c3, c4_strong, c5_sparse: bench_extras.py)")
     ap.add_argument("--extra-scale", type=float, default=1.0, help="shrink the extras' genomes (debug only)")
     ap.add_argument("--c5-single", action="store_true", help="run c5_sparse on one GPU too (> 100 GB of workspace)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned (rank 0's genomes) to DIR/<name>.npy: a fixed sample "
+                         "of the count and frequency rows, and the window totals")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl ours)")
+    return args
 
 
 # ------------------------------------------------------------------ workload
@@ -83,6 +91,49 @@ def make_genome_gpu(i, scale, device, torch):
             parts.append(seq[full:])
             parts.append(nl)
     return torch.cat(parts), sum(lens)
+
+
+# ------------------------------------------------------------------ --dump-outputs
+DUMP_BINS_PER_K = 4096
+DUMP_BUDGET_BYTES = 48 << 20          # what --dump-outputs writes stays below 64 MB
+
+
+def dump_selection(n_gen, ks):
+    """(genome rows, row columns) that --dump-outputs writes: every bin of a level with at most 4096 bins and a seeded
+    sample of 4096 bins of each larger one, for every genome unless that would exceed the budget (then a seeded
+    sample of the genomes).  It depends on the arguments only, so two builds write the same entries."""
+    from kmerml_b200 import engine
+    lay, _ = engine.row_layout(ks)
+    cols = []
+    for k, (off, n) in lay.items():
+        if n <= DUMP_BINS_PER_K:
+            cols.append(np.arange(off, off + n))
+        else:
+            cols.append(off + np.sort(np.random.default_rng(k).choice(n, DUMP_BINS_PER_K, replace=False)))
+    cols = np.concatenate(cols)
+    per_genome = cols.size * (8 + 4) + len(ks) * 8           # float64 counts, float32 frequencies, float64 totals
+    n_rows = max(1, min(n_gen, DUMP_BUDGET_BYTES // per_genome))
+    if n_rows == n_gen:
+        return np.arange(n_gen), cols
+    return np.sort(np.random.default_rng(n_gen).choice(n_gen, n_rows, replace=False)), cols
+
+
+def dump_sample(counts, freq, totals, ks, torch):
+    """The selected entries of the count rows (uint32 as float64), frequency rows (float32) and window totals
+    (float64), copied to host numpy arrays."""
+    rows, cols = dump_selection(counts.shape[0], ks)
+    r = torch.from_numpy(rows).to(counts.device)
+    c = torch.from_numpy(cols).to(counts.device)
+    pick = lambda t: t.index_select(1, c).index_select(0, r)      # columns first: never copies whole rows
+    return {"counts": (pick(counts).to(torch.int64) & 0xFFFFFFFF).cpu().numpy().astype(np.float64),
+            "freq": pick(freq).cpu().numpy().astype(np.float32),
+            "totals": totals.index_select(0, r).cpu().numpy().astype(np.float64)}
+
+
+def write_dump(out_dir, arrays):
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
 
 
 class ClockSampler:
@@ -330,6 +381,7 @@ def run_ours(args):
     e1.record()
     barrier()
     t1 = time.time()
+    dumped = dump_sample(counts, freq, totals, ks, torch) if args.dump_outputs and rank == 0 else None
     ms = e0.elapsed_time(e1)
     step_ms = sorted(marks[i].elapsed_time(marks[i + 1]) for i in range(args.steps))
     prof = ctx.profile_read(reset=True)
@@ -487,7 +539,7 @@ def run_ours(args):
             hf = freq[:n_e2e]          # the feature matrix stays resident in HBM (what the ML stage consumes)
             ht = torch.zeros((n_e2e, len(ks)), dtype=torch.int64, pin_memory=True)
             torch.cuda.synchronize()
-            n_e2e_steps = max(1, min(args.steps, 2))
+            n_e2e_steps = args.steps
 
             def timed(fn):
                 fn()                                              # warm-up (allocates the slots)
@@ -568,6 +620,8 @@ def run_ours(args):
             "gpu_launches": int(prof["launches"]), "clocks": clocks, "parity": parity,
         }
         line.update(extras)
+        if dumped:
+            write_dump(args.dump_outputs, dumped)
         print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()

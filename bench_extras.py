@@ -254,7 +254,7 @@ def run_c4(torch, dist, device, rank, world, steps, warmup, scale=1.0):
     # single-GPU result of the whole genome on this rank: timed (the strong-scaling reference) and compared
     def single():
         return engine.count_dense_device(fasta, [0, int(fasta.numel())], [k], canonical=True, want_freq=False)
-    ms1, whole = T.timed(single, max(1, min(steps, 2)), 1)
+    ms1, whole = T.timed(single, steps, 1)
     n = part.numel()
     same = bool(torch.equal(part, whole.counts[0, off:off + n])) and int(totals[0]) == int(whole.totals[0, 0])
     slice_sum = T.sum_over_ranks(float((part.to(torch.int64) & 0xFFFFFFFF).sum().item()))
@@ -337,7 +337,7 @@ def run_extras(args, torch, dist, device, rank, world):
     out = {}
     t0 = time.time()
     sc = args.extra_scale
-    steps = max(1, min(args.steps, 3))
+    steps = args.steps
     try:
         out["c3"] = run_c3(torch, dist, device, rank, world, steps, 1, n_genomes=max(8, int(1000 * min(sc, 1.0))), mbp=5.0)
     except Exception as exc:                                              # report, never fake
@@ -362,7 +362,7 @@ def run_extras(args, torch, dist, device, rank, world):
                                            f"{3.1 * sc / world:.2f} G windows); {float(free.item()) / 1e9:.0f} GB free: run with more GPUs"}
         else:
             try:
-                out["c5_sparse"] = run_c5(torch, dist, device, rank, world, max(1, min(steps, 2)), 1, scale=sc)
+                out["c5_sparse"] = run_c5(torch, dist, device, rank, world, steps, 1, scale=sc)
             except Exception as exc:
                 out["c5_sparse"] = {"error": repr(exc)[:300]}
         torch.cuda.empty_cache()

@@ -1,8 +1,9 @@
-import sys, json, base64, ctypes, random
+import os, sys, json, base64, ctypes, random
 import numpy as np
-sys.path.insert(0,'/root/repo')
+HERE = os.path.dirname(os.path.abspath(__file__))
+sys.path.insert(0, os.path.dirname(os.path.dirname(HERE)))
 import oracle
-L = ctypes.CDLL('/root/repo/tests/emu/libemu_dense.so')
+L = ctypes.CDLL(os.path.join(HERE, 'libemu_dense.so'))
 L.emu_count_dense.restype = ctypes.c_int64
 L.emu_count_dense.argtypes = [ctypes.c_void_p, ctypes.c_uint64, ctypes.c_uint64, ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_void_p, ctypes.c_void_p]
 
@@ -28,7 +29,7 @@ def check(data, kmax, min_rec, tpt, tps, base_off, tag):
     return ok
 
 rng = random.Random(7)
-cases = json.load(open('/root/repo/tests/golden/extract_cases.json'))
+cases = json.load(open(os.path.join(os.path.dirname(HERE), 'golden', 'extract_cases.json')))
 nbad = 0; n=0
 for c in cases:
     data = base64.b64decode(c['fasta_b64'])

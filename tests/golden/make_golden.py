@@ -1,11 +1,11 @@
 #!/usr/bin/env python
 """Generate the golden fixtures in tests/golden/ by running the UNMODIFIED
-reference (/root/reference) under the Bio.SeqIO shim in tests/_ref.
+reference (a source tree of the original kmer-ml project, named by
+KMERML_REFERENCE) under the Bio.SeqIO shim in tests/_ref.
 
-Runs ONLY in the build container (the reference tree does not exist on the GPU
-box).  The fixtures it writes are committed; tests read only the fixtures.
+The fixtures it writes are committed; tests read only the fixtures.
 
-    python tests/golden/make_golden.py
+    KMERML_REFERENCE=<kmer-ml source tree> python tests/golden/make_golden.py
 
 Outputs
   extract_cases.json  - FASTA texts + KmerExtractor outputs (k{k}.txt lines in
@@ -37,7 +37,10 @@ from pathlib import Path
 
 HERE = Path(__file__).resolve().parent
 sys.path.insert(0, str(HERE.parent / "_ref"))      # the Bio shim
-sys.path.insert(1, "/root/reference")              # the unmodified reference
+REFERENCE = os.environ.get("KMERML_REFERENCE", "")
+if not (REFERENCE and os.path.isdir(os.path.join(REFERENCE, "kmerml"))):
+    sys.exit("set KMERML_REFERENCE to a source tree of the original kmer-ml project")
+sys.path.insert(1, REFERENCE)                      # the unmodified reference
 
 from kmerml.kmers.generate import KmerExtractor              # noqa: E402
 from kmerml.kmers.statistics import KmerFeatureExtractor     # noqa: E402

@@ -156,11 +156,15 @@ def test_fast_csv_writer_equals_pandas(tmp_path):
     assert st._fast_csv(only, None) == pd.concat(only, ignore_index=True).to_csv(index=False)
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/kmerml"), reason="the reference tree exists only in the build container")
+REFERENCE = os.environ.get("KMERML_REFERENCE", "")
+
+
+@pytest.mark.skipif(not (REFERENCE and os.path.isdir(os.path.join(REFERENCE, "kmerml"))),
+                    reason="set KMERML_REFERENCE to a source tree of the original kmer-ml project")
 def test_statistics_csv_against_the_live_reference(tmp_path):
-    """Build container only: the unmodified KmerFeatureExtractor (child process) and the drop-in write the feature
-    CSV for the same fresh random k-mer files; identical except for the last ulps of the entropy columns, which
-    the reference sums in set-iteration (hash) order."""
+    """Where a source tree of the original project is at hand (KMERML_REFERENCE): the unmodified KmerFeatureExtractor
+    (child process) and the drop-in write the feature CSV for the same fresh random k-mer files; identical except for
+    the last ulps of the entropy columns, which the reference sums in set-iteration (hash) order."""
     import random
     import subprocess
     import sys
@@ -182,7 +186,7 @@ def test_statistics_csv_against_the_live_reference(tmp_path):
         specs.append((i, fs, wrote))
     script = (
         "import sys, json, contextlib, io\n"
-        "sys.path.insert(0, '/root/reference')\n"
+        f"sys.path.insert(0, {REFERENCE!r})\n"
         "from kmerml.kmers.statistics import KmerFeatureExtractor\n"
         "root, spec = sys.argv[1], json.loads(sys.argv[2])\n"
         "for i, fs, _ in spec:\n"
