@@ -304,7 +304,8 @@ int kmerml_normalize_rows(kmerml_ctx *ctx, const uint32_t *d_counts, uint64_t co
  * Genome x genome distance matrix of the rows of X (n x m): metric 0 = cosine,
  * 1 = Euclidean.  dtype 0 = float32, 1 = uint32 (count rows: the Gram matrix is then
  * exact), 2 = float64.  Accumulation is float64 (the north star's 1e-6 relative
- * tolerance).  d_out32 / d_out64: n x n, either may be NULL.
+ * tolerance).  d_out32 / d_out64: n x n, either may be NULL.  uint32 rows with m a multiple of 64 go to the
+ * tensor cores, for m up to 65535 x 32768 features (every concatenated dense row fits; longer: KMERML_ERR_RANGE).
  */
 #define KMERML_METRIC_COSINE 0
 #define KMERML_METRIC_EUCLIDEAN 1
@@ -356,7 +357,8 @@ int kmerml_column_stats(kmerml_ctx *ctx, const void *d_x, int dtype, uint64_t st
  * GPU computes when the genomes were counted on several GPUs and the rows gathered (the reference has no
  * distance code; nearest hooks are the stubs kmerml/ml/clustering.py:6-16).  All n rows must be resident;
  * d_out32 / d_out64: (row_end - row_begin) x n.  The Gram entries are exact integers (tcgen05 kind::i8), so
- * the block is bit-identical to the same rows of kmerml_pairwise_distance.
+ * the block is bit-identical to the same rows of kmerml_pairwise_distance.  m up to 65535 x 32768 features, as there
+ * (longer: KMERML_ERR_RANGE).
  */
 int kmerml_pairwise_distance_rows(kmerml_ctx *ctx, const uint32_t *d_counts, uint64_t stride, int n,
                                   uint64_t m, int row_begin, int row_end, int metric, float *d_out32,

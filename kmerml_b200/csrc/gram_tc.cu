@@ -6,7 +6,8 @@
 //      G = C C^T,   C = sum_d 256^d D_d   (D_d = d-th byte of every count, uint8)
 // is computed EXACTLY as   G = sum_{a,b} 256^(a+b) D_a D_b^T   with
 //      tcgen05.mma.cta_group::1.kind::i8   (u8 x u8 -> s32 accumulators in TMEM),
-// at most 8192 features per accumulation (255*255*8192 < 2^31), then summed in int64.
+// at most 8192 features per accumulation (255*255*8192 < 2^31; rows longer than 65535 * 8192 take up to 32768, the
+// most that stays below 2^31), then summed in int64.
 //
 // One CTA (128 threads) owns a 128 x 128 tile of one (a, b) digit pair and one K split:
 //   global uint8 rows --16 B loads--> registers --> shared memory in the UMMA canonical K-major,
@@ -21,7 +22,18 @@ namespace km {
 
 constexpr int GT_M = 128, GT_N = 128, GT_KB = 64;       // tile and K block (bytes = uint8 elements)
 constexpr int GT_KSPLIT = 8192;                         // features per accumulation: 255^2 * 8192 < 2^31
+constexpr int GT_KSPLIT_MAX = 32768;                    // ... and the most it can be: 255^2 * 32768 < 2^31
+constexpr uint64_t GT_MAX_SPLITS = 65535;               // the K splits run along gridDim.z
 constexpr int GT_THREADS = 128;
+
+// The shortest K range per CTA (a multiple of GT_KB) that covers a row of m features in at most GT_MAX_SPLITS splits.
+static uint64_t min_ksplit(uint64_t m) { return ((m + GT_MAX_SPLITS - 1) / GT_MAX_SPLITS + GT_KB - 1) / GT_KB * GT_KB; }
+
+static int ksplit_out_of_range(uint64_t m) {
+    set_error("count rows of " + std::to_string(m) + " features are longer than the Gram kernel's grid covers (" +
+              std::to_string(GT_MAX_SPLITS * GT_KSPLIT_MAX) + ")");
+    return KMERML_ERR_RANGE;
+}
 
 // One CTA per count row: its four byte planes (128-bit loads, one packed 32-bit store per plane and four bins), its
 // exact squared norm (uint64, then double -- the Gram diagonal a row-block distance needs for ALL genomes) and the
@@ -107,7 +119,7 @@ __device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
 __global__ void __launch_bounds__(GT_THREADS)
 gram_i8_kernel(const uint8_t* __restrict__ A, const uint8_t* __restrict__ B, int n, uint64_t m, int symmetric_pair,
                unsigned long long scale, unsigned long long* __restrict__ G, int row_tile0, int rows_only,
-               uint32_t ksplit, int n_planes, uint64_t plane_stride) {
+               uint32_t ksplit, int n_planes, uint64_t plane_stride, uint32_t launch_pairs, uint32_t pair0) {
     // rows_only (multi-GPU row block): tile rows row_tile0 .. row_tile0 + gridDim.y - 1 against ALL columns, every
     // (a, b) digit pair launched separately, nothing mirrored: G holds rows [128 row_tile0, ...) only, at their
     // global row index.
@@ -120,11 +132,12 @@ gram_i8_kernel(const uint8_t* __restrict__ A, const uint8_t* __restrict__ B, int
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     const int row0 = (blockIdx.y + row_tile0) * GT_M, col0 = blockIdx.x * GT_N;
     if (!rows_only && symmetric_pair && col0 < row0) return;   // D_a D_a^T: the upper triangle is enough
-    // n_planes > 0: ONE launch for every (a, b) digit pair -- blockIdx.z = pair * splits + split, A / B = the plane base
+    // n_planes > 0: digit pairs pair0 .. pair0 + launch_pairs - 1 in one launch -- blockIdx.z = (pair - pair0) * splits
+    // + split, A / B = the plane base
     uint32_t zsplit = blockIdx.z;
     if (n_planes > 0) {
-        const uint32_t splits = gridDim.z / (uint32_t)(n_planes * n_planes);
-        const uint32_t pair = blockIdx.z / splits;
+        const uint32_t splits = gridDim.z / launch_pairs;
+        const uint32_t pair = pair0 + blockIdx.z / splits;
         zsplit = blockIdx.z % splits;
         const uint32_t a = pair / (uint32_t)n_planes, b = pair % (uint32_t)n_planes;
         if (8 * (a + b) >= 64) return;                      // a multiple of 2^64
@@ -261,6 +274,8 @@ size_t gram_tc_workspace(int n, uint64_t m) { return (size_t)4 * n * m + (size_t
 // Exact Gram matrix (as doubles, exact below 2^53) of uint32 count rows.  m must be a multiple of 64.
 int launch_gram_tc(const uint32_t* d_counts, uint64_t stride, int n, uint64_t m, void* workspace, double* d_gram,
                    cudaStream_t s) {
+    const uint64_t ksplit = std::max<uint64_t>(GT_KSPLIT, min_ksplit(m));
+    if (ksplit > (uint64_t)GT_KSPLIT_MAX) return ksplit_out_of_range(m);
     uint8_t* planes = (uint8_t*)workspace;
     const size_t plane = (size_t)n * m;
     unsigned long long* G = (unsigned long long*)(planes + ((4 * plane + 255) / 256) * 256);
@@ -272,13 +287,14 @@ int launch_gram_tc(const uint32_t* d_counts, uint64_t stride, int n, uint64_t m,
     KM_CUDA(cudaStreamSynchronize(s));
     int nd = h_max >= (1u << 24) ? 4 : h_max >= (1u << 16) ? 3 : h_max >= (1u << 8) ? 2 : 1;
     const unsigned tiles = (unsigned)((n + GT_M - 1) / GT_M);
-    const unsigned ksplits = (unsigned)((m + GT_KSPLIT - 1) / GT_KSPLIT);
+    const unsigned ksplits = (unsigned)((m + ksplit - 1) / ksplit);
     for (int a = 0; a < nd; a++) {
         for (int b = a; b < nd; b++) {
             if (8 * (a + b) >= 64) continue;                 // would not fit 64 bits anyway (counts^2 sums < 2^63 assumed)
             const unsigned long long scale = 1ull << (8 * (a + b));
             gram_i8_kernel<<<dim3(tiles, tiles, ksplits), GT_THREADS, 0, s>>>(planes + a * plane, planes + b * plane, n, m,
-                                                                             a == b ? 1 : 0, scale, G, 0, 0, GT_KSPLIT, 0, 0);
+                                                                             a == b ? 1 : 0, scale, G, 0, 0,
+                                                                             (uint32_t)ksplit, 0, 0, 0, 0);
             KM_CUDA(cudaGetLastError());
         }
     }
@@ -320,6 +336,7 @@ int launch_distance_rows_planes(const uint8_t* d_planes, uint64_t plane_stride, 
                                 const double* d_sumsq, int row_begin, int row_end, int metric, void* workspace,
                                 float* d_out32, double* d_out64, cudaStream_t s) {
     if (row_begin >= row_end) return KMERML_OK;
+    if (min_ksplit(m) > (uint64_t)GT_KSPLIT_MAX) return ksplit_out_of_range(m);
     unsigned long long* G = (unsigned long long*)workspace;
     const int t0 = row_begin / GT_M, t1 = (row_end + GT_M - 1) / GT_M;
     KM_CUDA(cudaMemsetAsync(G + (size_t)t0 * GT_M * n, 0, (size_t)(std::min(t1 * GT_M, n) - t0 * GT_M) * n * 8, s));
@@ -332,12 +349,17 @@ int launch_distance_rows_planes(const uint8_t* d_planes, uint64_t plane_stride, 
     const uint64_t base = (uint64_t)tiles * (unsigned)(t1 - t0) * pairs;
     uint64_t splits = std::max<uint64_t>((m + GT_KSPLIT - 1) / GT_KSPLIT, (want_ctas + base - 1) / base);
     splits = std::min<uint64_t>(splits, std::max<uint64_t>(m / 1024, 1));
-    uint32_t ksplit = (uint32_t)(((m + splits - 1) / splits + GT_KB - 1) / GT_KB * GT_KB);
-    if (ksplit > (uint32_t)GT_KSPLIT) ksplit = GT_KSPLIT;
+    uint64_t ksplit = ((m + splits - 1) / splits + GT_KB - 1) / GT_KB * GT_KB;
+    ksplit = std::max<uint64_t>(std::min<uint64_t>(ksplit, GT_KSPLIT), min_ksplit(m));
     const unsigned ksplits = (unsigned)((m + ksplit - 1) / ksplit);
-    gram_i8_kernel<<<dim3(tiles, (unsigned)(t1 - t0), ksplits * pairs), GT_THREADS, 0, s>>>(
-        d_planes, d_planes, n, m, 0, 1ull, G, t0, 1, ksplit, n_planes, plane_stride);
-    KM_CUDA(cudaGetLastError());
+    // all digit pairs in one launch while K splits x pairs fit gridDim.z; otherwise (rows of k = 13 and 14) one
+    // launch per pair
+    const unsigned pairs_per_launch = (uint64_t)ksplits * pairs <= GT_MAX_SPLITS ? pairs : 1;
+    for (unsigned p0 = 0; p0 < pairs; p0 += pairs_per_launch) {
+        gram_i8_kernel<<<dim3(tiles, (unsigned)(t1 - t0), ksplits * pairs_per_launch), GT_THREADS, 0, s>>>(
+            d_planes, d_planes, n, m, 0, 1ull, G, t0, 1, (uint32_t)ksplit, n_planes, plane_stride, pairs_per_launch, p0);
+        KM_CUDA(cudaGetLastError());
+    }
     const uint64_t cells = (uint64_t)(row_end - row_begin) * n;
     distance_rows_kernel<<<(unsigned)((cells + 255) / 256), 256, 0, s>>>(G, d_sumsq, n, row_begin, row_end, metric, d_out32, d_out64);
     KM_CUDA(cudaGetLastError());
