@@ -190,11 +190,6 @@ struct Prof {
     }
 };
 
-static bool flags_no_tc() {                    // KMERML_NO_TC=1: fp64 CUDA-core Gram kernel instead (debugging)
-    const char* e = getenv("KMERML_NO_TC");
-    return e && e[0] == '1';
-}
-
 static int build_row(const int* k_list, int nk, RowSpec* row, int* kmax, int* kmin) {
     if (!k_list || nk < 1 || nk > 14) return fail(KMERML_ERR_ARG, "k_list must hold 1..14 values");
     row->nk = nk;
@@ -1315,17 +1310,16 @@ int kmerml_pairwise_distance(kmerml_ctx* ctx, const void* d_x, int dtype, uint64
     if (!guard.ok) return fail(KMERML_ERR_CUDA, "cudaSetDevice failed");
     Workspace& ws = ctx->ws[0];
     if (int orc = order_stream(ctx, (cudaStream_t)stream)) return orc;
+    // uint32 count rows: exact integer Gram matrix on the tensor cores (tcgen05 kind::i8)
+    if (dtype == 1 && n > 0 && m >= 64 && m % 64 == 0) {
+        int rc = ws.part.ensure(distance_rows_workspace(n, m));
+        if (rc) return rc;
+        return launch_distance_rows_tc((const uint32_t*)d_x, stride, n, m, 0, n, metric, ws.part.p, d_out32, d_out64,
+                                       (cudaStream_t)stream);
+    }
     int rc = ws.misc.ensure(256 + (size_t)n * n * sizeof(double));
     if (rc) return rc;
     double* d_gram = (double*)((uint8_t*)ws.misc.p + 256);
-    // uint32 count rows: exact integer Gram matrix on the tensor cores (tcgen05 kind::i8)
-    if (dtype == 1 && n > 0 && m >= 64 && m % 64 == 0 && !(flags_no_tc())) {
-        rc = ws.part.ensure(gram_tc_workspace(n, m));
-        if (rc) return rc;
-        rc = launch_gram_tc((const uint32_t*)d_x, stride, n, m, ws.part.p, d_gram, (cudaStream_t)stream);
-        if (rc) return rc;
-        return launch_distance_from_gram(d_gram, n, metric, d_out32, d_out64, (cudaStream_t)stream);
-    }
     return launch_pairwise(d_x, dtype, stride, n, m, metric, d_gram, d_out32, d_out64, (cudaStream_t)stream);
 }
 
@@ -1341,7 +1335,7 @@ int kmerml_pairwise_distance_rows(kmerml_ctx* ctx, const uint32_t* d_counts, uin
     if (!guard.ok) return fail(KMERML_ERR_CUDA, "cudaSetDevice failed");
     Workspace& ws = ctx->ws[0];
     if (int orc = order_stream(ctx, (cudaStream_t)stream)) return orc;
-    int rc = ws.part.ensure(gram_rows_workspace(n, m));
+    int rc = ws.part.ensure(distance_rows_workspace(n, m));
     if (rc) return rc;
     return launch_distance_rows_tc(d_counts, stride, n, m, row_begin, row_end, metric, ws.part.p, d_out32, d_out64,
                                    (cudaStream_t)stream);
@@ -1374,7 +1368,7 @@ int kmerml_distance_rows_planes(kmerml_ctx* ctx, const uint8_t* d_planes, uint64
     if (!guard.ok) return fail(KMERML_ERR_CUDA, "cudaSetDevice failed");
     Workspace& ws = ctx->ws[0];
     if (int orc = order_stream(ctx, (cudaStream_t)stream)) return orc;
-    int rc = ws.part.ensure(distance_planes_workspace(n));
+    int rc = ws.part.ensure(distance_rows_workspace(n, 0));
     if (rc) return rc;
     ctx->launches += 2;
     return launch_distance_rows_planes(d_planes, plane_stride, n_planes, n, m, d_sumsq, row_begin, row_end, metric, ws.part.p,

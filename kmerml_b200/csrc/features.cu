@@ -261,32 +261,13 @@ gram_kernel(const T* __restrict__ X, uint64_t stride, int n, uint64_t m, double*
         }
 }
 
-// metric 0: cosine distance 1 - G_ij / sqrt(G_ii G_jj); 1: Euclidean sqrt(G_ii + G_jj - 2 G_ij)
 __global__ void distance_from_gram_kernel(const double* __restrict__ G, int n, int metric, float* D32, double* D64) {
     const uint64_t idx = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (idx >= (uint64_t)n * n) return;
     const int i = (int)(idx / n), j = (int)(idx % n);
-    const double gii = G[(uint64_t)i * n + i], gjj = G[(uint64_t)j * n + j], gij = G[idx];
-    double d;
-    if (i == j) {
-        d = 0.0;
-    } else if (metric == 0) {
-        const double den = sqrt(gii) * sqrt(gjj);
-        d = den > 0.0 ? 1.0 - gij / den : nan("");
-    } else {
-        const double d2 = gii + gjj - 2.0 * gij;
-        d = d2 > 0.0 ? sqrt(d2) : 0.0;
-    }
+    const double d = i == j ? 0.0 : gram_distance(G[(uint64_t)i * n + i], G[(uint64_t)j * n + j], G[idx], metric);
     if (D32) D32[idx] = (float)d;
     if (D64) D64[idx] = d;
-}
-
-int launch_distance_from_gram(const double* d_gram, int n, int metric, float* d_out32, double* d_out64, cudaStream_t s) {
-    const uint64_t nn = (uint64_t)n * n;
-    if (!nn) return KMERML_OK;
-    distance_from_gram_kernel<<<(unsigned)((nn + 255) / 256), 256, 0, s>>>(d_gram, n, metric, d_out32, d_out64);
-    KM_CUDA(cudaGetLastError());
-    return KMERML_OK;
 }
 
 int launch_pairwise(const void* d_x, int dtype, uint64_t stride, int n, uint64_t m, int metric, double* d_gram,

@@ -14,8 +14,13 @@
 //   no-swizzle core-matrix layout (8 rows x 16 B per core matrix) --> two MMAs (K = 32 each) per
 //   64-byte K block, issued by one thread, tracked by an mbarrier (tcgen05.commit); the next
 //   block's global loads are in flight while the tensor core works.  Epilogue: tcgen05.ld
-//   (32 lanes x 32 columns per warp) and int64 atomicAdd of scale * acc into G (and its transpose
-//   for a != b).
+//   (32 lanes x 32 columns per warp) and int64 atomicAdd of 256^(a+b) * acc into G.
+//
+// One launcher, launch_gram_planes, computes rows [row_begin, row_end) of G from the planes, all digit
+// pairs in one launch where gridDim.z allows; over all n rows it runs only the tiles on or above the
+// diagonal and mirrors each entry.  Every distance of count rows -- the whole matrix, a row block of
+// uint32 rows, a row block of gathered planes -- is that Gram, then distance_rows_kernel on G and the
+// exact squared norms.
 #include "internal.h"
 
 namespace km {
@@ -117,12 +122,12 @@ __device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
 }
 
 __global__ void __launch_bounds__(GT_THREADS)
-gram_i8_kernel(const uint8_t* __restrict__ A, const uint8_t* __restrict__ B, int n, uint64_t m, int symmetric_pair,
-               unsigned long long scale, unsigned long long* __restrict__ G, int row_tile0, int rows_only,
-               uint32_t ksplit, int n_planes, uint64_t plane_stride, uint32_t launch_pairs, uint32_t pair0) {
-    // rows_only (multi-GPU row block): tile rows row_tile0 .. row_tile0 + gridDim.y - 1 against ALL columns, every
-    // (a, b) digit pair launched separately, nothing mirrored: G holds rows [128 row_tile0, ...) only, at their
-    // global row index.
+gram_i8_kernel(const uint8_t* __restrict__ planes, uint64_t plane_stride, int n_planes, int n, uint64_t m,
+               int row_tile0, int symmetric, uint32_t ksplit, uint32_t launch_pairs, uint32_t pair0,
+               unsigned long long* __restrict__ G) {
+    // Row block (symmetric = 0): tile rows row_tile0 .. row_tile0 + gridDim.y - 1 against all columns, G holds those
+    // rows at their global row index.  Symmetric: every row, tiles on or above the diagonal only; entry (i, j >= i) is
+    // added at (i, j) and, for j != i, at (j, i).
     // shared: A tile and B tile in core-matrix layout: [kg (4)][mg (16)][8 rows][16 B]
     __shared__ __align__(128) uint8_t sA[GT_M * GT_KB];
     __shared__ __align__(128) uint8_t sB[GT_N * GT_KB];
@@ -131,21 +136,15 @@ gram_i8_kernel(const uint8_t* __restrict__ A, const uint8_t* __restrict__ B, int
 
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     const int row0 = (blockIdx.y + row_tile0) * GT_M, col0 = blockIdx.x * GT_N;
-    if (!rows_only && symmetric_pair && col0 < row0) return;   // D_a D_a^T: the upper triangle is enough
-    // n_planes > 0: digit pairs pair0 .. pair0 + launch_pairs - 1 in one launch -- blockIdx.z = (pair - pair0) * splits
-    // + split, A / B = the plane base
-    uint32_t zsplit = blockIdx.z;
-    if (n_planes > 0) {
-        const uint32_t splits = gridDim.z / launch_pairs;
-        const uint32_t pair = pair0 + blockIdx.z / splits;
-        zsplit = blockIdx.z % splits;
-        const uint32_t a = pair / (uint32_t)n_planes, b = pair % (uint32_t)n_planes;
-        if (8 * (a + b) >= 64) return;                      // a multiple of 2^64
-        A += (uint64_t)a * plane_stride;
-        B += (uint64_t)b * plane_stride;
-        scale = 1ull << (8 * (a + b));
-    }
-    const uint64_t k_begin = (uint64_t)zsplit * ksplit;
+    if (symmetric && col0 < row0) return;
+    // digit pairs pair0 .. pair0 + launch_pairs - 1 in one launch: blockIdx.z = (pair - pair0) * splits + split
+    const uint32_t splits = gridDim.z / launch_pairs;
+    const uint32_t pair = pair0 + blockIdx.z / splits;
+    const uint32_t a = pair / (uint32_t)n_planes, b = pair % (uint32_t)n_planes;
+    const uint8_t* A = planes + (uint64_t)a * plane_stride;
+    const uint8_t* B = planes + (uint64_t)b * plane_stride;
+    const unsigned long long scale = 1ull << (8 * (a + b));  // n_planes <= 4: at most 2^48
+    const uint64_t k_begin = (uint64_t)(blockIdx.z % splits) * ksplit;
     const uint64_t k_end = min(m, k_begin + ksplit);
     if (k_begin >= k_end) return;
 
@@ -170,16 +169,27 @@ gram_i8_kernel(const uint8_t* __restrict__ A, const uint8_t* __restrict__ B, int
     // a/b K-major = 0, n_dim = N >> 3 [17,23), m_dim = M >> 4 [24,29)
     const uint32_t idesc = (2u << 4) | ((uint32_t)(GT_N >> 3) << 17) | ((uint32_t)(GT_M >> 4) << 24);
 
-    // each thread moves 4 + 4 16-byte pieces per K block: piece q -> row q / 4, 16-byte column q % 4
+    // each thread moves 4 + 4 16-byte pieces per K block: piece q -> row q / 4, 16-byte column q % 4.  The source
+    // pointers advance by one K block per load: computed from row * m instead, ptxas re-derives every address from the
+    // kernel parameters in each block, which lengthens the loop by a half.
     uint4 ra[4], rb[4];
-    auto load_block = [&](uint64_t k0) {
+    const uint8_t* srcA[4];
+    const uint8_t* srcB[4];
+#pragma unroll
+    for (int i = 0; i < 4; i++) {
+        const int q = tid + GT_THREADS * i, r = q >> 2, p = q & 3;
+        srcA[i] = A + (uint64_t)(row0 + r) * m + k_begin + 16 * p;
+        srcB[i] = B + (uint64_t)(col0 + r) * m + k_begin + 16 * p;
+    }
+    auto load_block = [&](uint64_t k0) {                    // called for k0 = k_begin, k_begin + GT_KB, ...
 #pragma unroll
         for (int i = 0; i < 4; i++) {
             const int q = tid + GT_THREADS * i, r = q >> 2, p = q & 3;
-            const uint64_t kk = k0 + 16 * p;
-            const bool kin = kk < k_end;
-            ra[i] = (row0 + r < n && kin) ? *reinterpret_cast<const uint4*>(A + (uint64_t)(row0 + r) * m + kk) : make_uint4(0, 0, 0, 0);
-            rb[i] = (col0 + r < n && kin) ? *reinterpret_cast<const uint4*>(B + (uint64_t)(col0 + r) * m + kk) : make_uint4(0, 0, 0, 0);
+            const bool kin = k0 + 16 * p < k_end;
+            ra[i] = (row0 + r < n && kin) ? *reinterpret_cast<const uint4*>(srcA[i]) : make_uint4(0, 0, 0, 0);
+            rb[i] = (col0 + r < n && kin) ? *reinterpret_cast<const uint4*>(srcB[i]) : make_uint4(0, 0, 0, 0);
+            srcA[i] += GT_KB;
+            srcB[i] += GT_KB;
         }
     };
     auto store_block = [&]() {
@@ -244,18 +254,10 @@ gram_i8_kernel(const uint8_t* __restrict__ A, const uint8_t* __restrict__ B, int
 #pragma unroll
             for (int c = 0; c < 32; c++) {
                 const int gj = col0 + c0 + c;
-                if (gj >= n || !v[c]) continue;
+                if (gj >= n || !v[c] || (symmetric && gj < gi)) continue;
                 const unsigned long long add = (unsigned long long)v[c] * scale;
-                if (rows_only) {
-                    atomicAdd(G + (uint64_t)gi * n + gj, add);
-                } else if (symmetric_pair) {
-                    if (gj < gi) continue;                                    // upper triangle (tiles on the diagonal)
-                    atomicAdd(G + (uint64_t)gi * n + gj, add);
-                    if (gj != gi) atomicAdd(G + (uint64_t)gj * n + gi, add);
-                } else {                                                       // D_a D_b^T + (D_a D_b^T)^T
-                    atomicAdd(G + (uint64_t)gi * n + gj, add);
-                    atomicAdd(G + (uint64_t)gj * n + gi, add);
-                }
+                atomicAdd(G + (uint64_t)gi * n + gj, add);
+                if (symmetric && gj != gi) atomicAdd(G + (uint64_t)gj * n + gi, add);
             }
         }
     }
@@ -264,89 +266,25 @@ gram_i8_kernel(const uint8_t* __restrict__ A, const uint8_t* __restrict__ B, int
     if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, 128;" ::"r"(tmem_acc));
 }
 
-__global__ void gram_to_double_kernel(const unsigned long long* __restrict__ G, double* __restrict__ out, uint64_t nn) {
-    const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < nn) out[i] = (double)G[i];
-}
-
-size_t gram_tc_workspace(int n, uint64_t m) { return (size_t)4 * n * m + (size_t)n * n * 8 + 512; }
-
-// Exact Gram matrix (as doubles, exact below 2^53) of uint32 count rows.  m must be a multiple of 64.
-int launch_gram_tc(const uint32_t* d_counts, uint64_t stride, int n, uint64_t m, void* workspace, double* d_gram,
-                   cudaStream_t s) {
-    const uint64_t ksplit = std::max<uint64_t>(GT_KSPLIT, min_ksplit(m));
-    if (ksplit > (uint64_t)GT_KSPLIT_MAX) return ksplit_out_of_range(m);
-    uint8_t* planes = (uint8_t*)workspace;
-    const size_t plane = (size_t)n * m;
-    unsigned long long* G = (unsigned long long*)(planes + ((4 * plane + 255) / 256) * 256);
-    unsigned int* d_max = (unsigned int*)(G + (size_t)n * n);
-    KM_CUDA(cudaMemsetAsync(G, 0, (size_t)n * n * 8 + 8, s));
-    if (int rc = launch_count_planes(d_counts, stride, n, m, planes, plane, nullptr, d_max, s)) return rc;
-    unsigned int h_max = 0;
-    KM_CUDA(cudaMemcpyAsync(&h_max, d_max, 4, cudaMemcpyDeviceToHost, s));
-    KM_CUDA(cudaStreamSynchronize(s));
-    int nd = h_max >= (1u << 24) ? 4 : h_max >= (1u << 16) ? 3 : h_max >= (1u << 8) ? 2 : 1;
-    const unsigned tiles = (unsigned)((n + GT_M - 1) / GT_M);
-    const unsigned ksplits = (unsigned)((m + ksplit - 1) / ksplit);
-    for (int a = 0; a < nd; a++) {
-        for (int b = a; b < nd; b++) {
-            if (8 * (a + b) >= 64) continue;                 // would not fit 64 bits anyway (counts^2 sums < 2^63 assumed)
-            const unsigned long long scale = 1ull << (8 * (a + b));
-            gram_i8_kernel<<<dim3(tiles, tiles, ksplits), GT_THREADS, 0, s>>>(planes + a * plane, planes + b * plane, n, m,
-                                                                             a == b ? 1 : 0, scale, G, 0, 0,
-                                                                             (uint32_t)ksplit, 0, 0, 0, 0);
-            KM_CUDA(cudaGetLastError());
-        }
-    }
-    const uint64_t nn = (uint64_t)n * n;
-    gram_to_double_kernel<<<(unsigned)((nn + 255) / 256), 256, 0, s>>>(G, d_gram, nn);
-    KM_CUDA(cudaGetLastError());
-    return KMERML_OK;
-}
-
-// rows [row_begin, row_end) of the distance matrix from the row block of G and the squared norms of all rows
-__global__ void distance_rows_kernel(const unsigned long long* __restrict__ G, const double* __restrict__ norm2, int n,
-                                     int row_begin, int row_end, int metric, float* D32, double* D64) {
-    const uint64_t idx = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (idx >= (uint64_t)(row_end - row_begin) * n) return;
-    const int i = row_begin + (int)(idx / n), j = (int)(idx % n);
-    const double gii = norm2[i], gjj = norm2[j], gij = (double)G[(uint64_t)i * n + j];
-    double d;
-    if (i == j) {
-        d = 0.0;
-    } else if (metric == 0) {
-        const double den = sqrt(gii) * sqrt(gjj);
-        d = den > 0.0 ? 1.0 - gij / den : nan("");
-    } else {
-        const double d2 = gii + gjj - 2.0 * gij;
-        d = d2 > 0.0 ? sqrt(d2) : 0.0;
-    }
-    if (D32) D32[idx] = (float)d;
-    if (D64) D64[idx] = d;
-}
-
-
-// Rows [row_begin, row_end) of the n x n distance matrix from the byte planes of ALL n count rows (plane d at
-// d_planes + d * plane_stride, n x m bytes) and their squared norms: the unit one rank computes when the genomes were
-// counted on several GPUs (SURVEY 8e, C3).  The Gram entries are exact (tcgen05 kind::i8), so the block is
-// bit-identical to the same rows of the single-GPU matrix.  workspace: n * n * 8 bytes.
-size_t distance_planes_workspace(int n) { return (size_t)n * n * 8 + 256; }
-
-int launch_distance_rows_planes(const uint8_t* d_planes, uint64_t plane_stride, int n_planes, int n, uint64_t m,
-                                const double* d_sumsq, int row_begin, int row_end, int metric, void* workspace,
-                                float* d_out32, double* d_out64, cudaStream_t s) {
-    if (row_begin >= row_end) return KMERML_OK;
+// Rows [row_begin, row_end) of the exact Gram matrix G (n x n, uint64) of the count rows whose n_planes (1..4) byte
+// planes start at planes (plane d at planes + d * plane_stride, n x m bytes, m a multiple of 64).  G holds the rows of
+// the touched tiles, at their global row index.  Over all n rows the launch is symmetric: only tiles with col0 >= row0,
+// for all n_planes^2 ordered digit pairs -- the upper triangle of sum_{a,b} 256^(a+b) D_a D_b^T is that of G -- and
+// each entry (i, j > i) is mirrored to (j, i).
+int launch_gram_planes(const uint8_t* planes, uint64_t plane_stride, int n_planes, int n, uint64_t m, int row_begin,
+                       int row_end, unsigned long long* G, cudaStream_t s) {
     if (min_ksplit(m) > (uint64_t)GT_KSPLIT_MAX) return ksplit_out_of_range(m);
-    unsigned long long* G = (unsigned long long*)workspace;
+    const bool symmetric = row_begin == 0 && row_end == n;
     const int t0 = row_begin / GT_M, t1 = (row_end + GT_M - 1) / GT_M;
     KM_CUDA(cudaMemsetAsync(G + (size_t)t0 * GT_M * n, 0, (size_t)(std::min(t1 * GT_M, n) - t0 * GT_M) * n * 8, s));
-    // one launch for all digit pairs; the K range of a CTA shrinks (down to 1024 features) until the grid holds about
-    // four CTAs per SM: a row block of one rank of eight is 8 x 1 tiles, which at 8192 features per CTA and one
+    // the K range of a CTA shrinks (down to 1024 features) until the tiles that do work, over all digit pairs, make
+    // about four CTAs per SM: a row block of one rank of eight is 8 x 1 tiles, which at 8192 features per CTA and one
     // launch per pair left 64 CTAs at a time on 148 SMs
     const unsigned tiles = (unsigned)((n + GT_N - 1) / GT_N);
     const unsigned pairs = (unsigned)(n_planes * n_planes);
+    const uint64_t live_tiles = symmetric ? (uint64_t)tiles * (tiles + 1) / 2 : (uint64_t)tiles * (unsigned)(t1 - t0);
     const uint64_t want_ctas = 148ull * 4;
-    const uint64_t base = (uint64_t)tiles * (unsigned)(t1 - t0) * pairs;
+    const uint64_t base = live_tiles * pairs;
     uint64_t splits = std::max<uint64_t>((m + GT_KSPLIT - 1) / GT_KSPLIT, (want_ctas + base - 1) / base);
     splits = std::min<uint64_t>(splits, std::max<uint64_t>(m / 1024, 1));
     uint64_t ksplit = ((m + splits - 1) / splits + GT_KB - 1) / GT_KB * GT_KB;
@@ -357,9 +295,41 @@ int launch_distance_rows_planes(const uint8_t* d_planes, uint64_t plane_stride, 
     const unsigned pairs_per_launch = (uint64_t)ksplits * pairs <= GT_MAX_SPLITS ? pairs : 1;
     for (unsigned p0 = 0; p0 < pairs; p0 += pairs_per_launch) {
         gram_i8_kernel<<<dim3(tiles, (unsigned)(t1 - t0), ksplits * pairs_per_launch), GT_THREADS, 0, s>>>(
-            d_planes, d_planes, n, m, 0, 1ull, G, t0, 1, (uint32_t)ksplit, n_planes, plane_stride, pairs_per_launch, p0);
+            planes, plane_stride, n_planes, n, m, t0, symmetric ? 1 : 0, (uint32_t)ksplit, pairs_per_launch, p0, G);
         KM_CUDA(cudaGetLastError());
     }
+    return KMERML_OK;
+}
+
+// rows [row_begin, row_end) of the distance matrix from the row block of G and the squared norms of all rows
+__global__ void distance_rows_kernel(const unsigned long long* __restrict__ G, const double* __restrict__ norm2, int n,
+                                     int row_begin, int row_end, int metric, float* D32, double* D64) {
+    const uint64_t idx = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (idx >= (uint64_t)(row_end - row_begin) * n) return;
+    const int i = row_begin + (int)(idx / n), j = (int)(idx % n);
+    const double d = i == j ? 0.0 : gram_distance(norm2[i], norm2[j], (double)G[(uint64_t)i * n + j], metric);
+    if (D32) D32[idx] = (float)d;
+    if (D64) D64[idx] = d;
+}
+
+static size_t round256(size_t bytes) { return (bytes + 255) / 256 * 256; }
+
+// Workspace of the distance rows: the uint64 Gram matrix, then the squared norms, the largest count and the byte planes
+// of n uint32 count rows of m features (m = 0 when the caller brings planes and norms).
+size_t distance_rows_workspace(int n, uint64_t m) {
+    return round256((size_t)n * n * 8) + round256((size_t)n * 8 + 8) + (size_t)4 * n * m;
+}
+
+// Rows [row_begin, row_end) of the n x n distance matrix from the byte planes of ALL n count rows (plane d at
+// d_planes + d * plane_stride, n x m bytes) and their squared norms: also the unit one rank computes when the genomes
+// were counted on several GPUs (SURVEY 8e, C3).  The Gram entries are exact (tcgen05 kind::i8), so the block is
+// bit-identical to the same rows of the whole matrix.
+int launch_distance_rows_planes(const uint8_t* d_planes, uint64_t plane_stride, int n_planes, int n, uint64_t m,
+                                const double* d_sumsq, int row_begin, int row_end, int metric, void* workspace,
+                                float* d_out32, double* d_out64, cudaStream_t s) {
+    if (row_begin >= row_end) return KMERML_OK;
+    unsigned long long* G = (unsigned long long*)workspace;
+    if (int rc = launch_gram_planes(d_planes, plane_stride, n_planes, n, m, row_begin, row_end, G, s)) return rc;
     const uint64_t cells = (uint64_t)(row_end - row_begin) * n;
     distance_rows_kernel<<<(unsigned)((cells + 255) / 256), 256, 0, s>>>(G, d_sumsq, n, row_begin, row_end, metric, d_out32, d_out64);
     KM_CUDA(cudaGetLastError());
@@ -371,23 +341,20 @@ int planes_needed(unsigned int max_count) {
 }
 
 // The same from uint32 count rows resident on this GPU: planes + norms + largest count in one pass, then the above.
-size_t gram_rows_workspace(int n, uint64_t m) { return (size_t)4 * n * m + 256 + (size_t)n * 8 + 256 + distance_planes_workspace(n); }
-
 int launch_distance_rows_tc(const uint32_t* d_counts, uint64_t stride, int n, uint64_t m, int row_begin, int row_end,
                             int metric, void* workspace, float* d_out32, double* d_out64, cudaStream_t s) {
     if (row_begin >= row_end) return KMERML_OK;
-    uint8_t* planes = (uint8_t*)workspace;
-    const size_t plane = (size_t)n * m;
-    double* d_norm = (double*)(planes + (4 * plane + 255) / 256 * 256);
+    double* d_norm = (double*)((uint8_t*)workspace + round256((size_t)n * n * 8));
     unsigned int* d_max = (unsigned int*)(d_norm + n);
-    void* gws = (uint8_t*)d_norm + ((size_t)n * 8 + 8 + 255) / 256 * 256;
+    uint8_t* planes = (uint8_t*)d_norm + round256((size_t)n * 8 + 8);
+    const size_t plane = (size_t)n * m;
     KM_CUDA(cudaMemsetAsync(d_max, 0, 8, s));
     if (int rc = launch_count_planes(d_counts, stride, n, m, planes, plane, d_norm, d_max, s)) return rc;
     unsigned int h_max = 0;
     KM_CUDA(cudaMemcpyAsync(&h_max, d_max, 4, cudaMemcpyDeviceToHost, s));
     KM_CUDA(cudaStreamSynchronize(s));
-    return launch_distance_rows_planes(planes, plane, planes_needed(h_max), n, m, d_norm, row_begin, row_end, metric, gws,
-                                       d_out32, d_out64, s);
+    return launch_distance_rows_planes(planes, plane, planes_needed(h_max), n, m, d_norm, row_begin, row_end, metric,
+                                       workspace, d_out32, d_out64, s);
 }
 
 }  // namespace km

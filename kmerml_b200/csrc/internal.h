@@ -204,20 +204,31 @@ int launch_genome_stats(const uint8_t* d_fasta, uint64_t nbytes, unsigned long l
 int launch_static_features(int k, int compat, int32_t* d_out, cudaStream_t s);
 int launch_normalize_rows(const uint32_t* d_counts, uint64_t counts_stride, const uint64_t* d_totals, int n_rows,
                           uint64_t m, float* d_out, uint64_t out_stride, cudaStream_t s);
-size_t gram_tc_workspace(int n, uint64_t m);
-int launch_gram_tc(const uint32_t* d_counts, uint64_t stride, int n, uint64_t m, void* workspace, double* d_gram,
-                   cudaStream_t s);
+int launch_pairwise(const void* d_x, int dtype, uint64_t stride, int n, uint64_t m, int metric, double* d_gram,
+                    float* d_out32, double* d_out64, cudaStream_t s);
+
+// ---- distances of count rows from the exact tensor-core Gram (gram_tc.cu) ---------
 int launch_count_planes(const uint32_t* d_counts, uint64_t stride, int n, uint64_t m, uint8_t* d_planes,
                         uint64_t plane_stride, double* d_sumsq, unsigned int* d_max, cudaStream_t s);
-size_t distance_planes_workspace(int n);
+size_t distance_rows_workspace(int n, uint64_t m);
 int launch_distance_rows_planes(const uint8_t* d_planes, uint64_t plane_stride, int n_planes, int n, uint64_t m,
                                 const double* d_sumsq, int row_begin, int row_end, int metric, void* workspace,
                                 float* d_out32, double* d_out64, cudaStream_t s);
-size_t gram_rows_workspace(int n, uint64_t m);
 int launch_distance_rows_tc(const uint32_t* d_counts, uint64_t stride, int n, uint64_t m, int row_begin, int row_end,
                             int metric, void* workspace, float* d_out32, double* d_out64, cudaStream_t s);
-int launch_distance_from_gram(const double* d_gram, int n, int metric, float* d_out32, double* d_out64, cudaStream_t s);
-int launch_pairwise(const void* d_x, int dtype, uint64_t stride, int n, uint64_t m, int metric, double* d_gram,
-                    float* d_out32, double* d_out64, cudaStream_t s);
+
+#ifdef __CUDACC__
+// Distance of rows i != j from their Gram entries -- metric 0: cosine 1 - G_ij / sqrt(G_ii G_jj) (NaN when a row is
+// all zero); 1: Euclidean sqrt(G_ii + G_jj - 2 G_ij).  The one formula of distance_rows_kernel (exact Gram of count
+// rows) and distance_from_gram_kernel (fp64 Gram).
+__device__ __forceinline__ double gram_distance(double gii, double gjj, double gij, int metric) {
+    if (metric == 0) {
+        const double den = sqrt(gii) * sqrt(gjj);
+        return den > 0.0 ? 1.0 - gij / den : nan("");
+    }
+    const double d2 = gii + gjj - 2.0 * gij;
+    return d2 > 0.0 ? sqrt(d2) : 0.0;
+}
+#endif
 
 }  // namespace km

@@ -192,12 +192,12 @@ def test_sparse_counts_match_oracle():
 
 def test_tensor_core_gram_is_exact():
     """tcgen05 kind::i8 Gram of count rows (uint8 digit planes): distances equal the int64/float64
-    reference to the last bit of the final float64 arithmetic, also with 2- and 3-byte counts and ragged
+    reference to the last bit of the final float64 arithmetic, also with 2-, 3- and 4-byte counts and ragged
     n; the float64 CUDA-core path (float input) agrees within 1e-12."""
     import torch
     from kmerml_b200 import engine
     rng = np.random.default_rng(5)
-    for n, m, hi in ((3, 64, 255), (129, 1024, 256), (77, 4096, 70_000), (260, 16384, 1000)):
+    for n, m, hi in ((3, 64, 255), (129, 1024, 256), (77, 4096, 70_000), (260, 16384, 1000), (40, 256, 1 << 26)):
         c = rng.integers(0, hi, size=(n, m), dtype=np.int64)
         c[rng.integers(0, n)] = 0                                     # an all-zero row -> nan cosine distances
         x = torch.from_numpy(c.astype(np.uint32).view(np.int32)).cuda()
