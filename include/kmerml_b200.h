@@ -381,6 +381,38 @@ int kmerml_distance_rows_planes(kmerml_ctx *ctx, const uint8_t *d_planes, uint64
                                 float *d_out32, double *d_out64, void *stream);
 
 /*
+ * MinHash genome sketches and their Mash / Jaccard distances, for any k up to 32 (Ondov et al. 2016).
+ *
+ * kmerml_sketch_batch: the bottom-s sketch of every genome of a batch laid out as for kmerml_count_dense_batch
+ * (genome g = bytes [h_offsets[g], h_offsets[g + 1]) of d_fasta, 16-byte aligned).  k-mer keys and window rules are
+ * those of kmerml_count_sparse (KMERML_FLAG_CANONICAL: min(forward, reverse complement); min_record_len 0 means k).
+ * A key is hashed as h = fmix64(key + 0x9E3779B97F4A7C15 * (seed + 1)) mod 2^64 (fmix64: MurmurHash3's 64-bit
+ * finalizer), a bijection, so distinct hashes are distinct k-mers.  The sketch of genome g is the min(s, D) smallest
+ * distinct hashes of its k-mers (D = its distinct k-mers), ascending, in d_sketches[g * sketch_stride ..]; slots past
+ * d_filled[g] = min(s, D) hold UINT64_MAX.  These sketches are not file-compatible with Mash or sourmash.
+ * Every window is hashed once per round; only those below a per-genome threshold (~3 s of them) are stored.  A genome
+ * with fewer than s distinct hashes below its threshold, or whose stored windows overflowed their region (tandem
+ * repeats of a low-hash k-mer), is run again with a larger threshold or region, up to "keep every window".
+ * 1 <= s <= KMERML_SKETCH_MAX, sketch_stride >= s.  Synchronous.
+ *
+ * kmerml_sketch_distance_rows: rows [row_begin, row_end) x all n columns of the distance matrix of n sketches of
+ * kmerml_sketch_batch (same k, s, seed and canonical flag).  For sketches A and B: U = the min(s, |A u B|) smallest
+ * values of A u B, x = |U n A n B|, j = x / |U| (0 when |U| = 0); KMERML_SKETCH_METRIC_JACCARD gives 1 - j,
+ * KMERML_SKETCH_METRIC_MASH gives -ln(2j / (1 + j)) / k (1 when j = 0, 0 when j = 1).  Computed in float64;
+ * d_out32 / d_out64 ((row_end - row_begin) x n, either may be NULL) receive that value (rounded for float32).  The
+ * matrix is exactly symmetric, and a row block is bit-identical to the same rows of the whole matrix.
+ */
+#define KMERML_SKETCH_MAX 16384
+#define KMERML_SKETCH_METRIC_MASH 0
+#define KMERML_SKETCH_METRIC_JACCARD 1
+int kmerml_sketch_batch(kmerml_ctx *ctx, const uint8_t *d_fasta, const uint64_t *h_offsets, int n_genomes,
+                        int k, int min_record_len, unsigned flags, int sketch_size, uint64_t seed,
+                        uint64_t *d_sketches, uint64_t sketch_stride, uint32_t *d_filled, void *stream);
+int kmerml_sketch_distance_rows(kmerml_ctx *ctx, const uint64_t *d_sketches, uint64_t sketch_stride,
+                                const uint32_t *d_filled, int n, int sketch_size, int k, int row_begin, int row_end,
+                                int metric, float *d_out32, double *d_out64, void *stream);
+
+/*
  * Measurement hooks (bench.py): with profiling enabled every kernel the library
  * launches is bracketed by CUDA events on the launching stream.  kmerml_profile_read
  * synchronises those events and returns the accumulated device time per kernel family

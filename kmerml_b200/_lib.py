@@ -18,6 +18,9 @@ FLAG_WIDE_D2H = 16
 FLAG_NO_NIBBLES = 32
 MAX_DENSE_K = 14
 MAX_K = 32
+SKETCH_MAX = 16384
+SKETCH_METRIC_MASH = 0
+SKETCH_METRIC_JACCARD = 1
 
 _lib = None
 
@@ -91,6 +94,8 @@ def load():
     L.kmerml_pairwise_distance_rows.argtypes = [vp, vp, u64, i32, u64, i32, i32, i32, vp, vp, vp]
     L.kmerml_count_planes.argtypes = [vp, vp, u64, i32, u64, vp, u64, vp, vp, vp]
     L.kmerml_distance_rows_planes.argtypes = [vp, vp, u64, i32, i32, u64, vp, i32, i32, i32, vp, vp, vp]
+    L.kmerml_sketch_batch.argtypes = [vp, vp, vp, i32, i32, i32, u32, i32, u64, vp, u64, vp, vp]
+    L.kmerml_sketch_distance_rows.argtypes = [vp, vp, u64, vp, i32, i32, i32, i32, i32, i32, vp, vp, vp]
     L.kmerml_profile_enable.argtypes = [vp, i32]
     L.kmerml_profile_read.argtypes = [vp, ctypes.POINTER(Profile), i32]
     for name in EXPORTS:
@@ -113,6 +118,7 @@ EXPORTS = [
     "kmerml_compact_row_bytes", "kmerml_count_dense_host_compact", "kmerml_compact_expand", "kmerml_compact_row_overflowed", "kmerml_compact_row_used_bytes",
     "kmerml_parse_kmer_lines", "kmerml_feature_keys", "kmerml_feature_line_lengths", "kmerml_feature_write_lines",
     "kmerml_emit_sparse_range", "kmerml_reduce_sparse_windows",
+    "kmerml_sketch_batch", "kmerml_sketch_distance_rows",
 ]
 
 

@@ -12,7 +12,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libkmerml_b200.so")
-SOURCES = ["api.cu", "dense.cu", "features.cu", "sparse.cu", "gram_tc.cu", "format.cu", "hostpipe.cu", "stats.cu", "featcsv.cu"]
+SOURCES = ["api.cu", "dense.cu", "features.cu", "sparse.cu", "sketch.cu", "gram_tc.cu", "format.cu", "hostpipe.cu", "stats.cu", "featcsv.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",
     "-O3", "-std=c++17", "-lineinfo",

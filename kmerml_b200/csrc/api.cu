@@ -1526,6 +1526,195 @@ int kmerml_first_occurrence(kmerml_ctx* ctx, const uint8_t* d_fasta, uint64_t nb
     return launch_first_occurrence(d_fasta, d_genomes, d_slices, n_slices, k, min_rec, d_first, s);
 }
 
+// ---- MinHash sketches (sketch.cu) ----
+// First threshold of a genome: ~3 s windows hash below it (windows <= bytes); every window when that is all of them.
+static uint64_t sketch_first_tau(uint64_t bytes, int s) {
+    const unsigned __int128 want = (unsigned __int128)3 * (unsigned)s;
+    if (want >= bytes) return ~0ull;
+    return (uint64_t)((want << 64) / bytes);
+}
+
+// Region of a genome at threshold tau: twice the survivors expected, one slot per byte at most (>= its windows).
+static uint64_t sketch_region(uint64_t bytes, uint64_t tau) {
+    if (tau == ~0ull) return bytes;
+    const uint64_t expect = (uint64_t)(((unsigned __int128)bytes * tau) >> 64);
+    return std::min<uint64_t>(bytes, 2 * expect + 1024);
+}
+
+constexpr uint64_t SKETCH_ROUND_SLOTS = 1ull << 28;     // survivor slots of one round (2 GiB, twice: sort in / out)
+
+static int sketch_batch_core(kmerml_ctx* ctx, const uint8_t* d_fasta, const uint64_t* h_offsets, int n, int k, int min_rec,
+                             bool canonical, int sketch_size, uint64_t seed, uint64_t* d_sketches, uint64_t stride,
+                             uint32_t* d_filled, cudaStream_t s) {
+    Workspace& ws = ctx->ws[0];
+    const uint64_t sb = SPARSE_SLICE_BYTES;
+    auto slice_range = [&](int g, uint64_t* b0, uint64_t* b1) {
+        *b0 = h_offsets[g] / sb;
+        *b1 = (h_offsets[g + 1] - 1) / sb + 1;
+    };
+    uint64_t max_slices = 0;
+    for (int g = 0; g < n; g++) {
+        if (h_offsets[g + 1] == h_offsets[g]) continue;
+        uint64_t b0, b1;
+        slice_range(g, &b0, &b1);
+        max_slices += b1 - b0;
+    }
+    if (max_slices > 0x7fffffffull) return fail(KMERML_ERR_RANGE, "too many slices");
+    // tables: offsets | genomes | stats | sketch genomes | active | segments | status | slices
+    const size_t off_bytes = align_up((size_t)(n + 1) * 8, 256);
+    const size_t gen_bytes = align_up((size_t)n * sizeof(GenomeDev), 256);
+    const size_t st_bytes = align_up((size_t)n * sizeof(GenomeStats), 256);
+    const size_t sg_bytes = align_up((size_t)n * sizeof(SketchGenome), 256);
+    const size_t act_bytes = align_up((size_t)n * 4, 256);
+    const size_t seg_bytes = align_up((size_t)n * 8, 256);
+    const size_t sl_bytes = align_up((size_t)(max_slices + 1) * sizeof(Slice), 256);     // + 1 scratch entry
+    int rc = ws.tables.ensure(off_bytes + gen_bytes + st_bytes + sg_bytes + act_bytes + seg_bytes + act_bytes + sl_bytes);
+    if (rc) return rc;
+    rc = ws.staging.ensure(off_bytes + sg_bytes + act_bytes + act_bytes + sl_bytes);
+    if (rc) return rc;
+    if (!ws.staging_free) KM_CUDA(cudaEventCreateWithFlags(&ws.staging_free, cudaEventDisableTiming));
+    KM_CUDA(cudaEventSynchronize(ws.staging_free));     // previous call's upload has left the staging buffer
+    uint8_t* base = (uint8_t*)ws.tables.p;
+    uint64_t* d_offsets = (uint64_t*)base;
+    GenomeDev* d_genomes = (GenomeDev*)(base += off_bytes);
+    GenomeStats* d_stats = (GenomeStats*)(base += gen_bytes);
+    SketchGenome* d_sg = (SketchGenome*)(base += st_bytes);
+    int* d_active = (int*)(base += sg_bytes);
+    int* d_seg = (int*)(base += act_bytes);
+    uint32_t* d_status = (uint32_t*)(base += seg_bytes);
+    Slice* d_slices = (Slice*)(base += act_bytes);
+    uint8_t* hs = (uint8_t*)ws.staging.p;
+    SketchGenome* h_sg = (SketchGenome*)(hs + off_bytes);
+    int* h_active = (int*)(hs + off_bytes + sg_bytes);
+    uint32_t* h_status = (uint32_t*)(hs + off_bytes + sg_bytes + act_bytes);
+    Slice* h_slices = (Slice*)(hs + off_bytes + sg_bytes + 2 * act_bytes);
+    memcpy(hs, h_offsets, (size_t)(n + 1) * 8);
+    KM_CUDA(cudaMemcpyAsync(d_offsets, hs, off_bytes, cudaMemcpyHostToDevice, s));
+    if ((rc = launch_prologue(d_fasta, d_offsets, d_genomes, d_stats, n, s))) return rc;
+
+    std::vector<uint64_t> tau(n), cap(n);
+    std::vector<int> pending(n);
+    for (int g = 0; g < n; g++) {
+        const uint64_t bytes = h_offsets[g + 1] - h_offsets[g];
+        tau[g] = sketch_first_tau(bytes, sketch_size);
+        cap[g] = sketch_region(bytes, tau[g]);
+        pending[g] = g;
+    }
+    while (!pending.empty()) {
+        // one round: the pending genomes (in buffer order) whose regions fit SKETCH_ROUND_SLOTS, at least one
+        memset(h_sg, 0, (size_t)n * sizeof(SketchGenome));
+        int n_round = 0;
+        uint64_t slots = 0, n_slices = 0;
+        for (int g : pending) {
+            if (n_round && slots + cap[g] > SKETCH_ROUND_SLOTS) break;
+            if (slots + cap[g] > 0x7fffffffull)
+                return fail(KMERML_ERR_RANGE, "a genome's sketch region exceeds 2^31 slots");
+            h_sg[g].tau = tau[g];
+            h_sg[g].region = slots;
+            h_sg[g].cap = cap[g];
+            h_active[n_round++] = g;
+            slots += cap[g];
+            if (h_offsets[g + 1] == h_offsets[g]) continue;
+            uint64_t b0, b1;
+            slice_range(g, &b0, &b1);
+            for (uint64_t b = b0; b < b1; b++) {
+                Slice& sl = h_slices[n_slices++];
+                memset(&sl, 0, sizeof(Slice));
+                sl.genome = (uint32_t)g;
+                // skip the empty tiles before the genome's first byte
+                sl.begin = std::max<uint64_t>(b * sb, h_offsets[g] / SPARSE_TILE_BYTES * SPARSE_TILE_BYTES);
+                sl.end = (b + 1) * sb;
+            }
+        }
+        h_slices[n_slices].genome = 0;                      // scratch entry of launch_slice_headers
+        const size_t region_bytes = align_up(std::max<uint64_t>(slots, 1) * 8, 256);
+        const size_t temp_bytes = sketch_sort_temp_bytes((int)slots, n_round);
+        if ((rc = ws.part.ensure(2 * region_bytes + temp_bytes))) return rc;
+        uint64_t* d_regions = (uint64_t*)ws.part.p;
+        uint64_t* d_sorted = (uint64_t*)((uint8_t*)ws.part.p + region_bytes);
+        void* d_temp = (uint8_t*)ws.part.p + 2 * region_bytes;
+        KM_CUDA(cudaMemcpyAsync(d_sg, h_sg, (size_t)n * sizeof(SketchGenome), cudaMemcpyHostToDevice, s));
+        KM_CUDA(cudaMemcpyAsync(d_active, h_active, (size_t)n_round * 4, cudaMemcpyHostToDevice, s));
+        KM_CUDA(cudaMemcpyAsync(d_slices, h_slices, (size_t)(n_slices + 1) * sizeof(Slice), cudaMemcpyHostToDevice, s));
+        {
+            Prof pr(ctx, s, 3, 7);      // the three slice-table kernels, emit, segments, sort, select
+            rc = launch_slice_headers(d_fasta, d_genomes, d_slices, (int)n_slices, s);
+            if (!rc) rc = launch_sketch_emit(d_fasta, d_genomes, d_slices, (int)n_slices, k, min_rec, canonical, seed, d_sg,
+                                             d_regions, s);
+            if (!rc) rc = launch_sketch_select(d_sg, d_active, n_round, d_seg, (int)slots, d_regions, d_sorted, d_temp,
+                                               temp_bytes, sketch_size, d_sketches, stride, d_filled, d_status, s);
+        }
+        if (rc) return rc;
+        KM_CUDA(cudaMemcpyAsync(h_status, d_status, (size_t)n_round * 4, cudaMemcpyDeviceToHost, s));
+        KM_CUDA(cudaStreamSynchronize(s));
+        // run again: too few distinct hashes below tau -> 16 tau (saturating at every window); overflow -> one slot
+        // per byte.  Every window with one slot per byte cannot fail, so the loop ends.
+        std::vector<int> next;
+        for (int i = 0; i < n_round; i++) {
+            const int g = h_active[i];
+            const uint64_t bytes = h_offsets[g + 1] - h_offsets[g];
+            if (h_status[i] == SKETCH_MORE) {
+                tau[g] = tau[g] > ~0ull / 16 ? ~0ull : tau[g] * 16;
+                cap[g] = sketch_region(bytes, tau[g]);
+            } else if (h_status[i] == SKETCH_OVERFLOW) {
+                cap[g] = bytes;
+            } else {
+                continue;
+            }
+            next.push_back(g);
+        }
+        next.insert(next.end(), pending.begin() + n_round, pending.end());
+        std::sort(next.begin(), next.end());            // the slice table stays in buffer order
+        pending.swap(next);
+    }
+    KM_CUDA(cudaEventRecord(ws.staging_free, s));
+    return KMERML_OK;
+}
+
+int kmerml_sketch_batch(kmerml_ctx* ctx, const uint8_t* d_fasta, const uint64_t* h_offsets, int n_genomes, int k,
+                        int min_record_len, unsigned flags, int sketch_size, uint64_t seed, uint64_t* d_sketches,
+                        uint64_t sketch_stride, uint32_t* d_filled, void* stream) {
+    if (!ctx) return fail(KMERML_ERR_ARG, "ctx is null");
+    if (k < 1 || k > KMERML_MAX_K) return fail(KMERML_ERR_ARG, "k must be in 1..32");
+    if (sketch_size < 1 || sketch_size > KMERML_SKETCH_MAX)
+        return fail(KMERML_ERR_ARG, "sketch_size must be in 1.." + std::to_string(KMERML_SKETCH_MAX));
+    if (sketch_stride < (uint64_t)sketch_size) return fail(KMERML_ERR_ARG, "sketch_stride must be >= sketch_size");
+    if (n_genomes < 0) return fail(KMERML_ERR_ARG, "n_genomes < 0");
+    const int min_rec = min_record_len > 0 ? min_record_len : k;
+    if (min_rec < k) return fail(KMERML_ERR_ARG, "min_record_len must be >= k");
+    if (n_genomes == 0) return KMERML_OK;
+    if (!h_offsets || !d_sketches || !d_filled) return fail(KMERML_ERR_ARG, "null pointer argument");
+    if (!d_fasta && h_offsets[n_genomes] > h_offsets[0]) return fail(KMERML_ERR_ARG, "d_fasta is null");
+    if ((uintptr_t)d_fasta & 15) return fail(KMERML_ERR_ARG, "device pointers must be 16-byte aligned");
+    for (int g = 0; g < n_genomes; g++)
+        if (h_offsets[g + 1] < h_offsets[g]) return fail(KMERML_ERR_ARG, "offsets must be non-decreasing");
+    DeviceGuard guard(ctx->device);
+    if (!guard.ok) return fail(KMERML_ERR_CUDA, "cudaSetDevice failed");
+    if (int orc = order_stream(ctx, (cudaStream_t)stream)) return orc;
+    return sketch_batch_core(ctx, d_fasta, h_offsets, n_genomes, k, min_rec, (flags & KMERML_FLAG_CANONICAL) != 0,
+                             sketch_size, seed, d_sketches, sketch_stride, d_filled, (cudaStream_t)stream);
+}
+
+int kmerml_sketch_distance_rows(kmerml_ctx* ctx, const uint64_t* d_sketches, uint64_t sketch_stride, const uint32_t* d_filled,
+                                int n, int sketch_size, int k, int row_begin, int row_end, int metric, float* d_out32,
+                                double* d_out64, void* stream) {
+    if (!ctx) return fail(KMERML_ERR_ARG, "ctx is null");
+    if (k < 1 || k > KMERML_MAX_K) return fail(KMERML_ERR_ARG, "k must be in 1..32");
+    if (sketch_size < 1 || sketch_size > KMERML_SKETCH_MAX)
+        return fail(KMERML_ERR_ARG, "sketch_size must be in 1.." + std::to_string(KMERML_SKETCH_MAX));
+    if (sketch_stride < (uint64_t)sketch_size) return fail(KMERML_ERR_ARG, "sketch_stride must be >= sketch_size");
+    if (metric != KMERML_SKETCH_METRIC_MASH && metric != KMERML_SKETCH_METRIC_JACCARD)
+        return fail(KMERML_ERR_ARG, "unknown sketch metric");
+    if (n < 0 || row_begin < 0 || row_end > n || row_begin > row_end) return fail(KMERML_ERR_ARG, "bad row range");
+    if (row_begin == row_end) return KMERML_OK;
+    if (!d_sketches || !d_filled || (!d_out32 && !d_out64)) return fail(KMERML_ERR_ARG, "null pointer argument");
+    DeviceGuard guard(ctx->device);
+    if (!guard.ok) return fail(KMERML_ERR_CUDA, "cudaSetDevice failed");
+    ctx->launches += 1;
+    return launch_sketch_distance(d_sketches, sketch_stride, d_filled, n, sketch_size, k, row_begin, row_end, metric,
+                                  d_out32, d_out64, (cudaStream_t)stream);
+}
+
 // NCCL through the process that called us (no link-time dependency): the four entry points the exchange needs.
 namespace {
 struct NcclApi {

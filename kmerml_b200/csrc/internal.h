@@ -187,6 +187,27 @@ int run_merge_sparse(void* workspace, int k, const uint64_t* d_keys, const uint3
                      uint64_t n, uint64_t* d_keys_out, uint32_t* d_counts_out, uint32_t* d_first_out, uint64_t out_cap,
                      uint64_t* h_unique, cudaStream_t s);
 
+// ---- MinHash sketches (sketch.cu) -----------------------------------------------
+constexpr uint64_t SPARSE_TILE_BYTES = 8192, SPARSE_SLICE_BYTES = 131072;   // the sparse walker's tile and CTA slice
+struct SketchGenome {                 // one genome of a sketch round
+    uint64_t tau;                     // windows whose hash is <= tau survive (~0: every window)
+    uint64_t region;                  // first slot of the genome's survivor region
+    uint64_t cap;                     // slots of that region
+    unsigned long long count;         // survivors (zeroed by the host; above cap: the region overflowed)
+};
+enum : uint32_t { SKETCH_DONE = 0, SKETCH_MORE = 1, SKETCH_OVERFLOW = 2 };    // status of a genome after a round
+// the seed term of the hash, added to the key before fmix64
+inline uint64_t sketch_seed_add(uint64_t seed) { return 0x9E3779B97F4A7C15ull * (seed + 1); }
+int launch_sketch_emit(const uint8_t* d_fasta, const GenomeDev* d_genomes, const Slice* d_slices, int n_slices, int k,
+                       int min_rec, bool canonical, uint64_t seed, SketchGenome* d_sg, uint64_t* d_regions, cudaStream_t s);
+size_t sketch_sort_temp_bytes(int n_items, int n_segments);
+// d_seg: 2 * n_active ints of scratch; d_status[i] is the status of genome d_active[i]
+int launch_sketch_select(const SketchGenome* d_sg, const int* d_active, int n_active, int* d_seg, int n_items,
+                         const uint64_t* d_regions, uint64_t* d_sorted, void* temp, size_t temp_bytes, int sketch_size,
+                         uint64_t* d_sketches, uint64_t stride, uint32_t* d_filled, uint32_t* d_status, cudaStream_t s);
+int launch_sketch_distance(const uint64_t* d_sketches, uint64_t stride, const uint32_t* d_filled, int n, int sketch_size,
+                           int k, int row_begin, int row_end, int metric, float* d_out32, double* d_out64, cudaStream_t s);
+
 // ---- k{k}.txt text (format.cu) --------------------------------------------------
 size_t format_workspace_bytes(uint64_t n_bins, uint64_t max_lines);
 int run_format_dense(void* workspace, int k, const uint32_t* d_counts, const uint32_t* d_first, bool canonical,

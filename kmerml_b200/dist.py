@@ -258,6 +258,47 @@ def distance_matrix_from_shards(counts, shards, metric="cosine", planes_fn=None,
     return Dg[pos][:, pos]
 
 
+def sketch_distance_from_shards(sk_local, shards, metric="mash", rows_fn=None):
+    """n x n Mash / Jaccard distance matrix of genomes sketched on several GPUs: rank r holds the sketches of the
+    genomes shards[r] (in that order).  The sketches and fill counts of all ranks are all-gathered (every rank padded
+    to the largest shard), every rank computes the row block of its own genomes (kmerml_sketch_distance_rows) and one
+    all_gather assembles the matrix, which is then put into genome order.  Bit-identical to the single-GPU matrix.
+    `rows_fn(sketches, row_begin, row_end, metric)` can be injected (the CPU tests use numpy)."""
+    import torch
+    from . import engine
+    rank, world = _world()
+    rows_fn = rows_fn if rows_fn is not None else engine.sketch_distance_rows_device
+    n_max = max(max(len(s) for s in shards), 1)
+    mine = len(shards[rank])
+    dev = sk_local.hashes.device
+    s = sk_local.s
+    # k, s, seed and canonical travel with the fill counts: sketches made with other parameters are not comparable
+    params = torch.tensor([sk_local.k, s, sk_local.seed, int(sk_local.canonical)], dtype=torch.int64, device=dev)
+    hashes = torch.full((n_max, s), -1, dtype=torch.int64, device=dev)
+    hashes[:mine] = sk_local.hashes[:mine, :s]
+    meta = torch.zeros((n_max + 4,), dtype=torch.int64, device=dev)
+    meta[:mine] = sk_local.filled[:mine].to(torch.int64)
+    meta[n_max:] = params
+    pos = _gathered_positions(shards, dev)
+    if world == 1:
+        block = rows_fn(engine.Sketches(hashes, meta[:n_max].to(torch.int32), *sk_local.params()), 0, n_max, metric)
+        return block[pos][:, pos]
+    metas = torch.empty((world * (n_max + 4),), dtype=torch.int64, device=dev)
+    _all_gather_rows(metas, meta)
+    metas = metas.view(world, n_max + 4)
+    for r in range(world):
+        if not torch.equal(metas[r, n_max:], params):
+            raise ValueError(f"rank {r} sketched with other parameters (k, s, seed, canonical): "
+                             f"{metas[r, n_max:].tolist()} vs {params.tolist()}")
+    all_hashes = torch.empty((world * n_max, s), dtype=torch.int64, device=dev)
+    _all_gather_rows(all_hashes, hashes)
+    sk_all = engine.Sketches(all_hashes, metas[:, :n_max].reshape(-1).to(torch.int32).contiguous(), *sk_local.params())
+    block = rows_fn(sk_all, rank * n_max, (rank + 1) * n_max, metric)
+    Dg = torch.empty((world * n_max, world * n_max), dtype=block.dtype, device=block.device)
+    _all_gather_rows(Dg, block)
+    return Dg[pos][:, pos]
+
+
 def count_genomes_sharded(fasta_list, k_values, *, min_record_len=None, canonical=False, gather=True, count_batch=None):
     """Dense counts of many genomes: this rank counts its LPT shard; with gather=True the rows
     of all ranks are assembled (in input order) on every rank with one all_gather per tensor.

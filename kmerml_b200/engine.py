@@ -603,3 +603,84 @@ def format_kmer_lines_device(codes, counts, k):
             text = torch.empty(int(nlen.value), dtype=torch.uint8, device=codes.device)
             continue
         return text[:int(nlen.value)]
+
+
+@dataclass
+class Sketches:
+    """Bottom-s MinHash sketches of a batch of genomes (kmerml_sketch_batch): row g of `hashes` holds the filled[g]
+    smallest distinct hashes of genome g's k-mers, ascending, then UINT64_MAX."""
+    hashes: torch.Tensor      # [n, s] int64 storage of uint64
+    filled: torch.Tensor      # [n] int32
+    k: int
+    s: int
+    seed: int
+    canonical: bool
+
+    def __len__(self):
+        return self.hashes.shape[0]
+
+    def params(self):
+        return (self.k, self.s, self.seed, self.canonical)
+
+
+_SKETCH_METRIC = {"mash": _lib.SKETCH_METRIC_MASH, "jaccard": _lib.SKETCH_METRIC_JACCARD}
+
+
+def sketch_batch_device(fasta, offsets, k, *, sketch_size=1000, seed=42, canonical=True, min_record_len=None):
+    """MinHash sketches of genomes already resident in HBM (laid out as for count_dense_device), any k <= 32."""
+    if not (fasta.is_cuda and fasta.dtype == torch.uint8 and fasta.is_contiguous()):
+        raise ValueError("fasta must be a contiguous uint8 CUDA tensor")
+    ctx = _lib.context(fasta.device.index)
+    n = len(offsets) - 1
+    s = int(sketch_size)
+    hashes = torch.empty((n, max(s, 1)), dtype=torch.int64, device=fasta.device)
+    filled = torch.zeros(n, dtype=torch.int32, device=fasta.device)
+    offs = np.asarray(offsets, dtype=np.uint64)
+    stream = torch.cuda.current_stream(fasta.device).cuda_stream
+    _retry_after_cache_release(lambda: _lib.check(_lib.load().kmerml_sketch_batch(
+        ctx.handle, fasta.data_ptr() if fasta.numel() else None, offs.ctypes.data, n, int(k), int(min_record_len or 0),
+        _lib.FLAG_CANONICAL if canonical else 0, s, int(seed) & 0xFFFFFFFFFFFFFFFF, hashes.data_ptr(), hashes.stride(0),
+        filled.data_ptr(), ctypes.c_void_p(stream))))
+    return Sketches(hashes, filled, int(k), s, int(seed), bool(canonical))
+
+
+def _check_sketches(*sketches):
+    for sk in sketches[1:]:
+        if sk.params() != sketches[0].params():
+            raise ValueError("sketches differ in k, sketch size, seed or canonical flag: "
+                             f"{sketches[0].params()} vs {sk.params()}")
+
+
+def sketch_distance_rows_device(sk, row_begin, row_end, metric="mash", *, out_dtype=torch.float32):
+    """Rows [row_begin, row_end) of the Mash or Jaccard distance matrix of the sketches; bit-identical to the same
+    rows of sketch_distance_device."""
+    if metric not in _SKETCH_METRIC:
+        raise ValueError(f"metric must be one of {sorted(_SKETCH_METRIC)}")
+    if out_dtype not in (torch.float32, torch.float64):
+        raise ValueError("out_dtype must be torch.float32 or torch.float64")
+    h = sk.hashes
+    n = h.shape[0]
+    out = torch.empty((max(int(row_end) - int(row_begin), 0), n), dtype=out_dtype, device=h.device)
+    if out.numel() == 0:
+        return out
+    ctx = _lib.context(h.device.index)
+    stream = torch.cuda.current_stream(h.device).cuda_stream
+    o32 = out.data_ptr() if out_dtype == torch.float32 else None
+    o64 = out.data_ptr() if out_dtype == torch.float64 else None
+    _lib.check(_lib.load().kmerml_sketch_distance_rows(
+        ctx.handle, h.data_ptr(), h.stride(0), sk.filled.data_ptr(), n, sk.s, sk.k, int(row_begin), int(row_end),
+        _SKETCH_METRIC[metric], o32, o64, ctypes.c_void_p(stream)))
+    return out
+
+
+def sketch_distance_device(sk, metric="mash", *, out_dtype=torch.float32):
+    """n x n Mash (default) or Jaccard distance matrix of the sketches (kmerml_sketch_distance_rows)."""
+    return sketch_distance_rows_device(sk, 0, len(sk), metric, out_dtype=out_dtype)
+
+
+def concat_sketches(*sketches):
+    """One Sketches of several batches (same k, s, seed and canonical flag), rows in argument order."""
+    _check_sketches(*sketches)
+    first = sketches[0]
+    return Sketches(torch.cat([sk.hashes for sk in sketches]), torch.cat([sk.filled for sk in sketches]),
+                    first.k, first.s, first.seed, first.canonical)
