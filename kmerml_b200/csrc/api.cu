@@ -190,6 +190,143 @@ struct Prof {
     }
 };
 
+// The tables the host builds for one call: 256-byte-aligned blocks at the same offsets in ws.staging, where the host
+// fills them, and in ws.tables, where the kernels read them.  take() every block, open(), then fill() and upload().
+struct Tables {
+    Workspace& ws;
+    size_t size = 0;
+    std::vector<std::pair<size_t, size_t>> filled;          // (offset, bytes) of the blocks to upload
+    size_t take(size_t bytes) {
+        const size_t at = size;
+        size += align_up(bytes, 256);
+        return at;
+    }
+    int open() {
+        int rc = ws.tables.ensure(size);
+        if (!rc) rc = ws.staging.ensure(size);
+        if (rc) return rc;
+        if (!ws.staging_free) KM_CUDA(cudaEventCreateWithFlags(&ws.staging_free, cudaEventDisableTiming));
+        KM_CUDA(cudaEventSynchronize(ws.staging_free));     // the previous call's upload has left the staging buffer
+        return KMERML_OK;
+    }
+    template <class T> T* dev(size_t at) const { return (T*)((uint8_t*)ws.tables.p + at); }
+    template <class T> T* host(size_t at) const { return (T*)((uint8_t*)ws.staging.p + at); }
+    // the host image of `bytes` bytes at `at`, uploaded by the next upload()
+    template <class T> T* fill(size_t at, size_t bytes) {
+        filled.push_back({at, bytes});
+        return host<T>(at);
+    }
+    int upload(cudaStream_t s) {                             // the filled blocks, in layout order
+        std::sort(filled.begin(), filled.end());
+        for (const auto& b : filled)
+            KM_CUDA(cudaMemcpyAsync(dev<uint8_t>(b.first), host<uint8_t>(b.first), b.second, cudaMemcpyHostToDevice, s));
+        filled.clear();
+        KM_CUDA(cudaEventRecord(ws.staging_free, s));
+        return KMERML_OK;
+    }
+};
+
+// The slice table of a walk over the FASTA bytes: every walker's CTAs take their work from one.  Genome g's bytes
+// [offsets[g], offsets[g + 1]), clipped to [range_begin, range_end) when range_end != 0, are cut at absolute multiples
+// of slice_bytes[g] (0: no slices for g).  A slice's end is clipped to the range; its begin never lies before the tile
+// (`tile` bytes) that holds the genome's first walked byte, so no CTA walks the empty tiles below a genome.  The slices
+// are in buffer order, genome g's are [first[g], first[g + 1]), and the last entry is the scratch entry of
+// launch_slice_headers.
+static int plan_slices(const uint64_t* offsets, int n, const uint64_t* slice_bytes, uint64_t tile, uint64_t range_begin,
+                       uint64_t range_end, std::vector<Slice>& slices, std::vector<uint32_t>& first) {
+    slices.clear();
+    first.resize(n + 1);
+    for (int g = 0; g < n; g++) {
+        first[g] = (uint32_t)slices.size();
+        const uint64_t sb = slice_bytes[g];
+        uint64_t lo = offsets[g], hi = offsets[g + 1];
+        if (range_end) { lo = std::max(lo, range_begin); hi = std::min(hi, range_end); }
+        if (!sb || lo >= hi) continue;
+        const uint64_t b0 = lo / sb, b1 = (hi - 1) / sb;
+        if (slices.size() + (b1 - b0 + 1) > 0x7fffffffull) return fail(KMERML_ERR_RANGE, "too many slices");
+        for (uint64_t b = b0; b <= b1; b++) {
+            Slice sl{};
+            sl.genome = (uint32_t)g;
+            sl.begin = std::max(b * sb, lo / tile * tile);
+            sl.end = range_end ? std::min((b + 1) * sb, range_end) : (b + 1) * sb;
+            slices.push_back(sl);
+        }
+    }
+    first[n] = (uint32_t)slices.size();
+    slices.push_back(Slice{});
+    return KMERML_OK;
+}
+
+// A slice table in a call's Tables: the blocks offsets | genome descriptors | stats, and the slices (+ the scratch
+// entry) in a block of their own, which a caller may lay out after its own tables.
+struct Walk {
+    size_t offsets, genomes, stats, slices = 0;
+    int n_genomes, n_slices = 0;
+    Walk(Tables& t, int n)
+        : offsets(t.take((size_t)(n + 1) * 8)), genomes(t.take((size_t)n * sizeof(GenomeDev))),
+          stats(t.take((size_t)n * sizeof(GenomeStats))), n_genomes(n) {}
+    void take_slices(Tables& t, size_t max_slices) { slices = t.take((max_slices + 1) * sizeof(Slice)); }
+};
+
+// Puts a walk on the device: uploads every block filled so far, plus the genome offsets when `h_offsets` is given
+// (then launch_prologue fills the genome descriptors and zeroes the stats) and the planned slices when `plan` is given
+// (then the slice-table kernels settle the header state at every slice start).
+static int put_walk(Tables& t, Walk& w, const uint8_t* d_fasta, const uint64_t* h_offsets, const std::vector<Slice>* plan,
+                    cudaStream_t s) {
+    if (h_offsets) memcpy(t.fill<uint64_t>(w.offsets, (size_t)(w.n_genomes + 1) * 8), h_offsets, (size_t)(w.n_genomes + 1) * 8);
+    if (plan) {
+        memcpy(t.fill<Slice>(w.slices, plan->size() * sizeof(Slice)), plan->data(), plan->size() * sizeof(Slice));
+        w.n_slices = (int)plan->size() - 1;
+    }
+    int rc = t.upload(s);
+    if (!rc && h_offsets)
+        rc = launch_prologue(d_fasta, t.dev<uint64_t>(w.offsets), t.dev<GenomeDev>(w.genomes), t.dev<GenomeStats>(w.stats),
+                             w.n_genomes, s);
+    if (!rc && plan) rc = launch_slice_headers(d_fasta, t.dev<GenomeDev>(w.genomes), t.dev<Slice>(w.slices), w.n_slices, s);
+    return rc;
+}
+
+// The walk of ONE genome that fills [0, nbytes) of the buffer, in slices of `slice_bytes` (first occurrence, encode,
+// sparse), on the device.  No bytes: no slices, nothing launched.
+struct DevWalk {
+    const GenomeDev* genomes = nullptr;
+    const Slice* slices = nullptr;
+    int n_slices = 0;
+};
+static int put_single_walk(Workspace& ws, const uint8_t* d_fasta, uint64_t nbytes, uint64_t slice_bytes, uint64_t tile,
+                           cudaStream_t s, DevWalk* out) {
+    if (!nbytes) return KMERML_OK;
+    const uint64_t offs[2] = {0, nbytes};
+    std::vector<Slice> plan;
+    std::vector<uint32_t> first;
+    int rc = plan_slices(offs, 1, &slice_bytes, tile, 0, 0, plan, first);
+    if (rc) return rc;
+    Tables t{ws};
+    Walk w(t, 1);
+    w.take_slices(t, plan.size() - 1);
+    if ((rc = t.open()) || (rc = put_walk(t, w, d_fasta, offs, &plan, s))) return rc;
+    *out = DevWalk{t.dev<GenomeDev>(w.genomes), t.dev<Slice>(w.slices), w.n_slices};
+    return KMERML_OK;
+}
+
+// Global-atomic counting: ~8 slices per SM over the genome, each of 1 to 64 tiles.
+static uint64_t atomic_slice_bytes(int sm_count, uint64_t genome_bytes) {
+    const uint64_t target = (uint64_t)sm_count * 8;
+    return align_up(std::min<uint64_t>(std::max<uint64_t>(genome_bytes / target, TILE_BYTES), 64ull * TILE_BYTES), TILE_BYTES);
+}
+
+// The buffer and genome offsets of a multi-genome call.  counts32: every genome's windows must fit 32-bit counters.
+static int check_batch(const uint8_t* d_fasta, const uint64_t* h_offsets, int n_genomes, bool counts32) {
+    if (!d_fasta && h_offsets[n_genomes] > h_offsets[0]) return fail(KMERML_ERR_ARG, "d_fasta is null");
+    if ((uintptr_t)d_fasta & 15) return fail(KMERML_ERR_ARG, "device pointers must be 16-byte aligned");
+    for (int g = 0; g < n_genomes; g++) {
+        if (h_offsets[g + 1] < h_offsets[g]) return fail(KMERML_ERR_ARG, "offsets must be non-decreasing");
+        if (counts32 && h_offsets[g + 1] - h_offsets[g] >= (1ull << 32))
+            return fail(KMERML_ERR_RANGE, "a genome of 4 GiB or more does not fit the 32-bit counters");
+    }
+    return KMERML_OK;
+}
+
 static int build_row(const int* k_list, int nk, RowSpec* row, int* kmax, int* kmin) {
     if (!k_list || nk < 1 || nk > 14) return fail(KMERML_ERR_ARG, "k_list must hold 1..14 values");
     row->nk = nk;
@@ -224,20 +361,15 @@ static int count_dense_core(kmerml_ctx* ctx, Workspace& ws, const uint8_t* d_fas
     if (n_genomes < 0) return fail(KMERML_ERR_ARG, "n_genomes < 0");
     if (n_genomes == 0) return KMERML_OK;
     if (!h_offsets || !d_counts) return fail(KMERML_ERR_ARG, "null pointer argument");
-    if (!d_fasta && h_offsets[n_genomes] > h_offsets[0]) return fail(KMERML_ERR_ARG, "d_fasta is null");
-    if (((uintptr_t)d_fasta & 15) || ((uintptr_t)d_counts & 15) || (d_freq && ((uintptr_t)d_freq & 15)))
-        return fail(KMERML_ERR_ARG, "device pointers must be 16-byte aligned");
     if (counts_stride < row.off[nk] || (counts_stride & 3))
         return fail(KMERML_ERR_ARG, "counts_stride must be >= row length and a multiple of 4");
     if (d_freq && (freq_stride < row.off[nk] || (freq_stride & 3)))
         return fail(KMERML_ERR_ARG, "freq_stride must be >= row length and a multiple of 4");
     int min_rec = min_record_len > 0 ? min_record_len : kmax;
     if (min_rec < kmax) return fail(KMERML_ERR_ARG, "min_record_len must be >= max(k_list)");
-    for (int g = 0; g < n_genomes; g++) {
-        if (h_offsets[g + 1] < h_offsets[g]) return fail(KMERML_ERR_ARG, "offsets must be non-decreasing");
-        if (h_offsets[g + 1] - h_offsets[g] >= (1ull << 32))
-            return fail(KMERML_ERR_RANGE, "a genome of 4 GiB or more does not fit the 32-bit counters");
-    }
+    if (((uintptr_t)d_counts & 15) || (d_freq && ((uintptr_t)d_freq & 15)))
+        return fail(KMERML_ERR_ARG, "device pointers must be 16-byte aligned");
+    if ((rc = check_batch(d_fasta, h_offsets, n_genomes, true))) return rc;
     // the level that is actually counted; every lower level comes from the cascade.  k = 8 does not
     // fit the shared histogram of count_kernel<1> (256 KB), so it is counted as 9-mers through the
     // partition path (level 9 is a pass-through scratch level) instead of with global atomics
@@ -303,81 +435,35 @@ static int count_dense_core(kmerml_ctx* ctx, Workspace& ws, const uint8_t* d_fas
         if (v >= 1 && v <= PART_MAX_TILES_PER_RUN) part_tiles_per_slice = v;
     }
     std::vector<uint64_t> slice_bytes(n_genomes);
-    std::vector<uint32_t> first_slice(n_genomes + 1);
-    uint64_t n_slices = 0;
     for (int g = 0; g < n_genomes; g++) {
-        uint64_t bytes = h_offsets[g + 1] - h_offsets[g];
-        uint64_t sb;
-        if (use_part) {
-            sb = (uint64_t)TILE_BYTES * part_tiles_per_slice;   // a CTA walks a run of consecutive tiles
-        } else if (use_smem) {
-            if ((uint64_t)n_genomes >= target) sb = 1ull << 40;
-            else sb = align_up(std::max<uint64_t>(total_bytes / target, 4ull * TILE_BYTES), TILE_BYTES);
-        } else {
-            sb = align_up(std::min<uint64_t>(std::max<uint64_t>(bytes / target, TILE_BYTES), 64ull * TILE_BYTES), TILE_BYTES);
-        }
-        slice_bytes[g] = sb;
-        first_slice[g] = (uint32_t)n_slices;
-        uint64_t lo = h_offsets[g], hi = h_offsets[g + 1];
-        if (range_end) { lo = std::max(lo, range_begin); hi = std::min(hi, range_end); }
-        if (lo < hi) {
-            uint64_t b0 = lo / sb, b1 = (hi - 1) / sb;
-            n_slices += b1 - b0 + 1;
-        }
-        if (n_slices > 0x7fffffffull) return fail(KMERML_ERR_RANGE, "too many slices");
+        if (use_part)
+            slice_bytes[g] = (uint64_t)TILE_BYTES * part_tiles_per_slice;   // a CTA walks a run of consecutive tiles
+        else if (use_smem)
+            slice_bytes[g] = (uint64_t)n_genomes >= target ? 1ull << 40      // a genome per CTA
+                             : align_up(std::max<uint64_t>(total_bytes / target, 4ull * TILE_BYTES), TILE_BYTES);
+        else
+            slice_bytes[g] = atomic_slice_bytes(ctx->sm_count, h_offsets[g + 1] - h_offsets[g]);
     }
-    first_slice[n_genomes] = (uint32_t)n_slices;
-    // ---- tables: offsets | genomes | stats | slices
-    const size_t off_bytes = align_up((size_t)(n_genomes + 1) * 8, 256);
-    const size_t gen_bytes = align_up((size_t)n_genomes * sizeof(GenomeDev), 256);
-    const size_t st_bytes = align_up((size_t)n_genomes * sizeof(GenomeStats), 256);
-    const size_t sl_bytes = align_up((size_t)(n_slices + 1) * sizeof(Slice), 256);   // + 1 scratch entry
-    const size_t gt_bytes = align_up((size_t)n_genomes * 8, 256);
-    rc = ws.tables.ensure(off_bytes + gen_bytes + st_bytes + sl_bytes + gt_bytes);
+    std::vector<Slice> plan;
+    std::vector<uint32_t> first_slice;
+    rc = plan_slices(h_offsets, n_genomes, slice_bytes.data(), TILE_BYTES, range_begin, range_end, plan, first_slice);
     if (rc) return rc;
-    rc = ws.staging.ensure(off_bytes + sl_bytes + gt_bytes);
-    if (rc) return rc;
-    if (!ws.staging_free) KM_CUDA(cudaEventCreateWithFlags(&ws.staging_free, cudaEventDisableTiming));
-    KM_CUDA(cudaEventSynchronize(ws.staging_free));     // previous call's upload has left the staging buffer
-    uint8_t* base = (uint8_t*)ws.tables.p;
-    uint64_t* d_offsets = (uint64_t*)base;
-    GenomeDev* d_genomes = (GenomeDev*)(base + off_bytes);
-    GenomeStats* d_stats = (GenomeStats*)(base + off_bytes + gen_bytes);
-    Slice* d_slices = (Slice*)(base + off_bytes + gen_bytes + st_bytes);
-    uint8_t* hs = (uint8_t*)ws.staging.p;
-    memcpy(hs, h_offsets, (size_t)(n_genomes + 1) * 8);
-    Slice* h_slices = (Slice*)(hs + off_bytes);
-    {
-        uint64_t si = 0;
-        for (int g = 0; g < n_genomes; g++) {
-            uint64_t lo = h_offsets[g], hi = h_offsets[g + 1];
-            if (range_end) { lo = std::max(lo, range_begin); hi = std::min(hi, range_end); }
-            if (lo >= hi) continue;
-            uint64_t sb = slice_bytes[g];
-            uint64_t b0 = lo / sb, b1 = (hi - 1) / sb;
-            for (uint64_t b = b0; b <= b1; b++) {
-                h_slices[si].genome = (uint32_t)g;
-                h_slices[si].prev_ok = 0;
-                h_slices[si].prev16 = 0;
-                // a range cuts whole tiles: clip the slice to it (range_begin is tile-aligned)
-                h_slices[si].begin = range_end ? std::max(b * sb, range_begin) : b * sb;
-                h_slices[si].end = range_end ? std::min((b + 1) * sb, range_end) : (b + 1) * sb;
-                if (use_part)     // skip the empty tiles before the genome's first byte
-                    h_slices[si].begin = std::max<uint64_t>(h_slices[si].begin, lo / TILE_BYTES * TILE_BYTES);
-                h_slices[si].tile0 = 0;
-                h_slices[si].hdr_until = 0;
-                si++;
-            }
-        }
-        h_slices[n_slices].genome = 0;                      // scratch entry of launch_slice_headers
-    }
+    const uint64_t n_slices = first_slice[n_genomes];
+    // ---- tables: the walk | partition path: genome -> (first run, runs)
+    Tables t{ws};
+    Walk walk(t, n_genomes);
+    walk.take_slices(t, n_slices);
+    const size_t at_gruns = t.take((size_t)n_genomes * 8);
+    if ((rc = t.open())) return rc;
+    const GenomeDev* d_genomes = t.dev<GenomeDev>(walk.genomes);
+    GenomeStats* d_stats = t.dev<GenomeStats>(walk.stats);
+    const Slice* d_slices = t.dev<Slice>(walk.slices);
     // partition path: genomes are processed in groups whose payload workspace is bounded; a slice is a run
     // (the tiles one partition CTA walks), and a run's regions take tiles_per_run * 64 KB of payload
-    uint32_t* d_gruns = (uint32_t*)(base + off_bytes + gen_bytes + st_bytes + sl_bytes);
-    uint32_t* h_gruns = (uint32_t*)(hs + off_bytes + sl_bytes);
     std::vector<int> group_end;                              // exclusive genome index per group
     const uint64_t run_payload_bytes = (uint64_t)part_tiles_per_slice * PART_STAGE_ENTRIES * 2;
     if (use_part) {
+        uint32_t* h_gruns = t.fill<uint32_t>(at_gruns, (size_t)n_genomes * 8);
         const uint64_t max_runs = std::max<uint64_t>(ctx->max_group_payload / run_payload_bytes, 1);
         uint64_t in_group = 0;
         uint32_t group_run0 = 0;
@@ -394,15 +480,9 @@ static int count_dense_core(kmerml_ctx* ctx, Workspace& ws, const uint8_t* d_fas
         }
         group_end.push_back(n_genomes);
     }
-    KM_CUDA(cudaMemcpyAsync(d_offsets, hs, off_bytes, cudaMemcpyHostToDevice, s));
-    KM_CUDA(cudaMemcpyAsync(d_slices, h_slices, sl_bytes, cudaMemcpyHostToDevice, s));
-    if (use_part) KM_CUDA(cudaMemcpyAsync(d_gruns, h_gruns, gt_bytes, cudaMemcpyHostToDevice, s));
-    KM_CUDA(cudaEventRecord(ws.staging_free, s));
-
     {
         Prof pr(ctx, s, 3, 4);      // prologue + the three slice-table kernels
-        rc = launch_prologue(d_fasta, d_offsets, d_genomes, d_stats, n_genomes, s);
-        if (!rc) rc = launch_slice_headers(d_fasta, d_genomes, d_slices, (int)n_slices, s);
+        rc = put_walk(t, walk, d_fasta, h_offsets, &plan, s);
     }
     if (rc) return rc;
     const int n_cascade = cascade_launches(kcount, kmin);
@@ -458,7 +538,7 @@ static int count_dense_core(kmerml_ctx* ctx, Workspace& ws, const uint8_t* d_fas
             if (rc) return rc;
             {
                 Prof pr(ctx, s, 5, 1);
-                rc = launch_bucket(lm, row, kcount, kmin, d_gruns, part_tiles_per_slice, d_payload, d_nsec, d_stats,
+                rc = launch_bucket(lm, row, kcount, kmin, t.dev<uint32_t>(at_gruns), part_tiles_per_slice, d_payload, d_nsec, d_stats,
                                    canonical ? nullptr : d_freq, freq_stride, d_totals, (uint32_t)g0, ng, s);
             }
             if (rc) return rc;
@@ -552,50 +632,6 @@ static int count_dense_group(kmerml_ctx* ctx, Workspace& ws, const uint8_t* d_fa
     }
     return count_dense_core(ctx, ws, d_fasta, starts, n, k_list, nk, min_record_len, flags, d_counts, counts_stride, d_freq,
                             freq_stride, d_totals, s);
-}
-
-// Slice table of ONE genome that fills the whole buffer (first occurrence, encode): prologue + header state.
-static int single_genome_tables(kmerml_ctx* ctx, Workspace& ws, const uint8_t* d_fasta, uint64_t nbytes, cudaStream_t s,
-                                const GenomeDev** d_genomes, const Slice** d_slices, int* n_slices_out) {
-    const uint64_t sb = align_up(std::min<uint64_t>(std::max<uint64_t>(nbytes / ((uint64_t)ctx->sm_count * 8), TILE_BYTES),
-                                                    64ull * TILE_BYTES), TILE_BYTES);
-    const uint64_t n_slices = (nbytes - 1) / sb + 1;
-    const size_t off_bytes = 256, gen_bytes = 256, st_bytes = 256;
-    const size_t sl_bytes = align_up((size_t)(n_slices + 1) * sizeof(Slice), 256);   // + 1 scratch entry
-    int rc = ws.tables.ensure(off_bytes + gen_bytes + st_bytes + sl_bytes);
-    if (rc) return rc;
-    if ((rc = ws.staging.ensure(off_bytes + sl_bytes))) return rc;
-    if (!ws.staging_free) KM_CUDA(cudaEventCreateWithFlags(&ws.staging_free, cudaEventDisableTiming));
-    KM_CUDA(cudaEventSynchronize(ws.staging_free));
-    uint8_t* base = (uint8_t*)ws.tables.p;
-    uint8_t* hs = (uint8_t*)ws.staging.p;
-    uint64_t* ho = (uint64_t*)hs;
-    ho[0] = 0;
-    ho[1] = nbytes;
-    Slice* h_slices = (Slice*)(hs + off_bytes);
-    for (uint64_t b = 0; b < n_slices; b++) {
-        h_slices[b].genome = 0;
-        h_slices[b].prev_ok = 0;
-        h_slices[b].prev16 = 0;
-        h_slices[b].tile0 = 0;
-        h_slices[b].begin = b * sb;
-        h_slices[b].end = (b + 1) * sb;
-        h_slices[b].hdr_until = 0;
-    }
-    h_slices[n_slices].genome = 0;                          // scratch entry of launch_slice_headers
-    KM_CUDA(cudaMemcpyAsync(base, hs, off_bytes, cudaMemcpyHostToDevice, s));
-    KM_CUDA(cudaMemcpyAsync(base + off_bytes + gen_bytes + st_bytes, h_slices, sl_bytes, cudaMemcpyHostToDevice, s));
-    KM_CUDA(cudaEventRecord(ws.staging_free, s));
-    rc = launch_prologue(d_fasta, (const uint64_t*)base, (GenomeDev*)(base + off_bytes),
-                         (GenomeStats*)(base + off_bytes + gen_bytes), 1, s);
-    if (rc) return rc;
-    rc = launch_slice_headers(d_fasta, (const GenomeDev*)(base + off_bytes),
-                              (Slice*)(base + off_bytes + gen_bytes + st_bytes), (int)n_slices, s);
-    if (rc) return rc;
-    *d_genomes = (const GenomeDev*)(base + off_bytes);
-    *d_slices = (const Slice*)(base + off_bytes + gen_bytes + st_bytes);
-    *n_slices_out = (int)n_slices;
-    return KMERML_OK;
 }
 
 }  // namespace km
@@ -1396,13 +1432,14 @@ static int count_sparse_core(kmerml_ctx* ctx, const uint8_t* d_fasta, uint64_t n
     if (int orc = order_stream(ctx, (cudaStream_t)stream)) return orc;
     // at most one window ends at every byte of the range; the slice table covers the whole file
     const uint64_t cap = std::max<uint64_t>(range_end - range_begin, 1);
-    int rc = ws.part.ensure(sparse_workspace_bytes(cap, nbytes));
+    int rc = ws.part.ensure(sparse_workspace_bytes(cap));
     if (rc) return rc;
-    rc = run_sparse_in(ws.part.p, d_fasta, nbytes, range_begin, range_end, k, min_rec,
+    DevWalk w;
+    if ((rc = put_single_walk(ws, d_fasta, nbytes, SPARSE_SLICE_BYTES, SPARSE_TILE_BYTES, (cudaStream_t)stream, &w))) return rc;
+    rc = run_sparse_in(ws.part.p, d_fasta, w.genomes, w.slices, w.n_slices, range_begin, range_end, k, min_rec,
                        (flags & KMERML_FLAG_CANONICAL) != 0, cap, d_keys, d_counts, d_first, out_cap, h_unique,
                        h_windows, &ctx->sparse_pending, (cudaStream_t)stream);
     ctx->sparse_pending.cap = cap;
-    ctx->sparse_pending.nbytes = nbytes;
     ctx->sparse_pending.workspace = ws.part.p;
     return rc;
 }
@@ -1427,10 +1464,12 @@ int kmerml_emit_sparse_range(kmerml_ctx* ctx, const uint8_t* d_fasta, uint64_t n
     Workspace& ws = ctx->ws[0];
     if (int orc = order_stream(ctx, (cudaStream_t)stream)) return orc;
     const uint64_t cap = std::max<uint64_t>(range_end - range_begin, 1);
-    int rc = ws.part.ensure(sparse_workspace_bytes(cap, nbytes));
+    int rc = ws.part.ensure(sparse_workspace_bytes(cap));
     if (rc) return rc;
     ctx->sparse_pending.valid = false;
-    return run_sparse_emit_by_owner(ws.part.p, d_fasta, nbytes, range_begin, range_end, k, min_rec,
+    DevWalk w;
+    if ((rc = put_single_walk(ws, d_fasta, nbytes, SPARSE_SLICE_BYTES, SPARSE_TILE_BYTES, (cudaStream_t)stream, &w))) return rc;
+    return run_sparse_emit_by_owner(ws.part.p, d_fasta, w.genomes, w.slices, w.n_slices, range_begin, range_end, k, min_rec,
                                     (flags & KMERML_FLAG_CANONICAL) != 0, owner_bits, cap, d_keys, d_ends, out_cap, h_windows,
                                     h_owner_counts, (cudaStream_t)stream);
 }
@@ -1447,12 +1486,11 @@ int kmerml_reduce_sparse_windows(kmerml_ctx* ctx, int sort_bits, const uint64_t*
     Workspace& ws = ctx->ws[0];
     if (int orc = order_stream(ctx, (cudaStream_t)stream)) return orc;
     const uint64_t cap = std::max<uint64_t>(n, 1);
-    int rc = ws.part.ensure(sparse_workspace_bytes(cap, 0));
+    int rc = ws.part.ensure(sparse_workspace_bytes(cap));
     if (rc) return rc;
     rc = run_sparse_reduce_windows(ws.part.p, sort_bits, d_keys, d_ends, n, d_keys_out, d_counts_out, d_first_out, out_cap,
                                    h_unique, &ctx->sparse_pending, (cudaStream_t)stream);
     ctx->sparse_pending.cap = cap;
-    ctx->sparse_pending.nbytes = 0;
     ctx->sparse_pending.workspace = ws.part.p;
     return rc;
 }
@@ -1467,7 +1505,7 @@ int kmerml_sparse_fetch(kmerml_ctx* ctx, uint64_t* d_keys, uint32_t* d_counts, u
     DeviceGuard guard(ctx->device);
     if (!guard.ok) return fail(KMERML_ERR_CUDA, "cudaSetDevice failed");
     if (int orc = order_stream(ctx, (cudaStream_t)stream)) return orc;
-    return sparse_fetch(ctx->ws[0].part.p, p.cap, p.nbytes, p, d_keys, d_counts, d_first, (cudaStream_t)stream);
+    return sparse_fetch(ctx->ws[0].part.p, p, d_keys, d_counts, d_first, (cudaStream_t)stream);
 }
 
 int kmerml_count_sparse(kmerml_ctx* ctx, const uint8_t* d_fasta, uint64_t nbytes, int k, int min_record_len,
@@ -1518,12 +1556,10 @@ int kmerml_first_occurrence(kmerml_ctx* ctx, const uint8_t* d_fasta, uint64_t nb
     if (int orc = order_stream(ctx, (cudaStream_t)stream)) return orc;
     KM_CUDA(cudaMemsetAsync(d_first, 0xFF, (size_t)(1ull << (2 * k)) * 4, s));
     if (!nbytes) return KMERML_OK;
-    const GenomeDev* d_genomes = nullptr;
-    const Slice* d_slices = nullptr;
-    int n_slices = 0;
-    int rc = single_genome_tables(ctx, ws, d_fasta, nbytes, s, &d_genomes, &d_slices, &n_slices);
+    DevWalk w;
+    int rc = put_single_walk(ws, d_fasta, nbytes, atomic_slice_bytes(ctx->sm_count, nbytes), TILE_BYTES, s, &w);
     if (rc) return rc;
-    return launch_first_occurrence(d_fasta, d_genomes, d_slices, n_slices, k, min_rec, d_first, s);
+    return launch_first_occurrence(d_fasta, w.genomes, w.slices, w.n_slices, k, min_rec, d_first, s);
 }
 
 // ---- MinHash sketches (sketch.cu) ----
@@ -1546,51 +1582,23 @@ constexpr uint64_t SKETCH_ROUND_SLOTS = 1ull << 28;     // survivor slots of one
 static int sketch_batch_core(kmerml_ctx* ctx, const uint8_t* d_fasta, const uint64_t* h_offsets, int n, int k, int min_rec,
                              bool canonical, int sketch_size, uint64_t seed, uint64_t* d_sketches, uint64_t stride,
                              uint32_t* d_filled, cudaStream_t s) {
-    Workspace& ws = ctx->ws[0];
-    const uint64_t sb = SPARSE_SLICE_BYTES;
-    auto slice_range = [&](int g, uint64_t* b0, uint64_t* b1) {
-        *b0 = h_offsets[g] / sb;
-        *b1 = (h_offsets[g + 1] - 1) / sb + 1;
-    };
-    uint64_t max_slices = 0;
-    for (int g = 0; g < n; g++) {
-        if (h_offsets[g + 1] == h_offsets[g]) continue;
-        uint64_t b0, b1;
-        slice_range(g, &b0, &b1);
-        max_slices += b1 - b0;
-    }
-    if (max_slices > 0x7fffffffull) return fail(KMERML_ERR_RANGE, "too many slices");
+    // the slice table of a round holds at most the slices of every genome
+    std::vector<uint64_t> slice_bytes(n, SPARSE_SLICE_BYTES);
+    std::vector<Slice> plan;
+    std::vector<uint32_t> first;
+    int rc = plan_slices(h_offsets, n, slice_bytes.data(), SPARSE_TILE_BYTES, 0, 0, plan, first);
+    if (rc) return rc;
     // tables: offsets | genomes | stats | sketch genomes | active | segments | status | slices
-    const size_t off_bytes = align_up((size_t)(n + 1) * 8, 256);
-    const size_t gen_bytes = align_up((size_t)n * sizeof(GenomeDev), 256);
-    const size_t st_bytes = align_up((size_t)n * sizeof(GenomeStats), 256);
-    const size_t sg_bytes = align_up((size_t)n * sizeof(SketchGenome), 256);
-    const size_t act_bytes = align_up((size_t)n * 4, 256);
-    const size_t seg_bytes = align_up((size_t)n * 8, 256);
-    const size_t sl_bytes = align_up((size_t)(max_slices + 1) * sizeof(Slice), 256);     // + 1 scratch entry
-    int rc = ws.tables.ensure(off_bytes + gen_bytes + st_bytes + sg_bytes + act_bytes + seg_bytes + act_bytes + sl_bytes);
-    if (rc) return rc;
-    rc = ws.staging.ensure(off_bytes + sg_bytes + act_bytes + act_bytes + sl_bytes);
-    if (rc) return rc;
-    if (!ws.staging_free) KM_CUDA(cudaEventCreateWithFlags(&ws.staging_free, cudaEventDisableTiming));
-    KM_CUDA(cudaEventSynchronize(ws.staging_free));     // previous call's upload has left the staging buffer
-    uint8_t* base = (uint8_t*)ws.tables.p;
-    uint64_t* d_offsets = (uint64_t*)base;
-    GenomeDev* d_genomes = (GenomeDev*)(base += off_bytes);
-    GenomeStats* d_stats = (GenomeStats*)(base += gen_bytes);
-    SketchGenome* d_sg = (SketchGenome*)(base += st_bytes);
-    int* d_active = (int*)(base += sg_bytes);
-    int* d_seg = (int*)(base += act_bytes);
-    uint32_t* d_status = (uint32_t*)(base += seg_bytes);
-    Slice* d_slices = (Slice*)(base += act_bytes);
-    uint8_t* hs = (uint8_t*)ws.staging.p;
-    SketchGenome* h_sg = (SketchGenome*)(hs + off_bytes);
-    int* h_active = (int*)(hs + off_bytes + sg_bytes);
-    uint32_t* h_status = (uint32_t*)(hs + off_bytes + sg_bytes + act_bytes);
-    Slice* h_slices = (Slice*)(hs + off_bytes + sg_bytes + 2 * act_bytes);
-    memcpy(hs, h_offsets, (size_t)(n + 1) * 8);
-    KM_CUDA(cudaMemcpyAsync(d_offsets, hs, off_bytes, cudaMemcpyHostToDevice, s));
-    if ((rc = launch_prologue(d_fasta, d_offsets, d_genomes, d_stats, n, s))) return rc;
+    Tables t{ctx->ws[0]};
+    Walk walk(t, n);
+    const size_t at_sg = t.take((size_t)n * sizeof(SketchGenome)), at_active = t.take((size_t)n * 4);
+    const size_t at_seg = t.take((size_t)n * 8), at_status = t.take((size_t)n * 4);
+    walk.take_slices(t, plan.size() - 1);
+    if ((rc = t.open()) || (rc = put_walk(t, walk, d_fasta, h_offsets, nullptr, s))) return rc;
+    const GenomeDev* d_genomes = t.dev<GenomeDev>(walk.genomes);
+    const Slice* d_slices = t.dev<Slice>(walk.slices);
+    uint32_t* h_status = t.host<uint32_t>(at_status);
+    Workspace& ws = ctx->ws[0];
 
     std::vector<uint64_t> tau(n), cap(n);
     std::vector<int> pending(n);
@@ -1602,9 +1610,12 @@ static int sketch_batch_core(kmerml_ctx* ctx, const uint8_t* d_fasta, const uint
     }
     while (!pending.empty()) {
         // one round: the pending genomes (in buffer order) whose regions fit SKETCH_ROUND_SLOTS, at least one
+        SketchGenome* h_sg = t.fill<SketchGenome>(at_sg, (size_t)n * sizeof(SketchGenome));
+        int* h_active = t.host<int>(at_active);
         memset(h_sg, 0, (size_t)n * sizeof(SketchGenome));
+        std::fill(slice_bytes.begin(), slice_bytes.end(), 0);
         int n_round = 0;
-        uint64_t slots = 0, n_slices = 0;
+        uint64_t slots = 0;
         for (int g : pending) {
             if (n_round && slots + cap[g] > SKETCH_ROUND_SLOTS) break;
             if (slots + cap[g] > 0x7fffffffull)
@@ -1614,38 +1625,26 @@ static int sketch_batch_core(kmerml_ctx* ctx, const uint8_t* d_fasta, const uint
             h_sg[g].cap = cap[g];
             h_active[n_round++] = g;
             slots += cap[g];
-            if (h_offsets[g + 1] == h_offsets[g]) continue;
-            uint64_t b0, b1;
-            slice_range(g, &b0, &b1);
-            for (uint64_t b = b0; b < b1; b++) {
-                Slice& sl = h_slices[n_slices++];
-                memset(&sl, 0, sizeof(Slice));
-                sl.genome = (uint32_t)g;
-                // skip the empty tiles before the genome's first byte
-                sl.begin = std::max<uint64_t>(b * sb, h_offsets[g] / SPARSE_TILE_BYTES * SPARSE_TILE_BYTES);
-                sl.end = (b + 1) * sb;
-            }
+            slice_bytes[g] = SPARSE_SLICE_BYTES;
         }
-        h_slices[n_slices].genome = 0;                      // scratch entry of launch_slice_headers
+        t.fill<int>(at_active, (size_t)n_round * 4);
+        if ((rc = plan_slices(h_offsets, n, slice_bytes.data(), SPARSE_TILE_BYTES, 0, 0, plan, first))) return rc;
         const size_t region_bytes = align_up(std::max<uint64_t>(slots, 1) * 8, 256);
         const size_t temp_bytes = sketch_sort_temp_bytes((int)slots, n_round);
         if ((rc = ws.part.ensure(2 * region_bytes + temp_bytes))) return rc;
         uint64_t* d_regions = (uint64_t*)ws.part.p;
         uint64_t* d_sorted = (uint64_t*)((uint8_t*)ws.part.p + region_bytes);
         void* d_temp = (uint8_t*)ws.part.p + 2 * region_bytes;
-        KM_CUDA(cudaMemcpyAsync(d_sg, h_sg, (size_t)n * sizeof(SketchGenome), cudaMemcpyHostToDevice, s));
-        KM_CUDA(cudaMemcpyAsync(d_active, h_active, (size_t)n_round * 4, cudaMemcpyHostToDevice, s));
-        KM_CUDA(cudaMemcpyAsync(d_slices, h_slices, (size_t)(n_slices + 1) * sizeof(Slice), cudaMemcpyHostToDevice, s));
         {
             Prof pr(ctx, s, 3, 7);      // the three slice-table kernels, emit, segments, sort, select
-            rc = launch_slice_headers(d_fasta, d_genomes, d_slices, (int)n_slices, s);
-            if (!rc) rc = launch_sketch_emit(d_fasta, d_genomes, d_slices, (int)n_slices, k, min_rec, canonical, seed, d_sg,
+            rc = put_walk(t, walk, d_fasta, nullptr, &plan, s);
+            if (!rc) rc = launch_sketch_emit(d_fasta, d_genomes, d_slices, walk.n_slices, k, min_rec, canonical, seed, t.dev<SketchGenome>(at_sg),
                                              d_regions, s);
-            if (!rc) rc = launch_sketch_select(d_sg, d_active, n_round, d_seg, (int)slots, d_regions, d_sorted, d_temp,
-                                               temp_bytes, sketch_size, d_sketches, stride, d_filled, d_status, s);
+            if (!rc) rc = launch_sketch_select(t.dev<SketchGenome>(at_sg), t.dev<int>(at_active), n_round, t.dev<int>(at_seg), (int)slots, d_regions, d_sorted, d_temp,
+                                               temp_bytes, sketch_size, d_sketches, stride, d_filled, t.dev<uint32_t>(at_status), s);
         }
         if (rc) return rc;
-        KM_CUDA(cudaMemcpyAsync(h_status, d_status, (size_t)n_round * 4, cudaMemcpyDeviceToHost, s));
+        KM_CUDA(cudaMemcpyAsync(h_status, t.dev<uint32_t>(at_status), (size_t)n_round * 4, cudaMemcpyDeviceToHost, s));
         KM_CUDA(cudaStreamSynchronize(s));
         // run again: too few distinct hashes below tau -> 16 tau (saturating at every window); overflow -> one slot
         // per byte.  Every window with one slot per byte cannot fail, so the loop ends.
@@ -1667,7 +1666,6 @@ static int sketch_batch_core(kmerml_ctx* ctx, const uint8_t* d_fasta, const uint
         std::sort(next.begin(), next.end());            // the slice table stays in buffer order
         pending.swap(next);
     }
-    KM_CUDA(cudaEventRecord(ws.staging_free, s));
     return KMERML_OK;
 }
 
@@ -1684,10 +1682,7 @@ int kmerml_sketch_batch(kmerml_ctx* ctx, const uint8_t* d_fasta, const uint64_t*
     if (min_rec < k) return fail(KMERML_ERR_ARG, "min_record_len must be >= k");
     if (n_genomes == 0) return KMERML_OK;
     if (!h_offsets || !d_sketches || !d_filled) return fail(KMERML_ERR_ARG, "null pointer argument");
-    if (!d_fasta && h_offsets[n_genomes] > h_offsets[0]) return fail(KMERML_ERR_ARG, "d_fasta is null");
-    if ((uintptr_t)d_fasta & 15) return fail(KMERML_ERR_ARG, "device pointers must be 16-byte aligned");
-    for (int g = 0; g < n_genomes; g++)
-        if (h_offsets[g + 1] < h_offsets[g]) return fail(KMERML_ERR_ARG, "offsets must be non-decreasing");
+    if (int rc = check_batch(d_fasta, h_offsets, n_genomes, false)) return rc;
     DeviceGuard guard(ctx->device);
     if (!guard.ok) return fail(KMERML_ERR_CUDA, "cudaSetDevice failed");
     if (int orc = order_stream(ctx, (cudaStream_t)stream)) return orc;
@@ -1793,13 +1788,11 @@ int kmerml_encode(kmerml_ctx* ctx, const uint8_t* d_fasta, uint64_t nbytes, uint
     }
     if (!nbytes) return KMERML_OK;
     KM_CUDA(cudaMemsetAsync(d_symbols, 0xFF, (size_t)nbytes, s));
-    const GenomeDev* d_genomes = nullptr;
-    const Slice* d_slices = nullptr;
-    int n_slices = 0;
-    int rc = single_genome_tables(ctx, ws, d_fasta, nbytes, s, &d_genomes, &d_slices, &n_slices);
+    DevWalk w;
+    int rc = put_single_walk(ws, d_fasta, nbytes, atomic_slice_bytes(ctx->sm_count, nbytes), TILE_BYTES, s, &w);
     if (rc) return rc;
     ctx->launches += 1;
-    return launch_encode(d_fasta, d_genomes, d_slices, n_slices, d_symbols, s);
+    return launch_encode(d_fasta, w.genomes, w.slices, w.n_slices, d_symbols, s);
 }
 
 }  // extern "C"

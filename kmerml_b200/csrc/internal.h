@@ -38,7 +38,6 @@ struct Slice {                // unit of work of one CTA: bytes [begin, end) of 
     uint64_t begin, end;      // multiples of the tile size (absolute buffer offsets)
     uint64_t hdr_until;       // slice_header_kernel: `begin` lies in a header line that ends here (else 0)
     uint32_t prev16;          // ... and these are its last 16 bases (the carry of the slice's first chunk)
-    uint32_t tile0;           // partition path: index of the slice's first tile in the group's tile list
     uint64_t line_start;      // slice_header_kernel: start of the line holding `begin` (LS_UNRESOLVED: long line)
     uint64_t scan_last;       // slice_long_scan_kernel: last line start inside the slice before (long lines only)
 };
@@ -162,22 +161,22 @@ struct SparsePending {        // the reduced result of the last sparse count, st
     bool valid = false;
     uint64_t* sorted_keys = nullptr;
     uint32_t* sorted_ends = nullptr;
-    uint64_t* uniq = nullptr;
-    uint32_t* runs = nullptr;
-    uint64_t n = 0, nu = 0, cap = 0, nbytes = 0;
+    uint64_t n = 0, nu = 0, cap = 0;
     const void* workspace = nullptr;
 };
-size_t sparse_workspace_bytes(uint64_t cap, uint64_t nbytes);
-int sparse_fetch(void* workspace, uint64_t cap, uint64_t nbytes, const SparsePending& p, uint64_t* d_keys_out,
-                 uint32_t* d_counts_out, uint32_t* d_first_out, cudaStream_t s);
-int run_sparse_in(void* workspace, const uint8_t* d_fasta, uint64_t nbytes, uint64_t range_begin, uint64_t range_end,
-                  int k, int min_rec, bool canonical, uint64_t cap, uint64_t* d_keys_out, uint32_t* d_counts_out, uint32_t* d_first_out, uint64_t out_cap,
-                  uint64_t* h_unique, uint64_t* h_windows, SparsePending* pending, cudaStream_t s);
-
-int run_sparse_emit_by_owner(void* workspace, const uint8_t* d_fasta, uint64_t nbytes, uint64_t range_begin,
-                             uint64_t range_end, int k, int min_rec, bool canonical, int owner_bits, uint64_t cap,
-                             uint64_t* d_keys_out, uint32_t* d_ends_out, uint64_t out_cap, uint64_t* h_windows,
-                             uint64_t* h_owner_counts, cudaStream_t s);
+size_t sparse_workspace_bytes(uint64_t cap);
+int sparse_fetch(void* workspace, const SparsePending& p, uint64_t* d_keys_out, uint32_t* d_counts_out,
+                 uint32_t* d_first_out, cudaStream_t s);
+// The slice table (d_genomes, d_slices, n_slices) covers the whole file in SPARSE_SLICE_BYTES slices; the slices of
+// [range_begin, range_end) emit their windows.
+int run_sparse_in(void* workspace, const uint8_t* d_fasta, const GenomeDev* d_genomes, const Slice* d_slices, int n_slices,
+                  uint64_t range_begin, uint64_t range_end, int k, int min_rec, bool canonical, uint64_t cap,
+                  uint64_t* d_keys_out, uint32_t* d_counts_out, uint32_t* d_first_out, uint64_t out_cap, uint64_t* h_unique,
+                  uint64_t* h_windows, SparsePending* pending, cudaStream_t s);
+int run_sparse_emit_by_owner(void* workspace, const uint8_t* d_fasta, const GenomeDev* d_genomes, const Slice* d_slices,
+                             int n_slices, uint64_t range_begin, uint64_t range_end, int k, int min_rec, bool canonical,
+                             int owner_bits, uint64_t cap, uint64_t* d_keys_out, uint32_t* d_ends_out, uint64_t out_cap,
+                             uint64_t* h_windows, uint64_t* h_owner_counts, cudaStream_t s);
 int run_sparse_reduce_windows(void* workspace, int sort_bits, const uint64_t* d_keys, const uint32_t* d_ends, uint64_t n,
                               uint64_t* d_keys_out, uint32_t* d_counts_out, uint32_t* d_first_out, uint64_t out_cap,
                               uint64_t* h_unique, SparsePending* pending, cudaStream_t s);

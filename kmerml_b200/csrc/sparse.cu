@@ -59,24 +59,6 @@ struct WindowSink {
     }
 };
 
-__global__ void sparse_setup_kernel(const uint8_t* __restrict__ buf, uint64_t nbytes, GenomeDev* gd, Slice* slices,
-                                    int n_slices) {
-    const int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i == 0) {
-        gd->file_lo = 0;
-        gd->lo = first_header(buf, 0, nbytes);       // text before the first header line is ignored
-        gd->hi = nbytes;
-    }
-    if (i <= n_slices) {                             // entry n_slices = scratch of launch_slice_headers
-        Slice sl;
-        sl.genome = 0; sl.prev_ok = 0; sl.prev16 = 0; sl.tile0 = 0; sl.hdr_until = 0;
-        sl.begin = (uint64_t)i * SPARSE_TILE * SPARSE_TILES_PER_SLICE;
-        sl.end = sl.begin + (uint64_t)SPARSE_TILE * SPARSE_TILES_PER_SLICE;
-        sl.line_start = 0; sl.scan_last = 0;
-        slices[i] = sl;
-    }
-}
-
 __global__ void __launch_bounds__(SPARSE_THREADS)
 sparse_emit_kernel(const uint8_t* __restrict__ buf, const GenomeDev* __restrict__ gds, const Slice* __restrict__ slices,
                    SparseParams P, uint64_t* keys, uint32_t* ends, unsigned long long* cursor, uint64_t cap) {
@@ -85,11 +67,6 @@ sparse_emit_kernel(const uint8_t* __restrict__ buf, const GenomeDev* __restrict_
     WindowSink sink;
     sink.keys = keys; sink.ends = ends; sink.cursor = cursor; sink.cap = cap;
     walk_sparse_slice(buf, gd, sl, P, sink);
-}
-
-__global__ void gather_u32_kernel(const uint32_t* __restrict__ src, uint32_t* dst, uint64_t n) {
-    uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < n) dst[i] = src[i];
 }
 
 struct CountFirst {               // count in the high word, first (smallest) offset in the low word
@@ -154,14 +131,12 @@ struct SparseWork {
     uint32_t* ends_b;
     unsigned long long* cursor;
     unsigned long long* n_runs;
-    GenomeDev* genome;
-    Slice* slices;
     void* temp;
     size_t temp_bytes;
 };
 
 // Layout of the workspace for `cap` windows; returns the total number of bytes.
-size_t sparse_workspace(uint64_t cap, uint64_t nbytes, SparseWork* w, uint8_t* base) {
+static size_t sparse_workspace(uint64_t cap, SparseWork* w, uint8_t* base) {
     size_t off = 0;
     auto take = [&](size_t bytes) {
         uint8_t* p = base ? base + off : nullptr;
@@ -175,10 +150,7 @@ size_t sparse_workspace(uint64_t cap, uint64_t nbytes, SparseWork* w, uint8_t* b
     local.ends_b = (uint32_t*)take(cap * 4);
     local.cursor = (unsigned long long*)take(256);
     local.n_runs = (unsigned long long*)take(256);
-    local.genome = (GenomeDev*)take(256);
-    // one slice entry per 128 KB of the whole file + scratch
-    local.slices = (Slice*)take((nbytes / ((uint64_t)SPARSE_TILE * SPARSE_TILES_PER_SLICE) + 3) * sizeof(Slice));
-    size_t t1 = 0, t2 = 0, t3 = 0;
+    size_t t1 = 0, t2 = 0;
     cub::DoubleBuffer<uint64_t> dk(nullptr, nullptr);
     cub::DoubleBuffer<uint32_t> dv(nullptr, nullptr);
     cub::DeviceRadixSort::SortPairs(nullptr, t1, dk, dv, (uint64_t)cap, 0, 64);
@@ -188,21 +160,18 @@ size_t sparse_workspace(uint64_t cap, uint64_t nbytes, SparseWork* w, uint8_t* b
                                        SplitCountFirst{nullptr, nullptr}, (unsigned long long*)nullptr, CountFirst(),
                                        (uint64_t)cap);
     }
-    (void)t3;
-    local.temp_bytes = std::max(t1, std::max(t2, t3));
+    local.temp_bytes = std::max(t1, t2);
     local.temp = take(local.temp_bytes);
     if (w) *w = local;
     return off;
 }
 
-// The reduced result (distinct k-mers in `uniq`, their counts in `runs`) to the caller's buffers; the first
-// offsets are the minimum end offset of every run of the sorted windows.
-static int sparse_copy_out(const SparseWork& w, uint64_t* sorted_keys, uint32_t* sorted_ends, uint64_t* uniq, uint32_t* runs,
-                           uint64_t n, uint64_t nu, uint64_t* d_keys_out, uint32_t* d_counts_out, uint32_t* d_first_out,
-                           cudaStream_t s) {
+// The reduced result to the caller's buffers; the first offsets are the minimum end offset of every run of the sorted
+// windows.
+static int sparse_copy_out(const SparseWork& w, const uint64_t* sorted_keys, const uint32_t* sorted_ends, uint64_t n,
+                           uint64_t* d_keys_out, uint32_t* d_counts_out, uint32_t* d_first_out, cudaStream_t s) {
     // ONE segmented reduction over the sorted windows: distinct k-mers to the caller's key array, (run length, smallest
     // end offset) through a splitting output iterator to its count / first-offset arrays
-    (void)uniq; (void)runs; (void)nu;
     cub::TransformInputIterator<unsigned long long, OneWindow, const uint32_t*> vin(sorted_ends, OneWindow());
     size_t tb = w.temp_bytes;
     KM_CUDA(cub::DeviceReduce::ReduceByKey(w.temp, tb, (const uint64_t*)sorted_keys, d_keys_out, vin,
@@ -212,9 +181,9 @@ static int sparse_copy_out(const SparseWork& w, uint64_t* sorted_keys, uint32_t*
 }
 
 // Emit the windows of the byte range into w.keys_a / w.ends_a; *h_windows receives their number.
-static int sparse_emit_phase(const uint8_t* d_fasta, uint64_t nbytes, uint64_t range_begin, uint64_t range_end, int k,
-                             int min_rec, bool canonical, const SparseWork& w, uint64_t cap, uint64_t* h_windows,
-                             cudaStream_t s) {
+static int sparse_emit_phase(const uint8_t* d_fasta, const GenomeDev* d_genomes, const Slice* d_slices, int n_slices,
+                             uint64_t range_begin, uint64_t range_end, int k, int min_rec, bool canonical,
+                             const SparseWork& w, uint64_t cap, uint64_t* h_windows, cudaStream_t s) {
     SparseParams P;
     P.k = k;
     P.min_rec = min_rec;
@@ -222,18 +191,13 @@ static int sparse_emit_phase(const uint8_t* d_fasta, uint64_t nbytes, uint64_t r
     P.mask = k >= 32 ? ~0ull : ((1ull << (2 * k)) - 1ull);
     KM_CUDA(cudaMemsetAsync(w.cursor, 0, 8, s));
     *h_windows = 0;
-    if (!nbytes) return KMERML_OK;
-    const uint64_t slice_bytes = (uint64_t)SPARSE_TILE * SPARSE_TILES_PER_SLICE;
-    const int n_slices = (int)((nbytes + slice_bytes - 1) / slice_bytes);
-    sparse_setup_kernel<<<(n_slices + 1 + 127) / 128, 128, 0, s>>>(d_fasta, nbytes, w.genome, w.slices, n_slices);
-    KM_CUDA(cudaGetLastError());
-    if (int rc = launch_slice_headers(d_fasta, w.genome, w.slices, n_slices, s)) return rc;
-    // the header state of every slice start is settled over the whole file; only the slices of the
-    // requested byte range (whole slices: the multi-GPU unit) emit their windows
-    const int s0 = (int)std::min<uint64_t>(range_begin / slice_bytes, (uint64_t)n_slices);
-    const int s1 = (int)std::min<uint64_t>((range_end + slice_bytes - 1) / slice_bytes, (uint64_t)n_slices);
+    if (!n_slices) return KMERML_OK;
+    // the slices cover the whole file, so the header state of every slice start is settled over the whole file; only
+    // the slices of the requested byte range (whole slices: the multi-GPU unit) emit their windows
+    const int s0 = (int)std::min<uint64_t>(range_begin / SPARSE_SLICE_BYTES, (uint64_t)n_slices);
+    const int s1 = (int)std::min<uint64_t>((range_end + SPARSE_SLICE_BYTES - 1) / SPARSE_SLICE_BYTES, (uint64_t)n_slices);
     if (s1 > s0) {
-        sparse_emit_kernel<<<s1 - s0, SPARSE_THREADS, 0, s>>>(d_fasta, w.genome, w.slices + s0, P, w.keys_a, w.ends_a,
+        sparse_emit_kernel<<<s1 - s0, SPARSE_THREADS, 0, s>>>(d_fasta, d_genomes, d_slices + s0, P, w.keys_a, w.ends_a,
                                                               w.cursor, cap);
         KM_CUDA(cudaGetLastError());
     }
@@ -263,8 +227,6 @@ static int sparse_sort_reduce_phase(const SparseWork& w, uint64_t n, int sort_bi
     KM_CUDA(cub::DeviceRadixSort::SortPairs(w.temp, tb, dk, dv, (uint64_t)n, 0, sort_bits, s));
     uint64_t* sorted_keys = dk.Current();
     uint32_t* sorted_ends = dv.Current();
-    uint64_t* uniq = dk.Alternate();
-    uint32_t* runs = dv.Alternate();
     // number of distinct k-mers first (one read of the sorted keys): the caller's buffers may be too small
     count_boundaries_kernel<<<148 * 8, 256, 0, s>>>(sorted_keys, (uint64_t)n, w.n_runs);
     KM_CUDA(cudaGetLastError());
@@ -273,21 +235,26 @@ static int sparse_sort_reduce_phase(const SparseWork& w, uint64_t n, int sort_bi
     KM_CUDA(cudaStreamSynchronize(s));
     *h_unique = nu;
     if (pending) {
-        pending->sorted_keys = sorted_keys; pending->sorted_ends = sorted_ends; pending->uniq = uniq; pending->runs = runs;
+        pending->sorted_keys = sorted_keys; pending->sorted_ends = sorted_ends;
         pending->n = n; pending->nu = nu; pending->valid = true;
     }
     if (nu > out_cap) return KMERML_OK;             // caller sizes its outputs and fetches (kmerml_sparse_fetch)
-    return sparse_copy_out(w, sorted_keys, sorted_ends, uniq, runs, n, nu, d_keys_out, d_counts_out, d_first_out, s);
+    return sparse_copy_out(w, sorted_keys, sorted_ends, n, d_keys_out, d_counts_out, d_first_out, s);
 }
 
 // Emits, sorts and reduces.  On return (after a stream sync) *h_windows / *h_unique are valid; when
 // *h_unique > out_cap nothing was written to the outputs (kmerml_sparse_fetch copies them out later).
-int run_sparse(const uint8_t* d_fasta, uint64_t nbytes, uint64_t range_begin, uint64_t range_end, int k, int min_rec,
-               bool canonical, const SparseWork& w, uint64_t cap, uint64_t* d_keys_out, uint32_t* d_counts_out, uint32_t* d_first_out, uint64_t out_cap,
-               uint64_t* h_unique, uint64_t* h_windows, SparsePending* pending, cudaStream_t s) {
+int run_sparse_in(void* workspace, const uint8_t* d_fasta, const GenomeDev* d_genomes, const Slice* d_slices, int n_slices,
+                  uint64_t range_begin, uint64_t range_end, int k, int min_rec, bool canonical, uint64_t cap,
+                  uint64_t* d_keys_out, uint32_t* d_counts_out, uint32_t* d_first_out, uint64_t out_cap, uint64_t* h_unique,
+                  uint64_t* h_windows, SparsePending* pending, cudaStream_t s) {
+    SparseWork w;
+    sparse_workspace(cap, &w, (uint8_t*)workspace);
     if (pending) pending->valid = false;
     *h_unique = 0;
-    if (int rc = sparse_emit_phase(d_fasta, nbytes, range_begin, range_end, k, min_rec, canonical, w, cap, h_windows, s)) return rc;
+    if (int rc = sparse_emit_phase(d_fasta, d_genomes, d_slices, n_slices, range_begin, range_end, k, min_rec, canonical, w,
+                                   cap, h_windows, s))
+        return rc;
     return sparse_sort_reduce_phase(w, *h_windows, 2 * k, d_keys_out, d_counts_out, d_first_out, out_cap, h_unique, pending, s);
 }
 
@@ -307,15 +274,17 @@ __global__ void owner_bounds_kernel(const uint64_t* __restrict__ keys, uint64_t 
     bounds[r] = lo;
 }
 
-int run_sparse_emit_by_owner(void* workspace, const uint8_t* d_fasta, uint64_t nbytes, uint64_t range_begin,
-                             uint64_t range_end, int k, int min_rec, bool canonical, int owner_bits, uint64_t cap,
-                             uint64_t* d_keys_out, uint32_t* d_ends_out, uint64_t out_cap, uint64_t* h_windows,
-                             uint64_t* h_owner_counts, cudaStream_t s) {
+int run_sparse_emit_by_owner(void* workspace, const uint8_t* d_fasta, const GenomeDev* d_genomes, const Slice* d_slices,
+                             int n_slices, uint64_t range_begin, uint64_t range_end, int k, int min_rec, bool canonical,
+                             int owner_bits, uint64_t cap, uint64_t* d_keys_out, uint32_t* d_ends_out, uint64_t out_cap,
+                             uint64_t* h_windows, uint64_t* h_owner_counts, cudaStream_t s) {
     SparseWork w;
-    sparse_workspace(cap, nbytes, &w, (uint8_t*)workspace);
+    sparse_workspace(cap, &w, (uint8_t*)workspace);
     const int n_owners = 1 << owner_bits;
     for (int r = 0; r < n_owners; r++) h_owner_counts[r] = 0;
-    if (int rc = sparse_emit_phase(d_fasta, nbytes, range_begin, range_end, k, min_rec, canonical, w, cap, h_windows, s)) return rc;
+    if (int rc = sparse_emit_phase(d_fasta, d_genomes, d_slices, n_slices, range_begin, range_end, k, min_rec, canonical, w,
+                                   cap, h_windows, s))
+        return rc;
     const uint64_t n = *h_windows;
     if (!n || n > out_cap) return KMERML_OK;
     uint64_t* keys = w.keys_a;
@@ -347,30 +316,20 @@ int run_sparse_reduce_windows(void* workspace, int sort_bits, const uint64_t* d_
     *h_unique = 0;
     if (!n) return KMERML_OK;
     SparseWork w;
-    sparse_workspace(n, 0, &w, (uint8_t*)workspace);
+    sparse_workspace(n, &w, (uint8_t*)workspace);
     KM_CUDA(cudaMemcpyAsync(w.keys_a, d_keys, n * 8, cudaMemcpyDeviceToDevice, s));
     KM_CUDA(cudaMemcpyAsync(w.ends_a, d_ends, n * 4, cudaMemcpyDeviceToDevice, s));
     return sparse_sort_reduce_phase(w, n, sort_bits, d_keys_out, d_counts_out, d_first_out, out_cap, h_unique, pending, s);
 }
 
-int sparse_fetch(void* workspace, uint64_t cap, uint64_t nbytes, const SparsePending& p, uint64_t* d_keys_out,
-                 uint32_t* d_counts_out, uint32_t* d_first_out, cudaStream_t s) {
+int sparse_fetch(void* workspace, const SparsePending& p, uint64_t* d_keys_out, uint32_t* d_counts_out,
+                 uint32_t* d_first_out, cudaStream_t s) {
     SparseWork w;
-    sparse_workspace(cap, nbytes, &w, (uint8_t*)workspace);
-    return sparse_copy_out(w, p.sorted_keys, p.sorted_ends, p.uniq, p.runs, p.n, p.nu, d_keys_out, d_counts_out,
-                           d_first_out, s);
+    sparse_workspace(p.cap, &w, (uint8_t*)workspace);
+    return sparse_copy_out(w, p.sorted_keys, p.sorted_ends, p.n, d_keys_out, d_counts_out, d_first_out, s);
 }
 
-size_t sparse_workspace_bytes(uint64_t cap, uint64_t nbytes) { return sparse_workspace(cap, nbytes, nullptr, nullptr); }
-
-int run_sparse_in(void* workspace, const uint8_t* d_fasta, uint64_t nbytes, uint64_t range_begin, uint64_t range_end,
-                  int k, int min_rec, bool canonical, uint64_t cap, uint64_t* d_keys_out, uint32_t* d_counts_out, uint32_t* d_first_out, uint64_t out_cap,
-                  uint64_t* h_unique, uint64_t* h_windows, SparsePending* pending, cudaStream_t s) {
-    SparseWork w;
-    sparse_workspace(cap, nbytes, &w, (uint8_t*)workspace);
-    return run_sparse(d_fasta, nbytes, range_begin, range_end, k, min_rec, canonical, w, cap, d_keys_out, d_counts_out, d_first_out, out_cap,
-                      h_unique, h_windows, pending, s);
-}
+size_t sparse_workspace_bytes(uint64_t cap) { return sparse_workspace(cap, nullptr, nullptr); }
 
 // ---- merge of partial results (multi-GPU: every rank receives the (k-mer, count, first) triples of its
 // key range from all ranks): sort by k-mer, add the counts, keep the smallest first offset.

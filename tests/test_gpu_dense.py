@@ -87,6 +87,12 @@ def test_fuzz_small():
         ks = sorted(rng.sample(range(1, 13), rng.randint(1, 4)), reverse=rng.random() < 0.3)
         mr = None if rng.random() < 0.7 else max(ks) + rng.randint(1, 10)
         check_against_oracle(datas, ks, min_record_len=mr, partition=(it % 3 != 0))
+    # at least 8 x SMs genomes: the shared-histogram paths (k <= 8) walk each genome with one CTA
+    torch = torch_mod()
+    n = 8 * torch.cuda.get_device_properties(0).multi_processor_count + 16
+    datas = [fuzz_fasta(rng) for _ in range(n)]
+    check_against_oracle(datas, [8, 3])
+    check_against_oracle(datas, [7, 2])
 
 
 def test_canonical_opt_in():
