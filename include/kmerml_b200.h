@@ -413,6 +413,50 @@ int kmerml_sketch_distance_rows(kmerml_ctx *ctx, const uint64_t *d_sketches, uin
                                 int metric, float *d_out32, double *d_out64, void *stream);
 
 /*
+ * Scaled (FracMinHash) genome sketches and their containment, Jaccard and containment ANI, for any k up to 32
+ * (Irber et al. 2022; containment ANI: Hera et al. 2023).  Unlike a bottom-s sketch, a scaled sketch grows with the
+ * genome, so a small genome (a plasmid, a MAG) can be compared with a large one by containment.
+ *
+ * kmerml_fmh_batch: the scaled sketch of every genome of a batch laid out as for kmerml_sketch_batch, with the same
+ * keys, window rules, KMERML_FLAG_CANONICAL, min_record_len (0 means k) and hash h = fmix64(key + 0x9E3779B97F4A7C15 *
+ * (seed + 1)).  The sketch of genome g is every distinct hash h <= T = floor((2^64 - 1) / scale) of its k-mers,
+ * ascending (scale 1: every distinct k-mer).  With equal k, seed and canonical flag, its first s values are the
+ * bottom-s sketch of kmerml_sketch_batch whenever it holds at least s values.  The sketches come out in genome order
+ * as CSR: genome g is d_hashes[off[g] .. off[g + 1]), off = d_sketch_offsets (n_genomes + 1 values, always written).
+ * *h_total always receives off[n_genomes]; when it exceeds out_cap the hashes are not written: call
+ * kmerml_fmh_fetch with outputs that large.  Every window is hashed once; the windows at or below T are stored in a
+ * region of about twice the expected count per genome, and a genome whose region overflowed (tandem repeats of a
+ * low-hash k-mer) runs again with a region of exactly its stored windows.  A genome whose windows at or below T
+ * exceed 2^31 - 1 returns KMERML_ERR_RANGE (scale 1 on a genome of more than 2 Gbp: use a larger scale).
+ * scale >= 1.  Synchronous.
+ *
+ * kmerml_fmh_fetch: the result of the last kmerml_fmh_batch call of this context, copied out of the context without
+ * walking the FASTA again (out_cap >= its total).  Later calls of other functions do not disturb it.  Synchronous.
+ *
+ * kmerml_fmh_compare: for every query q < n_q and reference r < n_r (two CSR sets of sketches of kmerml_fmh_batch,
+ * made with the same k, scale, seed and canonical flag -- not checked here; the two sets may be the same pointers),
+ * x = |Q n R| exactly, and the metric in float64 from x, |Q| and |R|: KMERML_FMH_CONTAINMENT x / |Q|,
+ * KMERML_FMH_MAX_CONTAINMENT x / min(|Q|, |R|), KMERML_FMH_JACCARD x / (|Q| + |R| - x), KMERML_FMH_CONTAINMENT_ANI
+ * (x / |Q|)^(1/k), KMERML_FMH_MAX_CONTAINMENT_ANI (x / min(|Q|, |R|))^(1/k); 0 when x = 0 (so also when a
+ * denominator is 0).  All are similarities.  Row q, column r of d_intersections (uint32), d_out32 and d_out64
+ * (n_q x n_r each, any of them NULL, not all three) receive x and the metric (rounded for float32).  Asynchronous on
+ * `stream`; the result of one query does not depend on the others, so a block of query rows is bit-identical to
+ * the same rows of the whole matrix.
+ */
+#define KMERML_FMH_CONTAINMENT 0
+#define KMERML_FMH_MAX_CONTAINMENT 1
+#define KMERML_FMH_JACCARD 2
+#define KMERML_FMH_CONTAINMENT_ANI 3
+#define KMERML_FMH_MAX_CONTAINMENT_ANI 4
+int kmerml_fmh_batch(kmerml_ctx *ctx, const uint8_t *d_fasta, const uint64_t *h_offsets, int n_genomes, int k,
+                     int min_record_len, unsigned flags, uint64_t scale, uint64_t seed, uint64_t *d_hashes,
+                     uint64_t out_cap, uint64_t *d_sketch_offsets, uint64_t *h_total, void *stream);
+int kmerml_fmh_fetch(kmerml_ctx *ctx, uint64_t *d_hashes, uint64_t out_cap, uint64_t *d_sketch_offsets, void *stream);
+int kmerml_fmh_compare(kmerml_ctx *ctx, const uint64_t *d_q_hashes, const uint64_t *d_q_offsets, int n_q,
+                       const uint64_t *d_r_hashes, const uint64_t *d_r_offsets, int n_r, int k, int metric,
+                       uint32_t *d_intersections, float *d_out32, double *d_out64, void *stream);
+
+/*
  * Measurement hooks (bench.py): with profiling enabled every kernel the library
  * launches is bracketed by CUDA events on the launching stream.  kmerml_profile_read
  * synchronises those events and returns the accumulated device time per kernel family

@@ -21,6 +21,11 @@ MAX_K = 32
 SKETCH_MAX = 16384
 SKETCH_METRIC_MASH = 0
 SKETCH_METRIC_JACCARD = 1
+FMH_CONTAINMENT = 0
+FMH_MAX_CONTAINMENT = 1
+FMH_JACCARD = 2
+FMH_CONTAINMENT_ANI = 3
+FMH_MAX_CONTAINMENT_ANI = 4
 
 _lib = None
 
@@ -96,6 +101,9 @@ def load():
     L.kmerml_distance_rows_planes.argtypes = [vp, vp, u64, i32, i32, u64, vp, i32, i32, i32, vp, vp, vp]
     L.kmerml_sketch_batch.argtypes = [vp, vp, vp, i32, i32, i32, u32, i32, u64, vp, u64, vp, vp]
     L.kmerml_sketch_distance_rows.argtypes = [vp, vp, u64, vp, i32, i32, i32, i32, i32, i32, vp, vp, vp]
+    L.kmerml_fmh_batch.argtypes = [vp, vp, vp, i32, i32, i32, u32, u64, u64, vp, u64, vp, p64, vp]
+    L.kmerml_fmh_fetch.argtypes = [vp, vp, u64, vp, vp]
+    L.kmerml_fmh_compare.argtypes = [vp, vp, vp, i32, vp, vp, i32, i32, i32, vp, vp, vp, vp]
     L.kmerml_profile_enable.argtypes = [vp, i32]
     L.kmerml_profile_read.argtypes = [vp, ctypes.POINTER(Profile), i32]
     for name in EXPORTS:
@@ -119,6 +127,7 @@ EXPORTS = [
     "kmerml_parse_kmer_lines", "kmerml_feature_keys", "kmerml_feature_line_lengths", "kmerml_feature_write_lines",
     "kmerml_emit_sparse_range", "kmerml_reduce_sparse_windows",
     "kmerml_sketch_batch", "kmerml_sketch_distance_rows",
+    "kmerml_fmh_batch", "kmerml_fmh_fetch", "kmerml_fmh_compare",
 ]
 
 

@@ -116,6 +116,10 @@ struct kmerml_ctx {
     km::Workspace ws[8];                          // [0]: device-resident calls; [0..n): the host pipeline's slots
     int host_slots = 6;                           // (measured: 2 slots 29.8, 3: 39.4, 4: 34.9, 6: 45.3, 8: 44.7 Gbp/s for the compact call, 60 C2 genomes)
     km::SparsePending sparse_pending;             // kmerml_count_sparse -> kmerml_sparse_fetch
+    km::DevBuf fmh_kept;                          // kmerml_fmh_batch -> kmerml_fmh_fetch: the kept values of every round,
+    km::DevBuf fmh_index;                         // where each genome's begin there | the CSR offsets
+    int fmh_n = -1;                               // genomes of that result (< 0: none)
+    uint64_t fmh_total = 0;
     km::HostPool* host_pool = nullptr;            // host threads that widen the narrow D2H format
     cudaStream_t last_stream = nullptr;           // ws[0] is scratch shared by every device-resident call: a call on
     bool last_stream_valid = false;               // another stream than the one before waits for that one (order_stream)
@@ -683,6 +687,8 @@ int kmerml_ctx_destroy(kmerml_ctx* ctx) {
     DeviceGuard guard(ctx->device);
     cudaDeviceSynchronize();
     for (auto& w : ctx->ws) w.release();
+    ctx->fmh_kept.release();
+    ctx->fmh_index.release();
     if (ctx->order_ev) cudaEventDestroy(ctx->order_ev);
     if (ctx->host_pool) host_pool_destroy(ctx->host_pool);
     for (auto& r : ctx->recs) { cudaEventDestroy(r.a); cudaEventDestroy(r.b); }
@@ -1579,9 +1585,32 @@ static uint64_t sketch_region(uint64_t bytes, uint64_t tau) {
 
 constexpr uint64_t SKETCH_ROUND_SLOTS = 1ull << 28;     // survivor slots of one round (2 GiB, twice: sort in / out)
 
-static int sketch_batch_core(kmerml_ctx* ctx, const uint8_t* d_fasta, const uint64_t* h_offsets, int n, int k, int min_rec,
-                             bool canonical, int sketch_size, uint64_t seed, uint64_t* d_sketches, uint64_t stride,
-                             uint32_t* d_filled, cudaStream_t s) {
+// One emit round of sketch_rounds, as the caller's stage sees it: the genomes h_active[0 .. n_active) (buffer order;
+// the same on the device at d_active) with their thresholds, regions and survivor counts at d_sg[genome], the
+// survivors of each region sorted into d_sorted, d_seg the sort's 2 n_active int segment bounds (begins | ends),
+// n_active status words (device d_status, pinned host h_status) and the stage's own scratch.
+struct SketchRound {
+    int n_active;
+    const int* h_active;
+    const int* d_active;
+    const SketchGenome* d_sg;
+    const int* d_seg;
+    uint64_t slots;
+    const uint64_t* d_sorted;
+    void* scratch;
+    uint32_t* d_status;
+    uint32_t* h_status;
+};
+
+// The round loop of the sketch calls.  Genomes still pending, in buffer order, are packed into rounds of at most
+// SKETCH_ROUND_SLOTS survivor slots (at least one genome); a round walks their slices with sketch_emit_kernel (genome
+// g: threshold tau[g], region of cap[g] slots) and sorts every region.  `stage_bytes(slots, n_active)` is the scratch
+// the caller's stage needs; `stage` launches its selection, waits for it and lists the genomes to run again, for
+// which it has set tau and cap anew.
+static int sketch_rounds(kmerml_ctx* ctx, const uint8_t* d_fasta, const uint64_t* h_offsets, int n, int k, int min_rec,
+                         bool canonical, uint64_t seed, std::vector<uint64_t>& tau, std::vector<uint64_t>& cap,
+                         const std::function<size_t(uint64_t, int)>& stage_bytes,
+                         const std::function<int(const SketchRound&, std::vector<int>&)>& stage, cudaStream_t s) {
     // the slice table of a round holds at most the slices of every genome
     std::vector<uint64_t> slice_bytes(n, SPARSE_SLICE_BYTES);
     std::vector<Slice> plan;
@@ -1597,17 +1626,10 @@ static int sketch_batch_core(kmerml_ctx* ctx, const uint8_t* d_fasta, const uint
     if ((rc = t.open()) || (rc = put_walk(t, walk, d_fasta, h_offsets, nullptr, s))) return rc;
     const GenomeDev* d_genomes = t.dev<GenomeDev>(walk.genomes);
     const Slice* d_slices = t.dev<Slice>(walk.slices);
-    uint32_t* h_status = t.host<uint32_t>(at_status);
     Workspace& ws = ctx->ws[0];
 
-    std::vector<uint64_t> tau(n), cap(n);
     std::vector<int> pending(n);
-    for (int g = 0; g < n; g++) {
-        const uint64_t bytes = h_offsets[g + 1] - h_offsets[g];
-        tau[g] = sketch_first_tau(bytes, sketch_size);
-        cap[g] = sketch_region(bytes, tau[g]);
-        pending[g] = g;
-    }
+    for (int g = 0; g < n; g++) pending[g] = g;
     while (!pending.empty()) {
         // one round: the pending genomes (in buffer order) whose regions fit SKETCH_ROUND_SLOTS, at least one
         SketchGenome* h_sg = t.fill<SketchGenome>(at_sg, (size_t)n * sizeof(SketchGenome));
@@ -1630,43 +1652,165 @@ static int sketch_batch_core(kmerml_ctx* ctx, const uint8_t* d_fasta, const uint
         t.fill<int>(at_active, (size_t)n_round * 4);
         if ((rc = plan_slices(h_offsets, n, slice_bytes.data(), SPARSE_TILE_BYTES, 0, 0, plan, first))) return rc;
         const size_t region_bytes = align_up(std::max<uint64_t>(slots, 1) * 8, 256);
-        const size_t temp_bytes = sketch_sort_temp_bytes((int)slots, n_round);
-        if ((rc = ws.part.ensure(2 * region_bytes + temp_bytes))) return rc;
+        const size_t temp_bytes = align_up(sketch_sort_temp_bytes((int)slots, n_round), 256);
+        if ((rc = ws.part.ensure(2 * region_bytes + temp_bytes + stage_bytes(slots, n_round)))) return rc;
         uint64_t* d_regions = (uint64_t*)ws.part.p;
         uint64_t* d_sorted = (uint64_t*)((uint8_t*)ws.part.p + region_bytes);
         void* d_temp = (uint8_t*)ws.part.p + 2 * region_bytes;
         {
-            Prof pr(ctx, s, 3, 7);      // the three slice-table kernels, emit, segments, sort, select
+            Prof pr(ctx, s, 3, 6);      // the three slice-table kernels, emit, segments, sort
             rc = put_walk(t, walk, d_fasta, nullptr, &plan, s);
             if (!rc) rc = launch_sketch_emit(d_fasta, d_genomes, d_slices, walk.n_slices, k, min_rec, canonical, seed, t.dev<SketchGenome>(at_sg),
                                              d_regions, s);
-            if (!rc) rc = launch_sketch_select(t.dev<SketchGenome>(at_sg), t.dev<int>(at_active), n_round, t.dev<int>(at_seg), (int)slots, d_regions, d_sorted, d_temp,
-                                               temp_bytes, sketch_size, d_sketches, stride, d_filled, t.dev<uint32_t>(at_status), s);
+            if (!rc) rc = launch_sketch_sort(t.dev<SketchGenome>(at_sg), t.dev<int>(at_active), n_round, t.dev<int>(at_seg), (int)slots,
+                                             d_regions, d_sorted, d_temp, temp_bytes, s);
         }
         if (rc) return rc;
-        KM_CUDA(cudaMemcpyAsync(h_status, t.dev<uint32_t>(at_status), (size_t)n_round * 4, cudaMemcpyDeviceToHost, s));
-        KM_CUDA(cudaStreamSynchronize(s));
-        // run again: too few distinct hashes below tau -> 16 tau (saturating at every window); overflow -> one slot
-        // per byte.  Every window with one slot per byte cannot fail, so the loop ends.
+        const SketchRound round{n_round, h_active, t.dev<int>(at_active), t.dev<SketchGenome>(at_sg), t.dev<int>(at_seg), slots,
+                                d_sorted, (uint8_t*)d_temp + temp_bytes, t.dev<uint32_t>(at_status), t.host<uint32_t>(at_status)};
         std::vector<int> next;
-        for (int i = 0; i < n_round; i++) {
-            const int g = h_active[i];
-            const uint64_t bytes = h_offsets[g + 1] - h_offsets[g];
-            if (h_status[i] == SKETCH_MORE) {
-                tau[g] = tau[g] > ~0ull / 16 ? ~0ull : tau[g] * 16;
-                cap[g] = sketch_region(bytes, tau[g]);
-            } else if (h_status[i] == SKETCH_OVERFLOW) {
-                cap[g] = bytes;
-            } else {
-                continue;
-            }
-            next.push_back(g);
-        }
+        if ((rc = stage(round, next))) return rc;
         next.insert(next.end(), pending.begin() + n_round, pending.end());
         std::sort(next.begin(), next.end());            // the slice table stays in buffer order
         pending.swap(next);
     }
     return KMERML_OK;
+}
+
+static int sketch_batch_core(kmerml_ctx* ctx, const uint8_t* d_fasta, const uint64_t* h_offsets, int n, int k, int min_rec,
+                             bool canonical, int sketch_size, uint64_t seed, uint64_t* d_sketches, uint64_t stride,
+                             uint32_t* d_filled, cudaStream_t s) {
+    std::vector<uint64_t> tau(n), cap(n);
+    for (int g = 0; g < n; g++) {
+        const uint64_t bytes = h_offsets[g + 1] - h_offsets[g];
+        tau[g] = sketch_first_tau(bytes, sketch_size);
+        cap[g] = sketch_region(bytes, tau[g]);
+    }
+    auto select = [&](const SketchRound& r, std::vector<int>& again) {
+        {
+            Prof pr(ctx, s, 3, 1);
+            int rc = launch_sketch_select(r.d_sg, r.d_active, r.n_active, r.d_sorted, sketch_size, d_sketches, stride,
+                                          d_filled, r.d_status, s);
+            if (rc) return rc;
+        }
+        KM_CUDA(cudaMemcpyAsync(r.h_status, r.d_status, (size_t)r.n_active * 4, cudaMemcpyDeviceToHost, s));
+        KM_CUDA(cudaStreamSynchronize(s));
+        // run again: too few distinct hashes below tau -> 16 tau (saturating at every window); overflow -> one slot
+        // per byte.  Every window with one slot per byte cannot fail, so the loop ends.
+        for (int i = 0; i < r.n_active; i++) {
+            const int g = r.h_active[i];
+            const uint64_t bytes = h_offsets[g + 1] - h_offsets[g];
+            if (r.h_status[i] == SKETCH_MORE) {
+                tau[g] = tau[g] > ~0ull / 16 ? ~0ull : tau[g] * 16;
+                cap[g] = sketch_region(bytes, tau[g]);
+            } else if (r.h_status[i] == SKETCH_OVERFLOW) {
+                cap[g] = bytes;
+            } else {
+                continue;
+            }
+            again.push_back(g);
+        }
+        return KMERML_OK;
+    };
+    return sketch_rounds(ctx, d_fasta, h_offsets, n, k, min_rec, canonical, seed, tau, cap,
+                         [](uint64_t, int) { return (size_t)0; }, select, s);
+}
+
+// Grows `b` to `bytes`, keeping its first `used` bytes (`s` is idle when this is called).
+static int grow_keeping(DevBuf& b, size_t used, size_t bytes, cudaStream_t s) {
+    if (bytes <= b.cap) return KMERML_OK;
+    DevBuf nb;
+    int rc = nb.ensure(std::max(bytes, b.cap * 2));
+    if (rc) return rc;
+    if (used) KM_CUDA(cudaMemcpyAsync(nb.p, b.p, used, cudaMemcpyDeviceToDevice, s));
+    KM_CUDA(cudaStreamSynchronize(s));
+    b.release();
+    b = nb;
+    return KMERML_OK;
+}
+
+// Scaled sketches: the rounds of sketch_rounds with tau = T for every genome.  After each round the distinct values of
+// the genomes that did not overflow are appended to ctx->fmh_kept; at the end the CSR offsets and the gather into the
+// caller's buffer put them in genome order.
+static int fmh_batch_core(kmerml_ctx* ctx, const uint8_t* d_fasta, const uint64_t* h_offsets, int n, int k, int min_rec,
+                          bool canonical, uint64_t scale, uint64_t seed, uint64_t* d_hashes, uint64_t out_cap,
+                          uint64_t* d_offsets, uint64_t* h_total, cudaStream_t s) {
+    const uint64_t T = ~0ull / scale;
+    const auto too_large = [&](int g) {
+        return fail(KMERML_ERR_RANGE, "genome " + std::to_string(g) + ": its k-mers at or below the threshold of scale " +
+                                          std::to_string(scale) + " may exceed 2^31 - 1; use a larger scale");
+    };
+    std::vector<uint64_t> tau(n, T), cap(n), begin(n, 0), size(n, 0);
+    for (int g = 0; g < n; g++) {
+        cap[g] = sketch_region(h_offsets[g + 1] - h_offsets[g], T);
+        if (cap[g] > 0x7fffffffull) return too_large(g);
+    }
+    ctx->fmh_n = -1;
+    uint64_t kept = 0;                                 // values in ctx->fmh_kept
+    auto scratch = [](uint64_t slots, int n_active) {
+        return 2 * align_up(std::max<uint64_t>(slots, 1) * 4, 256) + align_up(fmh_scan_temp_bytes((int)slots), 256) +
+               (size_t)n_active * sizeof(FmhRoundGenome);
+    };
+    auto distinct = [&](const SketchRound& r, std::vector<int>& again) {
+        const size_t flag_bytes = align_up(std::max<uint64_t>(r.slots, 1) * 4, 256);
+        const size_t temp_bytes = align_up(fmh_scan_temp_bytes((int)r.slots), 256);
+        uint32_t* d_flags = (uint32_t*)r.scratch;
+        uint32_t* d_pos = (uint32_t*)((uint8_t*)r.scratch + flag_bytes);
+        void* d_temp = (uint8_t*)r.scratch + 2 * flag_bytes;
+        FmhRoundGenome* d_out = (FmhRoundGenome*)((uint8_t*)d_temp + temp_bytes);
+        {
+            Prof pr(ctx, s, 3, 3);
+            int rc = launch_fmh_distinct(r.d_sg, r.d_active, r.n_active, r.d_seg, (int)r.slots, r.d_sorted, d_flags, d_pos,
+                                         d_temp, temp_bytes, d_out, s);
+            if (rc) return rc;
+        }
+        std::vector<FmhRoundGenome> out(r.n_active);
+        KM_CUDA(cudaMemcpyAsync(out.data(), d_out, out.size() * sizeof(FmhRoundGenome), cudaMemcpyDeviceToHost, s));
+        KM_CUDA(cudaStreamSynchronize(s));
+        uint64_t round_kept = 0;
+        for (int i = 0; i < r.n_active; i++) {
+            const int g = r.h_active[i];
+            if (out[i].count > cap[g]) {               // overflow: the cursor counted every survivor
+                if (out[i].count > 0x7fffffffull) return too_large(g);
+                cap[g] = out[i].count;
+                again.push_back(g);
+                continue;
+            }
+            begin[g] = kept + out[i].first;
+            size[g] = out[i].distinct;
+            round_kept += out[i].distinct;
+        }
+        if (!round_kept) return KMERML_OK;
+        int rc = grow_keeping(ctx->fmh_kept, kept * 8, (kept + round_kept) * 8, s);
+        if (!rc) {
+            Prof pr(ctx, s, 3, 1);
+            rc = launch_fmh_scatter(r.d_sorted, d_flags, d_pos, (int)r.slots, (uint64_t*)ctx->fmh_kept.p + kept, s);
+        }
+        kept += round_kept;
+        return rc;
+    };
+    int rc = sketch_rounds(ctx, d_fasta, h_offsets, n, k, min_rec, canonical, seed, tau, cap, scratch, distinct, s);
+    if (rc) return rc;
+    // the index: begin | CSR offsets, uploaded from pageable memory (the call is synchronous)
+    std::vector<uint64_t> index(2 * (size_t)n + 1);
+    for (int g = 0; g < n; g++) {
+        index[g] = begin[g];
+        index[n + g + 1] = index[n + g] + size[g];
+    }
+    if ((rc = ctx->fmh_index.ensure(index.size() * 8))) return rc;
+    KM_CUDA(cudaMemcpyAsync(ctx->fmh_index.p, index.data(), index.size() * 8, cudaMemcpyHostToDevice, s));
+    KM_CUDA(cudaStreamSynchronize(s));
+    ctx->fmh_n = n;
+    ctx->fmh_total = index[2 * (size_t)n];
+    *h_total = ctx->fmh_total;
+    KM_CUDA(cudaMemcpyAsync(d_offsets, (uint64_t*)ctx->fmh_index.p + n, (size_t)(n + 1) * 8, cudaMemcpyDeviceToDevice, s));
+    if (ctx->fmh_total <= out_cap) {
+        ctx->launches += 1;
+        rc = launch_fmh_gather((const uint64_t*)ctx->fmh_kept.p, (const uint64_t*)ctx->fmh_index.p,
+                               (const uint64_t*)ctx->fmh_index.p + n, n, ctx->fmh_total, d_hashes, s);
+    }
+    if (!rc) KM_CUDA(cudaStreamSynchronize(s));
+    return rc;
 }
 
 int kmerml_sketch_batch(kmerml_ctx* ctx, const uint8_t* d_fasta, const uint64_t* h_offsets, int n_genomes, int k,
@@ -1708,6 +1852,66 @@ int kmerml_sketch_distance_rows(kmerml_ctx* ctx, const uint64_t* d_sketches, uin
     ctx->launches += 1;
     return launch_sketch_distance(d_sketches, sketch_stride, d_filled, n, sketch_size, k, row_begin, row_end, metric,
                                   d_out32, d_out64, (cudaStream_t)stream);
+}
+
+int kmerml_fmh_batch(kmerml_ctx* ctx, const uint8_t* d_fasta, const uint64_t* h_offsets, int n_genomes, int k,
+                     int min_record_len, unsigned flags, uint64_t scale, uint64_t seed, uint64_t* d_hashes, uint64_t out_cap,
+                     uint64_t* d_sketch_offsets, uint64_t* h_total, void* stream) {
+    if (!ctx) return fail(KMERML_ERR_ARG, "ctx is null");
+    if (k < 1 || k > KMERML_MAX_K) return fail(KMERML_ERR_ARG, "k must be in 1..32");
+    if (scale < 1) return fail(KMERML_ERR_ARG, "scale must be >= 1");
+    if (n_genomes < 0) return fail(KMERML_ERR_ARG, "n_genomes < 0");
+    const int min_rec = min_record_len > 0 ? min_record_len : k;
+    if (min_rec < k) return fail(KMERML_ERR_ARG, "min_record_len must be >= k");
+    if (!h_offsets || !d_sketch_offsets || !h_total || (out_cap && !d_hashes)) return fail(KMERML_ERR_ARG, "null pointer argument");
+    if (int rc = check_batch(d_fasta, h_offsets, n_genomes, false)) return rc;
+    DeviceGuard guard(ctx->device);
+    if (!guard.ok) return fail(KMERML_ERR_CUDA, "cudaSetDevice failed");
+    if (int orc = order_stream(ctx, (cudaStream_t)stream)) return orc;
+    return fmh_batch_core(ctx, d_fasta, h_offsets, n_genomes, k, min_rec, (flags & KMERML_FLAG_CANONICAL) != 0, scale, seed,
+                          d_hashes, out_cap, d_sketch_offsets, h_total, (cudaStream_t)stream);
+}
+
+int kmerml_fmh_fetch(kmerml_ctx* ctx, uint64_t* d_hashes, uint64_t out_cap, uint64_t* d_sketch_offsets, void* stream) {
+    if (!ctx || !d_sketch_offsets || (out_cap && !d_hashes)) return fail(KMERML_ERR_ARG, "null pointer argument");
+    if (ctx->fmh_n < 0) return fail(KMERML_ERR_ARG, "no scaled-sketch result to fetch");
+    if (out_cap < ctx->fmh_total) return fail(KMERML_ERR_ARG, "out_cap is smaller than the total of the sketches");
+    DeviceGuard guard(ctx->device);
+    if (!guard.ok) return fail(KMERML_ERR_CUDA, "cudaSetDevice failed");
+    if (int orc = order_stream(ctx, (cudaStream_t)stream)) return orc;
+    cudaStream_t s = (cudaStream_t)stream;
+    const int n = ctx->fmh_n;
+    const uint64_t* index = (const uint64_t*)ctx->fmh_index.p;
+    KM_CUDA(cudaMemcpyAsync(d_sketch_offsets, index + n, (size_t)(n + 1) * 8, cudaMemcpyDeviceToDevice, s));
+    ctx->launches += 1;
+    int rc = launch_fmh_gather((const uint64_t*)ctx->fmh_kept.p, index, index + n, n, ctx->fmh_total, d_hashes, s);
+    if (!rc) KM_CUDA(cudaStreamSynchronize(s));
+    return rc;
+}
+
+int kmerml_fmh_compare(kmerml_ctx* ctx, const uint64_t* d_q_hashes, const uint64_t* d_q_offsets, int n_q,
+                       const uint64_t* d_r_hashes, const uint64_t* d_r_offsets, int n_r, int k, int metric,
+                       uint32_t* d_intersections, float* d_out32, double* d_out64, void* stream) {
+    if (!ctx) return fail(KMERML_ERR_ARG, "ctx is null");
+    if (k < 1 || k > KMERML_MAX_K) return fail(KMERML_ERR_ARG, "k must be in 1..32");
+    if (metric < KMERML_FMH_CONTAINMENT || metric > KMERML_FMH_MAX_CONTAINMENT_ANI)
+        return fail(KMERML_ERR_ARG, "unknown scaled-sketch metric");
+    if (n_q < 0 || n_r < 0) return fail(KMERML_ERR_ARG, "n_q and n_r must be >= 0");
+    if (!n_q || !n_r) return KMERML_OK;
+    if (!d_q_hashes || !d_q_offsets || !d_r_hashes || !d_r_offsets || (!d_intersections && !d_out32 && !d_out64))
+        return fail(KMERML_ERR_ARG, "null pointer argument");
+    DeviceGuard guard(ctx->device);
+    if (!guard.ok) return fail(KMERML_ERR_CUDA, "cudaSetDevice failed");
+    Workspace& ws = ctx->ws[0];
+    if (int orc = order_stream(ctx, (cudaStream_t)stream)) return orc;
+    // workspace: the reference chunk table | the intersections when the caller does not want them
+    const size_t table = align_up(fmh_compare_workspace(n_r), 256);
+    int rc = ws.misc.ensure(table + (d_intersections ? 0 : (size_t)n_q * n_r * 4));
+    if (rc) return rc;
+    uint32_t* inter = d_intersections ? d_intersections : (uint32_t*)((uint8_t*)ws.misc.p + table);
+    ctx->launches += 3;
+    return launch_fmh_compare(d_q_hashes, d_q_offsets, n_q, d_r_hashes, d_r_offsets, n_r, k, metric, ctx->sm_count, ws.misc.p,
+                              inter, d_out32, d_out64, (cudaStream_t)stream);
 }
 
 // NCCL through the process that called us (no link-time dependency): the four entry points the exchange needs.

@@ -200,12 +200,33 @@ inline uint64_t sketch_seed_add(uint64_t seed) { return 0x9E3779B97F4A7C15ull * 
 int launch_sketch_emit(const uint8_t* d_fasta, const GenomeDev* d_genomes, const Slice* d_slices, int n_slices, int k,
                        int min_rec, bool canonical, uint64_t seed, SketchGenome* d_sg, uint64_t* d_regions, cudaStream_t s);
 size_t sketch_sort_temp_bytes(int n_items, int n_segments);
-// d_seg: 2 * n_active ints of scratch; d_status[i] is the status of genome d_active[i]
-int launch_sketch_select(const SketchGenome* d_sg, const int* d_active, int n_active, int* d_seg, int n_items,
-                         const uint64_t* d_regions, uint64_t* d_sorted, void* temp, size_t temp_bytes, int sketch_size,
-                         uint64_t* d_sketches, uint64_t stride, uint32_t* d_filled, uint32_t* d_status, cudaStream_t s);
+// d_seg: 2 * n_active ints (segment begins | ends), filled here; every active genome's region sorted into d_sorted
+int launch_sketch_sort(const SketchGenome* d_sg, const int* d_active, int n_active, int* d_seg, int n_items,
+                       const uint64_t* d_regions, uint64_t* d_sorted, void* temp, size_t temp_bytes, cudaStream_t s);
+// d_status[i] is the status of genome d_active[i]
+int launch_sketch_select(const SketchGenome* d_sg, const int* d_active, int n_active, const uint64_t* d_sorted,
+                         int sketch_size, uint64_t* d_sketches, uint64_t stride, uint32_t* d_filled, uint32_t* d_status,
+                         cudaStream_t s);
 int launch_sketch_distance(const uint64_t* d_sketches, uint64_t stride, const uint32_t* d_filled, int n, int sketch_size,
                            int k, int row_begin, int row_end, int metric, float* d_out32, double* d_out64, cudaStream_t s);
+// scaled sketches: per active genome of a sorted round, its survivors (above its region's cap: overflow), the rank of
+// its first distinct value among the round's kept values and how many it keeps
+struct FmhRoundGenome {
+    unsigned long long count, first, distinct;
+};
+size_t fmh_scan_temp_bytes(int n_items);
+// d_flags, d_pos: n_items words each; d_seg as launch_sketch_sort left it
+int launch_fmh_distinct(const SketchGenome* d_sg, const int* d_active, int n_active, const int* d_seg, int n_items,
+                        const uint64_t* d_sorted, uint32_t* d_flags, uint32_t* d_pos, void* temp, size_t temp_bytes,
+                        FmhRoundGenome* d_out, cudaStream_t s);
+int launch_fmh_scatter(const uint64_t* d_sorted, const uint32_t* d_flags, const uint32_t* d_pos, int n_items, uint64_t* d_out,
+                       cudaStream_t s);
+int launch_fmh_gather(const uint64_t* d_kept, const uint64_t* d_begin, const uint64_t* d_offsets, int n, uint64_t total,
+                      uint64_t* d_out, cudaStream_t s);
+size_t fmh_compare_workspace(int n_r);
+int launch_fmh_compare(const uint64_t* d_qh, const uint64_t* d_q_off, int n_q, const uint64_t* d_rh, const uint64_t* d_r_off,
+                       int n_r, int k, int metric, int sm_count, void* workspace, uint32_t* d_inter, float* d_out32,
+                       double* d_out64, cudaStream_t s);
 
 // ---- k{k}.txt text (format.cu) --------------------------------------------------
 size_t format_workspace_bytes(uint64_t n_bins, uint64_t max_lines);

@@ -11,6 +11,17 @@
 //                           distinct survivors below tau (run again with a larger tau), or region overflow (run again
 //                           with a region of one slot per byte).  The host loop is kmerml_sketch_batch (api.cu).
 //   sketch_distance_kernel  rows [row_begin, row_end) x all n columns of the distance matrix, exact and symmetric.
+//
+// Scaled (FracMinHash) sketches (Irber et al. 2022) keep every distinct hash <= T = (2^64 - 1) / scale, so their size
+// grows with the genome and one genome's containment in another can be estimated.  They reuse the emitter and the
+// segmented sort with tau = T for every genome (the same host round loop, sketch_rounds in api.cu), then
+//   fmh_flag_kernel + CUB scan + fmh_round_kernel   which sorted slots are distinct values, and where each genome's
+//                           values go among the round's kept values; a region overflow runs again with exactly the
+//                           survivors the cursor counted
+//   fmh_scatter_kernel      the kept values of a round, appended to a buffer of the context
+//   fmh_gather_kernel       that buffer in genome order, as CSR
+//   fmh_intersect_kernel    exact |Q n R| of every (query, reference) pair of two sets of scaled sketches, and
+//   fmh_metric_kernel       containment, max-containment, Jaccard or containment ANI (Hera et al. 2023) from it.
 #include <cub/cub.cuh>
 
 #include "sparse_walk.cuh"
@@ -129,9 +140,8 @@ size_t sketch_sort_temp_bytes(int n_items, int n_segments) {
     return t;
 }
 
-int launch_sketch_select(const SketchGenome* d_sg, const int* d_active, int n_active, int* d_seg, int n_items,
-                         const uint64_t* d_regions, uint64_t* d_sorted, void* temp, size_t temp_bytes, int sketch_size,
-                         uint64_t* d_sketches, uint64_t stride, uint32_t* d_filled, uint32_t* d_status, cudaStream_t s) {
+int launch_sketch_sort(const SketchGenome* d_sg, const int* d_active, int n_active, int* d_seg, int n_items,
+                       const uint64_t* d_regions, uint64_t* d_sorted, void* temp, size_t temp_bytes, cudaStream_t s) {
     if (n_active <= 0) return KMERML_OK;
     int* seg_begin = d_seg;
     int* seg_end = d_seg + n_active;
@@ -140,6 +150,13 @@ int launch_sketch_select(const SketchGenome* d_sg, const int* d_active, int n_ac
     size_t tb = temp_bytes;
     KM_CUDA(cub::DeviceSegmentedSort::SortKeys(temp, tb, d_regions, d_sorted, n_items, n_active, (const int*)seg_begin,
                                                (const int*)seg_end, s));
+    return KMERML_OK;
+}
+
+int launch_sketch_select(const SketchGenome* d_sg, const int* d_active, int n_active, const uint64_t* d_sorted,
+                         int sketch_size, uint64_t* d_sketches, uint64_t stride, uint32_t* d_filled, uint32_t* d_status,
+                         cudaStream_t s) {
+    if (n_active <= 0) return KMERML_OK;
     sketch_select_kernel<<<n_active, SELECT_THREADS, 0, s>>>(d_sorted, d_sg, d_active, sketch_size, d_sketches, stride,
                                                              d_filled, d_status);
     KM_CUDA(cudaGetLastError());
@@ -222,6 +239,258 @@ int launch_sketch_distance(const uint64_t* d_sketches, uint64_t stride, const ui
     sketch_distance_kernel<<<grid, SKD_THREADS, smem, s>>>(d_sketches, stride, d_filled, n, sketch_size, k, row_begin,
                                                            row_end, metric, d_out32, d_out64);
     KM_CUDA(cudaGetLastError());
+    return KMERML_OK;
+}
+
+// ---- scaled (FracMinHash) sketches ------------------------------------------------------------------------------
+// A sorted round keeps slot i when it is a distinct value of a genome whose region did not overflow: the first slot of
+// the genome's segment, or one that differs from the slot before it.  The genome of slot i is the last active genome
+// whose segment begins at or before i (segments ascend with the active index; empty ones included).
+__global__ void fmh_flag_kernel(const uint64_t* __restrict__ sorted, const SketchGenome* __restrict__ sg,
+                                const int* __restrict__ active, const int* __restrict__ seg_begin,
+                                const int* __restrict__ seg_end, int n_active, int n_items, uint32_t* flags) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n_items) return;
+    int lo = 0, hi = n_active;
+    while (lo < hi) {
+        const int mid = (lo + hi) >> 1;
+        if (seg_begin[mid] <= i) lo = mid + 1; else hi = mid;
+    }
+    const int j = lo - 1;                             // >= 0: the first segment begins at slot 0
+    const SketchGenome me = sg[active[j]];
+    flags[i] = (i < seg_end[j] && me.count <= me.cap && (i == seg_begin[j] || sorted[i] != sorted[i - 1])) ? 1u : 0u;
+}
+
+// Per active genome: its survivors, the rank of its first distinct value among the round's kept values, and how many
+// it keeps (0 after an overflow).
+__global__ void fmh_round_kernel(const SketchGenome* __restrict__ sg, const int* __restrict__ active,
+                                 const int* __restrict__ seg_begin, const int* __restrict__ seg_end, int n_active,
+                                 const uint32_t* __restrict__ flags, const uint32_t* __restrict__ pos, FmhRoundGenome* out) {
+    const int j = blockIdx.x * blockDim.x + threadIdx.x;
+    if (j >= n_active) return;
+    const int b = seg_begin[j], e = seg_end[j];
+    FmhRoundGenome r;
+    r.count = sg[active[j]].count;
+    r.first = e > b ? pos[b] : 0;
+    r.distinct = e > b ? (unsigned long long)pos[e - 1] + flags[e - 1] - pos[b] : 0;
+    out[j] = r;
+}
+
+__global__ void fmh_scatter_kernel(const uint64_t* __restrict__ sorted, const uint32_t* __restrict__ flags,
+                                   const uint32_t* __restrict__ pos, int n_items, uint64_t* out) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < n_items && flags[i]) out[pos[i]] = sorted[i];
+}
+
+// out[offsets[g] + t] = kept[begin[g] + t] for t < offsets[g + 1] - offsets[g]: the kept values in genome order.
+__global__ void fmh_gather_kernel(const uint64_t* __restrict__ kept, const uint64_t* __restrict__ begin,
+                                  const uint64_t* __restrict__ offsets, int n, uint64_t total, uint64_t* out) {
+    for (uint64_t i = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x; i < total; i += (uint64_t)gridDim.x * blockDim.x) {
+        int lo = 0, hi = n;                           // the last genome whose output begins at or before i
+        while (lo < hi) {
+            const int mid = (lo + hi) >> 1;
+            if (offsets[mid] <= i) lo = mid + 1; else hi = mid;
+        }
+        const int g = lo - 1;
+        out[i] = kept[begin[g] + (i - offsets[g])];
+    }
+}
+
+size_t fmh_scan_temp_bytes(int n_items) {
+    size_t t = 0;
+    cub::DeviceScan::ExclusiveSum(nullptr, t, (const uint32_t*)nullptr, (uint32_t*)nullptr, n_items);
+    return t;
+}
+
+int launch_fmh_distinct(const SketchGenome* d_sg, const int* d_active, int n_active, const int* d_seg, int n_items,
+                        const uint64_t* d_sorted, uint32_t* d_flags, uint32_t* d_pos, void* temp, size_t temp_bytes,
+                        FmhRoundGenome* d_out, cudaStream_t s) {
+    if (n_active <= 0) return KMERML_OK;
+    if (n_items > 0) {
+        fmh_flag_kernel<<<(n_items + 255) / 256, 256, 0, s>>>(d_sorted, d_sg, d_active, d_seg, d_seg + n_active, n_active,
+                                                             n_items, d_flags);
+        KM_CUDA(cudaGetLastError());
+        size_t tb = temp_bytes;
+        KM_CUDA(cub::DeviceScan::ExclusiveSum(temp, tb, d_flags, d_pos, n_items, s));
+    }
+    fmh_round_kernel<<<(n_active + 255) / 256, 256, 0, s>>>(d_sg, d_active, d_seg, d_seg + n_active, n_active, d_flags,
+                                                            d_pos, d_out);
+    KM_CUDA(cudaGetLastError());
+    return KMERML_OK;
+}
+
+int launch_fmh_scatter(const uint64_t* d_sorted, const uint32_t* d_flags, const uint32_t* d_pos, int n_items, uint64_t* d_out,
+                       cudaStream_t s) {
+    if (n_items <= 0) return KMERML_OK;
+    fmh_scatter_kernel<<<(n_items + 255) / 256, 256, 0, s>>>(d_sorted, d_flags, d_pos, n_items, d_out);
+    KM_CUDA(cudaGetLastError());
+    return KMERML_OK;
+}
+
+int launch_fmh_gather(const uint64_t* d_kept, const uint64_t* d_begin, const uint64_t* d_offsets, int n, uint64_t total,
+                      uint64_t* d_out, cudaStream_t s) {
+    if (!total) return KMERML_OK;
+    const uint64_t blocks = std::min<uint64_t>((total + 255) / 256, 1ull << 16);
+    fmh_gather_kernel<<<(unsigned)blocks, 256, 0, s>>>(d_kept, d_begin, d_offsets, n, total, d_out);
+    KM_CUDA(cudaGetLastError());
+    return KMERML_OK;
+}
+
+// ---- |Q n R| of two sets of scaled sketches ----------------------------------------------------------------------
+constexpr int FMH_THREADS = 256;
+constexpr int FMH_CHUNK = 8192;                       // reference values one CTA holds in shared memory (64 KB)
+constexpr int FMH_QROWS = 32;                         // queries one CTA compares with its chunk
+constexpr int FMH_BUCKET_BITS = 11;                   // 2048 buckets index the chunk (8 KB)
+constexpr size_t FMH_SMEM = (size_t)FMH_CHUNK * 8 + ((1u << FMH_BUCKET_BITS) + 1) * 4;
+
+// chunks[r] = ceil(|R_r| / FMH_CHUNK), prefix[r] = chunks before reference r, prefix[n_r] = all chunks (one CTA).
+__global__ void __launch_bounds__(SELECT_THREADS)
+fmh_chunk_prefix_kernel(const uint64_t* __restrict__ r_off, int n_r, unsigned long long* prefix) {
+    using Scan = cub::BlockScan<unsigned long long, SELECT_THREADS>;
+    __shared__ typename Scan::TempStorage tmp;
+    unsigned long long carry = 0;
+    for (int base = 0; base < n_r; base += SELECT_THREADS) {
+        const int r = base + threadIdx.x;
+        const unsigned long long c = r < n_r ? (r_off[r + 1] - r_off[r] + FMH_CHUNK - 1) / FMH_CHUNK : 0;
+        unsigned long long x, total;
+        Scan(tmp).ExclusiveSum(c, x, total);
+        if (r < n_r) prefix[r] = carry + x;
+        carry += total;
+        __syncthreads();
+    }
+    if (threadIdx.x == 0) prefix[n_r] = carry;
+}
+
+// First index in [lo, hi) of the ascending list A whose value is >= x (hi if none), the same in every lane: 32 probes
+// per step cut the range into 33 parts, so a list of millions takes four or five dependent loads.
+__device__ __forceinline__ uint64_t warp_lower_bound(const uint64_t* __restrict__ A, uint64_t lo, uint64_t hi, uint64_t x,
+                                                     int lane) {
+    while (hi - lo > 32) {
+        const uint64_t p = lo + (hi - lo) * (uint64_t)(lane + 1) / 33;
+        const int c = __popc(__ballot_sync(0xffffffffu, A[p] < x));
+        const uint64_t below = __shfl_sync(0xffffffffu, p, c ? c - 1 : 0);
+        const uint64_t above = __shfl_sync(0xffffffffu, p, c < 32 ? c : 31);
+        if (c) lo = below + 1;
+        if (c < 32) hi = above;
+    }
+    const uint64_t p = lo + lane;
+    return lo + __popc(__ballot_sync(0xffffffffu, p < hi && A[p] < x));
+}
+
+// Work item = (chunk of FMH_CHUNK values of one reference, block of FMH_QROWS queries); CTAs stride over the items, so
+// a long reference is spread over many CTAs and the query count is not bounded by the grid.  The chunk sits in shared
+// memory with an index of 2^FMH_BUCKET_BITS buckets of (value - chunk min) >> shift; a warp per query finds the part
+// of its sketch inside [chunk min, chunk max] with two warp-wide searches in global memory, then looks up 32 values at
+// a time (index, then a binary search inside the bucket) and counts the hits with a ballot.  The chunks of a reference
+// split its values, so their partial counts add up to |Q n R| exactly (one atomic per query and chunk).
+__global__ void __launch_bounds__(FMH_THREADS)
+fmh_intersect_kernel(const uint64_t* __restrict__ qh, const uint64_t* __restrict__ q_off, int n_q,
+                     const uint64_t* __restrict__ rh, const uint64_t* __restrict__ r_off, int n_r,
+                     const unsigned long long* __restrict__ prefix, uint32_t* inter) {
+    extern __shared__ uint64_t s_r[];
+    uint32_t* s_idx = (uint32_t*)(s_r + FMH_CHUNK);
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const unsigned long long n_qb = (unsigned long long)(n_q + FMH_QROWS - 1) / FMH_QROWS;
+    const unsigned long long n_items = prefix[n_r] * n_qb;
+    for (unsigned long long item = blockIdx.x; item < n_items; item += gridDim.x) {
+        const unsigned long long c = item / n_qb;
+        const int qb = (int)(item % n_qb);
+        int lo = 0, hi = n_r - 1;                     // the reference of chunk c: the last one whose chunks begin <= c
+        while (lo < hi) {
+            const int mid = (lo + hi + 1) >> 1;
+            if (prefix[mid] <= c) lo = mid; else hi = mid - 1;
+        }
+        const int r = lo;
+        const uint64_t c_lo = r_off[r] + (c - prefix[r]) * FMH_CHUNK;
+        const int len = (int)min((uint64_t)FMH_CHUNK, r_off[r + 1] - c_lo);
+        __syncthreads();                              // the previous item is done with the chunk
+        for (int t = tid; t < len; t += FMH_THREADS) s_r[t] = rh[c_lo + t];
+        __syncthreads();
+        const uint64_t cmin = s_r[0], cmax = s_r[len - 1];
+        const uint64_t span = cmax - cmin;
+        const int bits = span ? 64 - __clzll((long long)span) : 0;
+        const int shift = bits > FMH_BUCKET_BITS ? bits - FMH_BUCKET_BITS : 0;
+        for (int t = tid; t < len; t += FMH_THREADS) {      // s_idx[b] = first position of bucket >= b
+            const int b = (int)((s_r[t] - cmin) >> shift);
+            const int bp = t ? (int)((s_r[t - 1] - cmin) >> shift) : -1;
+            for (int bb = bp + 1; bb <= b; bb++) s_idx[bb] = t;
+            if (t == len - 1) s_idx[b + 1] = len;
+        }
+        __syncthreads();
+        const int q_end = min(n_q, (qb + 1) * FMH_QROWS);
+        for (int q = qb * FMH_QROWS + warp; q < q_end; q += FMH_THREADS / 32) {
+            const uint64_t* Q = qh + q_off[q];
+            const uint64_t nq = q_off[q + 1] - q_off[q];
+            const uint64_t a = warp_lower_bound(Q, 0, nq, cmin, lane);
+            const uint64_t e = cmax == ~0ull ? nq : warp_lower_bound(Q, a, nq, cmax + 1, lane);
+            uint32_t hits = 0;
+            for (uint64_t t0 = a; t0 < e; t0 += 32) {
+                const uint64_t t = t0 + lane;
+                bool found = false;
+                if (t < e) {
+                    const uint64_t v = Q[t];
+                    const int b = (int)((v - cmin) >> shift);
+                    int l = (int)s_idx[b], h = (int)s_idx[b + 1];
+                    const int h0 = h;
+                    while (l < h) {
+                        const int mid = (l + h) >> 1;
+                        if (s_r[mid] < v) l = mid + 1; else h = mid;
+                    }
+                    found = l < h0 && s_r[l] == v;
+                }
+                hits += __popc(__ballot_sync(0xffffffffu, found));
+            }
+            if (lane == 0 && hits) atomicAdd(inter + (uint64_t)q * n_r + r, hits);
+        }
+    }
+}
+
+// The metric of x = |Q n R| (float64; 0 when x = 0, which covers every zero denominator).
+__device__ __forceinline__ double fmh_metric(uint32_t x, uint64_t nq, uint64_t nr, int k, int metric) {
+    if (!x) return 0.0;
+    const double dx = (double)x;
+    switch (metric) {
+        case KMERML_FMH_CONTAINMENT: return dx / (double)nq;
+        case KMERML_FMH_MAX_CONTAINMENT: return dx / (double)min(nq, nr);
+        case KMERML_FMH_JACCARD: return dx / (double)(nq + nr - x);
+        case KMERML_FMH_CONTAINMENT_ANI: return pow(dx / (double)nq, 1.0 / k);
+        default: return pow(dx / (double)min(nq, nr), 1.0 / k);
+    }
+}
+
+__global__ void fmh_metric_kernel(const uint32_t* __restrict__ inter, const uint64_t* __restrict__ q_off, int n_q,
+                                  const uint64_t* __restrict__ r_off, int n_r, int k, int metric, float* out32,
+                                  double* out64) {
+    const uint64_t n = (uint64_t)n_q * n_r;
+    for (uint64_t i = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x; i < n; i += (uint64_t)gridDim.x * blockDim.x) {
+        const int q = (int)(i / n_r), r = (int)(i % n_r);
+        const double d = fmh_metric(inter[i], q_off[q + 1] - q_off[q], r_off[r + 1] - r_off[r], k, metric);
+        if (out64) out64[i] = d;
+        if (out32) out32[i] = (float)d;
+    }
+}
+
+size_t fmh_compare_workspace(int n_r) { return (size_t)(n_r + 1) * 8; }
+
+int launch_fmh_compare(const uint64_t* d_qh, const uint64_t* d_q_off, int n_q, const uint64_t* d_rh, const uint64_t* d_r_off,
+                       int n_r, int k, int metric, int sm_count, void* workspace, uint32_t* d_inter, float* d_out32,
+                       double* d_out64, cudaStream_t s) {
+    if (n_q <= 0 || n_r <= 0) return KMERML_OK;
+    unsigned long long* prefix = (unsigned long long*)workspace;
+    KM_CUDA(cudaMemsetAsync(d_inter, 0, (size_t)n_q * n_r * 4, s));
+    fmh_chunk_prefix_kernel<<<1, SELECT_THREADS, 0, s>>>(d_r_off, n_r, prefix);
+    KM_CUDA(cudaGetLastError());
+    KM_CUDA(cudaFuncSetAttribute(fmh_intersect_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)FMH_SMEM));
+    // three CTAs fit an SM's shared memory; eight rounds of them let the CTAs of long items be balanced by the rest
+    fmh_intersect_kernel<<<sm_count * 3 * 8, FMH_THREADS, FMH_SMEM, s>>>(d_qh, d_q_off, n_q, d_rh, d_r_off, n_r, prefix,
+                                                                      d_inter);
+    KM_CUDA(cudaGetLastError());
+    if (d_out32 || d_out64) {
+        const uint64_t n = (uint64_t)n_q * n_r;
+        const uint64_t blocks = std::min<uint64_t>((n + 255) / 256, 1ull << 16);
+        fmh_metric_kernel<<<(unsigned)blocks, 256, 0, s>>>(d_inter, d_q_off, n_q, d_r_off, n_r, k, metric, d_out32, d_out64);
+        KM_CUDA(cudaGetLastError());
+    }
     return KMERML_OK;
 }
 

@@ -647,7 +647,7 @@ def sketch_batch_device(fasta, offsets, k, *, sketch_size=1000, seed=42, canonic
 def _check_sketches(*sketches):
     for sk in sketches[1:]:
         if sk.params() != sketches[0].params():
-            raise ValueError("sketches differ in k, sketch size, seed or canonical flag: "
+            raise ValueError("sketches differ in k, sketch size or scale, seed or canonical flag: "
                              f"{sketches[0].params()} vs {sk.params()}")
 
 
@@ -684,3 +684,99 @@ def concat_sketches(*sketches):
     first = sketches[0]
     return Sketches(torch.cat([sk.hashes for sk in sketches]), torch.cat([sk.filled for sk in sketches]),
                     first.k, first.s, first.seed, first.canonical)
+
+
+@dataclass
+class ScaledSketches:
+    """Scaled (FracMinHash) sketches of a batch of genomes (kmerml_fmh_batch): genome g's sketch is
+    hashes[offsets[g]:offsets[g + 1]], every distinct hash <= (2^64 - 1) // scale of its k-mers, ascending."""
+    hashes: torch.Tensor      # [total] int64 storage of uint64
+    offsets: torch.Tensor     # [n + 1] int64
+    k: int
+    scale: int
+    seed: int
+    canonical: bool
+
+    def __len__(self):
+        return self.offsets.shape[0] - 1
+
+    def sizes(self):
+        """[n] int64: the number of hashes of each sketch."""
+        return self.offsets[1:] - self.offsets[:-1]
+
+    def params(self):
+        return (self.k, self.scale, self.seed, self.canonical)
+
+
+_FMH_METRIC = {"containment": _lib.FMH_CONTAINMENT, "max_containment": _lib.FMH_MAX_CONTAINMENT,
+               "jaccard": _lib.FMH_JACCARD, "containment_ani": _lib.FMH_CONTAINMENT_ANI,
+               "max_containment_ani": _lib.FMH_MAX_CONTAINMENT_ANI}
+
+
+def fmh_batch_device(fasta, offsets, k, *, scale=1000, seed=42, canonical=True, min_record_len=None):
+    """Scaled sketches of genomes already resident in HBM (laid out as for count_dense_device), any k <= 32.  The
+    output is sized from a guess (1.25 hashes per `scale` bytes, + 256 per genome); a batch with more hashes than that
+    is copied out of the library's workspace once its size is known (kmerml_fmh_fetch), never sketched twice."""
+    if not (fasta.is_cuda and fasta.dtype == torch.uint8 and fasta.is_contiguous()):
+        raise ValueError("fasta must be a contiguous uint8 CUDA tensor")
+    ctx = _lib.context(fasta.device.index)
+    L = _lib.load()
+    n = len(offsets) - 1
+    offs = np.asarray(offsets, dtype=np.uint64)
+    scale = int(scale)
+    guess = int(sum(int(offs[g + 1] - offs[g]) / max(scale, 1) * 1.25 + 256 for g in range(n)))
+    hashes = torch.empty(max(guess, 1), dtype=torch.int64, device=fasta.device)
+    sk_offsets = torch.empty(n + 1, dtype=torch.int64, device=fasta.device)
+    total = ctypes.c_uint64(0)
+    stream = ctypes.c_void_p(torch.cuda.current_stream(fasta.device).cuda_stream)
+    _retry_after_cache_release(lambda: _lib.check(L.kmerml_fmh_batch(
+        ctx.handle, fasta.data_ptr() if fasta.numel() else None, offs.ctypes.data, n, int(k), int(min_record_len or 0),
+        _lib.FLAG_CANONICAL if canonical else 0, scale, int(seed) & 0xFFFFFFFFFFFFFFFF, hashes.data_ptr(), guess,
+        sk_offsets.data_ptr(), ctypes.byref(total), stream)))
+    if total.value > guess:
+        hashes = torch.empty(int(total.value), dtype=torch.int64, device=fasta.device)
+        _lib.check(L.kmerml_fmh_fetch(ctx.handle, hashes.data_ptr(), total.value, sk_offsets.data_ptr(), stream))
+    return ScaledSketches(hashes[:int(total.value)], sk_offsets, int(k), scale, int(seed), bool(canonical))
+
+
+def fmh_compare_device(queries, references=None, metric="containment", *, out_dtype=torch.float32,
+                       want_intersections=False):
+    """[n_q, n_r] similarity of every query sketch to every reference sketch (the queries themselves when
+    `references` is None): "containment" |Q n R| / |Q|, "max_containment" |Q n R| / min(|Q|, |R|), "jaccard",
+    "containment_ani" and "max_containment_ani" (the containment to the power 1/k); 0 when |Q n R| = 0.
+    With want_intersections, also the exact [n_q, n_r] int64 |Q n R|."""
+    if metric not in _FMH_METRIC:
+        raise ValueError(f"metric must be one of {sorted(_FMH_METRIC)}")
+    if out_dtype not in (torch.float32, torch.float64):
+        raise ValueError("out_dtype must be torch.float32 or torch.float64")
+    refs = queries if references is None else references
+    if not (isinstance(queries, ScaledSketches) and isinstance(refs, ScaledSketches)):
+        raise ValueError("queries and references must be ScaledSketches")
+    _check_sketches(queries, refs)
+    dev = queries.hashes.device
+    n_q, n_r = len(queries), len(refs)
+    out = torch.empty((n_q, n_r), dtype=out_dtype, device=dev)
+    inter = torch.empty((n_q, n_r), dtype=torch.int32, device=dev) if want_intersections else None
+    if out.numel():
+        ctx = _lib.context(dev.index)
+        stream = torch.cuda.current_stream(dev).cuda_stream
+        _lib.check(_lib.load().kmerml_fmh_compare(
+            ctx.handle, queries.hashes.data_ptr(), queries.offsets.data_ptr(), n_q, refs.hashes.data_ptr(),
+            refs.offsets.data_ptr(), n_r, queries.k, _FMH_METRIC[metric],
+            inter.data_ptr() if inter is not None else None, out.data_ptr() if out_dtype == torch.float32 else None,
+            out.data_ptr() if out_dtype == torch.float64 else None, ctypes.c_void_p(stream)))
+    if want_intersections:
+        return out, inter.to(torch.int64)
+    return out
+
+
+def concat_scaled_sketches(*sketches):
+    """One ScaledSketches of several batches (same k, scale, seed and canonical flag), genomes in argument order."""
+    _check_sketches(*sketches)
+    first = sketches[0]
+    offs, base = [first.offsets[:1]], 0
+    for sk in sketches:
+        offs.append(sk.offsets[1:] + base)
+        base += int(sk.offsets[-1])
+    return ScaledSketches(torch.cat([sk.hashes for sk in sketches]), torch.cat(offs), first.k, first.scale, first.seed,
+                          first.canonical)

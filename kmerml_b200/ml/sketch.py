@@ -1,6 +1,7 @@
 """Genome x genome Mash / Jaccard distances from MinHash sketches, for any k up to 32 (engine.sketch_batch_device,
 engine.sketch_distance_device).  The matrix feeds `hierarchical_clustering(..., distances=...)` and
-`dbscan_clustering(..., distances=...)` directly."""
+`dbscan_clustering(..., distances=...)` directly.  Query x reference containment, Jaccard and ANI from scaled
+(FracMinHash) sketches (engine.fmh_batch_device, engine.fmh_compare_device): `containment_matrix`."""
 from pathlib import Path
 
 import numpy as np
@@ -8,6 +9,14 @@ import pandas as pd
 import torch
 
 from .. import engine
+
+
+def _load_batch(paths, dev):
+    data = [np.fromfile(str(p), dtype=np.uint8) for p in paths]
+    offsets = np.concatenate(([0], np.cumsum([d.size for d in data]))).tolist()
+    host = np.concatenate(data) if data else np.zeros(0, np.uint8)
+    fasta = torch.from_numpy(host).to(dev) if host.size else torch.zeros(0, dtype=torch.uint8, device=dev)
+    return fasta, offsets
 
 
 def sketch_distance_matrix(fasta_paths, k=21, sketch_size=1000, seed=42, canonical=True, metric="mash",
@@ -28,3 +37,26 @@ def sketch_distance_matrix(fasta_paths, k=21, sketch_size=1000, seed=42, canonic
     sk = engine.sketch_batch_device(fasta, offsets, k, sketch_size=sketch_size, seed=seed, canonical=canonical)
     d = engine.sketch_distance_device(sk, metric, out_dtype=torch.float64).cpu().numpy()
     return pd.DataFrame(d, index=organism_ids, columns=organism_ids)
+
+
+def containment_matrix(query_paths, reference_paths=None, *, k=21, scale=1000, seed=42, canonical=True,
+                       metric="containment", query_ids=None, reference_ids=None, device=None):
+    """DataFrame of a similarity of every query genome to every reference genome (one FASTA file each) from scaled
+    sketches: index = query ids, columns = reference ids (file stems unless given).  Without `reference_paths` the
+    queries are compared with each other.  `metric` is one of engine.fmh_compare_device's; all are similarities, so
+    with "max_containment_ani" (symmetric) `1 - df` goes straight into `hierarchical_clustering(..., distances=...)`."""
+    q_paths = [Path(p) for p in query_paths]
+    r_paths = q_paths if reference_paths is None else [Path(p) for p in reference_paths]
+    q_ids = [p.stem for p in q_paths] if query_ids is None else list(query_ids)
+    if reference_ids is None:
+        r_ids = q_ids if reference_paths is None else [p.stem for p in r_paths]
+    else:
+        r_ids = list(reference_ids)
+    if len(q_ids) != len(q_paths) or len(r_ids) != len(r_paths):
+        raise ValueError("Number of ids must match number of genome paths")
+    dev = torch.device(device if device is not None else "cuda")
+    params = dict(scale=scale, seed=seed, canonical=canonical)
+    queries = engine.fmh_batch_device(*_load_batch(q_paths, dev), k, **params)
+    refs = None if reference_paths is None else engine.fmh_batch_device(*_load_batch(r_paths, dev), k, **params)
+    d = engine.fmh_compare_device(queries, refs, metric, out_dtype=torch.float64).cpu().numpy()
+    return pd.DataFrame(d, index=q_ids, columns=r_ids)
