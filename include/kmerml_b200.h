@@ -457,6 +457,29 @@ int kmerml_fmh_compare(kmerml_ctx *ctx, const uint64_t *d_q_hashes, const uint64
                        uint32_t *d_intersections, float *d_out32, double *d_out64, void *stream);
 
 /*
+ * kmerml_fmh_gather: split each query sketch greedily and exactly into the reference sketches that cover it (gather,
+ * Irber et al. 2022: a greedy minimum set cover).  The inputs are two CSR sets of sketches as for kmerml_fmh_compare
+ * (same k, scale, seed and canonical flag -- not checked here; the two sets may be the same pointers).  For query Q
+ * and references R_0 .. R_{n_r - 1}: Q_0 = Q; in round t = 1, 2, ..., u_t(r) = |Q_{t-1} n R_r| for every r, and
+ * r_t = argmax_r u_t(r), ties going to the smallest reference index.  The query stops, without recording, when
+ * u_t(r_t) < threshold or when max_matches matches have been recorded.  Otherwise match t - 1 records reference r_t,
+ * unique u_t(r_t), intersect |Q_0 n R_{r_t}| and remaining |Q_t| = |Q_{t-1}| - unique, and Q_t = Q_{t-1} \ R_{r_t}.
+ * So no reference is picked twice, unique never grows, and the result is a deterministic function of the sketches:
+ * a block of queries gives the same rows as the whole call.
+ * Outputs: d_n_matches[q] (n_q values, always written: 0 when n_r == 0); match t of query q in slot
+ * q * max_matches + t of d_match_ref, d_match_unique, d_match_intersect and d_match_remaining (n_q * max_matches
+ * values each); slots past d_n_matches[q] are not written.  Counts are uint32, as in kmerml_fmh_compare.
+ * threshold >= 1, max_matches >= 1; n_q == 0 returns at once.
+ * Device workspace (the context's, kept between calls): 4 n_q n_r bytes for |Q n R|, then for the n_c candidate
+ * references (those with |Q n R| >= threshold for some query) 8 (their total hashes) + 8 n_q n_c bytes, plus
+ * 9 (total query hashes) + 24 n_q bytes.  Synchronous: one host read per round.
+ */
+int kmerml_fmh_gather(kmerml_ctx *ctx, const uint64_t *d_q_hashes, const uint64_t *d_q_offsets, int n_q,
+                      const uint64_t *d_r_hashes, const uint64_t *d_r_offsets, int n_r, uint32_t threshold,
+                      int max_matches, int32_t *d_n_matches, int32_t *d_match_ref, uint32_t *d_match_unique,
+                      uint32_t *d_match_intersect, uint32_t *d_match_remaining, void *stream);
+
+/*
  * Measurement hooks (bench.py): with profiling enabled every kernel the library
  * launches is bracketed by CUDA events on the launching stream.  kmerml_profile_read
  * synchronises those events and returns the accumulated device time per kernel family

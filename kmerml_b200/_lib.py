@@ -104,6 +104,7 @@ def load():
     L.kmerml_fmh_batch.argtypes = [vp, vp, vp, i32, i32, i32, u32, u64, u64, vp, u64, vp, p64, vp]
     L.kmerml_fmh_fetch.argtypes = [vp, vp, u64, vp, vp]
     L.kmerml_fmh_compare.argtypes = [vp, vp, vp, i32, vp, vp, i32, i32, i32, vp, vp, vp, vp]
+    L.kmerml_fmh_gather.argtypes = [vp, vp, vp, i32, vp, vp, i32, u32, i32, vp, vp, vp, vp, vp, vp]
     L.kmerml_profile_enable.argtypes = [vp, i32]
     L.kmerml_profile_read.argtypes = [vp, ctypes.POINTER(Profile), i32]
     for name in EXPORTS:
@@ -127,7 +128,7 @@ EXPORTS = [
     "kmerml_parse_kmer_lines", "kmerml_feature_keys", "kmerml_feature_line_lengths", "kmerml_feature_write_lines",
     "kmerml_emit_sparse_range", "kmerml_reduce_sparse_windows",
     "kmerml_sketch_batch", "kmerml_sketch_distance_rows",
-    "kmerml_fmh_batch", "kmerml_fmh_fetch", "kmerml_fmh_compare",
+    "kmerml_fmh_batch", "kmerml_fmh_fetch", "kmerml_fmh_compare", "kmerml_fmh_gather",
 ]
 
 

@@ -1914,6 +1914,140 @@ int kmerml_fmh_compare(kmerml_ctx* ctx, const uint64_t* d_q_hashes, const uint64
                               inter, d_out32, d_out64, (cudaStream_t)stream);
 }
 
+// Gather: x = |Q n R| for every pair (launch_fmh_compare), the candidate references (x >= threshold for some query)
+// copied into a compact CSR in reference order, then rounds in lockstep over every running query: select (with the
+// last round's subtraction fused), remove (the hashes the pick takes, as a sorted CSR S_t) and subtract
+// (launch_fmh_compare of S_t against the candidates).  The host reads the number of picks after each select and
+// stops when there were none or max_matches rounds have run.
+static int fmh_gather_core(kmerml_ctx* ctx, const uint64_t* d_qh, const uint64_t* d_q_off, int n_q, const uint64_t* d_rh,
+                           const uint64_t* d_r_off, int n_r, uint32_t threshold, int max_matches, int32_t* d_n_matches,
+                           int32_t* d_ref, uint32_t* d_unique, uint32_t* d_inter, uint32_t* d_rem, cudaStream_t s) {
+    Workspace& ws = ctx->ws[0];
+    KM_CUDA(cudaMemsetAsync(d_n_matches, 0, (size_t)n_q * 4, s));
+    if (!n_r) {
+        KM_CUDA(cudaStreamSynchronize(s));
+        return KMERML_OK;
+    }
+    // ws.part: x (n_q x n_r) | the chunk table of launch_fmh_compare (n_r >= the candidates) | candidate flags
+    const size_t x_bytes = align_up((size_t)n_q * n_r * 4, 256);
+    const size_t table_bytes = align_up(fmh_compare_workspace(n_r), 256);
+    int rc = ws.part.ensure(x_bytes + table_bytes + align_up((size_t)n_r, 256));
+    if (rc) return rc;
+    uint32_t* d_x = (uint32_t*)ws.part.p;
+    void* d_table = (uint8_t*)ws.part.p + x_bytes;
+    uint8_t* d_flags = (uint8_t*)d_table + table_bytes;
+    {
+        Prof pr(ctx, s, 3, 4);
+        rc = launch_fmh_compare(d_qh, d_q_off, n_q, d_rh, d_r_off, n_r, 1, KMERML_FMH_CONTAINMENT, ctx->sm_count, d_table,
+                                d_x, nullptr, nullptr, s);
+        if (!rc) rc = launch_fmh_greedy_flag(d_x, n_q, n_r, threshold, d_flags, s);
+    }
+    if (rc) return rc;
+    std::vector<uint8_t> flags(n_r);
+    std::vector<uint64_t> r_off(n_r + 1);
+    uint64_t q_total = 0;
+    KM_CUDA(cudaMemcpyAsync(flags.data(), d_flags, (size_t)n_r, cudaMemcpyDeviceToHost, s));
+    KM_CUDA(cudaMemcpyAsync(r_off.data(), d_r_off, (size_t)(n_r + 1) * 8, cudaMemcpyDeviceToHost, s));
+    KM_CUDA(cudaMemcpyAsync(&q_total, d_q_off + n_q, 8, cudaMemcpyDeviceToHost, s));
+    KM_CUDA(cudaStreamSynchronize(s));
+    // the candidates: reference index | where its hashes begin | compact CSR offsets
+    std::vector<int> cand;
+    for (int r = 0; r < n_r; r++)
+        if (flags[r]) cand.push_back(r);
+    const int n_c = (int)cand.size();
+    if (!n_c) return KMERML_OK;
+    std::vector<uint64_t> index(2 * (size_t)n_c + 1);
+    for (int c = 0; c < n_c; c++) {
+        index[c] = r_off[cand[c]];
+        index[n_c + c + 1] = index[n_c + c] + (r_off[cand[c] + 1] - r_off[cand[c]]);
+    }
+    const uint64_t c_total = index[2 * (size_t)n_c];
+
+    // ws.scratch: candidate hashes | index | candidate list | u | d | pick | remaining | s_len | s_off | scan temp |
+    // assigned flags (one byte per query hash) | S_t (at most every query hash) | pick count, inconsistency flag
+    size_t at = 0;
+    auto take = [&](size_t bytes) { const size_t a = at; at += align_up(bytes, 256); return a; };
+    const size_t uq = (size_t)n_q * n_c * 4;
+    const size_t temp_bytes = align_up(fmh_greedy_scan_temp_bytes(n_q), 256);
+    const size_t at_ch = take(c_total * 8), at_index = take(index.size() * 8), at_cand = take((size_t)n_c * 4);
+    const size_t at_u = take(uq), at_d = take(uq), at_pick = take((size_t)n_q * 4), at_remaining = take((size_t)n_q * 4);
+    const size_t at_s_len = take((size_t)(n_q + 1) * 8), at_s_off = take((size_t)(n_q + 1) * 8), at_temp = take(temp_bytes);
+    const size_t at_assigned = take(q_total), at_s = take(q_total * 8), at_cnt = take(8);
+    if ((rc = ws.scratch.ensure(at))) return rc;
+    uint8_t* base = (uint8_t*)ws.scratch.p;
+    uint64_t* d_ch = (uint64_t*)(base + at_ch);
+    uint64_t* d_index = (uint64_t*)(base + at_index);
+    const uint64_t* d_c_off = d_index + n_c;
+    int* d_cand = (int*)(base + at_cand);
+    uint32_t* d_u = (uint32_t*)(base + at_u);
+    uint32_t* d_d = (uint32_t*)(base + at_d);
+    int* d_pick = (int*)(base + at_pick);
+    uint32_t* d_remaining = (uint32_t*)(base + at_remaining);
+    unsigned long long* d_s_len = (unsigned long long*)(base + at_s_len);
+    unsigned long long* d_s_off = (unsigned long long*)(base + at_s_off);
+    uint8_t* d_assigned = base + at_assigned;
+    uint64_t* d_s = (uint64_t*)(base + at_s);
+    unsigned int* d_cnt = (unsigned int*)(base + at_cnt);
+    // a pinned word pair for the per-round read of d_cnt
+    Tables t{ws};
+    const size_t at_h = t.take(8);
+    if ((rc = t.open())) return rc;
+    unsigned int* h_cnt = t.host<unsigned int>(at_h);
+
+    KM_CUDA(cudaMemcpyAsync(d_index, index.data(), index.size() * 8, cudaMemcpyHostToDevice, s));
+    KM_CUDA(cudaMemcpyAsync(d_cand, cand.data(), (size_t)n_c * 4, cudaMemcpyHostToDevice, s));
+    KM_CUDA(cudaMemsetAsync(d_pick, 0, (size_t)n_q * 4, s));
+    KM_CUDA(cudaMemsetAsync(d_s_len, 0, (size_t)(n_q + 1) * 8, s));
+    if (q_total) KM_CUDA(cudaMemsetAsync(d_assigned, 0, q_total, s));
+    KM_CUDA(cudaMemsetAsync(d_cnt, 0, 8, s));
+    {
+        Prof pr(ctx, s, 3, 1);
+        if ((rc = launch_fmh_gather(d_rh, d_index, d_c_off, n_c, c_total, d_ch, s))) return rc;
+    }
+    for (int round = 0; round < max_matches; round++) {
+        KM_CUDA(cudaMemsetAsync(d_cnt, 0, 4, s));
+        {
+            Prof pr(ctx, s, 3, 1);
+            rc = launch_fmh_greedy_select(d_u, d_d, n_c, d_x, n_q, n_r, d_cand, d_q_off, round, threshold, max_matches, d_pick,
+                                          d_remaining, d_s_len, d_n_matches, d_ref, d_unique, d_inter, d_rem, d_cnt, s);
+            if (rc) return rc;
+        }
+        KM_CUDA(cudaMemcpyAsync(h_cnt, d_cnt, 8, cudaMemcpyDeviceToHost, s));
+        KM_CUDA(cudaStreamSynchronize(s));
+        // the last round's remove assigned other counts than its select recorded: only unsorted or repeated input
+        // values do that (a round always ends in a select, so every remove is checked)
+        if (h_cnt[1]) return fail(KMERML_ERR_ARG, "fmh gather: the sketches must hold ascending, distinct values");
+        if (!h_cnt[0] || round + 1 == max_matches) break;
+        Prof pr(ctx, s, 3, 5);
+        rc = launch_fmh_greedy_remove(d_qh, d_q_off, n_q, d_ch, d_c_off, d_pick, d_s_len, d_s_off, base + at_temp,
+                                      temp_bytes, d_assigned, d_s, d_cnt + 1, s);
+        if (!rc) rc = launch_fmh_compare(d_s, (const uint64_t*)d_s_off, n_q, d_ch, d_c_off, n_c, 1, KMERML_FMH_CONTAINMENT,
+                                         ctx->sm_count, d_table, d_d, nullptr, nullptr, s);
+        if (rc) return rc;
+    }
+    return KMERML_OK;
+}
+
+int kmerml_fmh_gather(kmerml_ctx* ctx, const uint64_t* d_q_hashes, const uint64_t* d_q_offsets, int n_q,
+                      const uint64_t* d_r_hashes, const uint64_t* d_r_offsets, int n_r, uint32_t threshold, int max_matches,
+                      int32_t* d_n_matches, int32_t* d_match_ref, uint32_t* d_match_unique, uint32_t* d_match_intersect,
+                      uint32_t* d_match_remaining, void* stream) {
+    if (!ctx) return fail(KMERML_ERR_ARG, "ctx is null");
+    if (threshold < 1) return fail(KMERML_ERR_ARG, "threshold must be >= 1");
+    if (max_matches < 1) return fail(KMERML_ERR_ARG, "max_matches must be >= 1");
+    if (n_q < 0 || n_r < 0) return fail(KMERML_ERR_ARG, "n_q and n_r must be >= 0");
+    if (!n_q) return KMERML_OK;
+    if (!d_q_offsets || !d_r_offsets || !d_n_matches || !d_match_ref || !d_match_unique || !d_match_intersect ||
+        !d_match_remaining)
+        return fail(KMERML_ERR_ARG, "null pointer argument");
+    DeviceGuard guard(ctx->device);
+    if (!guard.ok) return fail(KMERML_ERR_CUDA, "cudaSetDevice failed");
+    if (int orc = order_stream(ctx, (cudaStream_t)stream)) return orc;
+    return fmh_gather_core(ctx, d_q_hashes, d_q_offsets, n_q, d_r_hashes, d_r_offsets, n_r, threshold, max_matches,
+                           d_n_matches, d_match_ref, d_match_unique, d_match_intersect, d_match_remaining,
+                           (cudaStream_t)stream);
+}
+
 // NCCL through the process that called us (no link-time dependency): the four entry points the exchange needs.
 namespace {
 struct NcclApi {

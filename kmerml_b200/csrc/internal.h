@@ -227,6 +227,20 @@ size_t fmh_compare_workspace(int n_r);
 int launch_fmh_compare(const uint64_t* d_qh, const uint64_t* d_q_off, int n_q, const uint64_t* d_rh, const uint64_t* d_r_off,
                        int n_r, int k, int metric, int sm_count, void* workspace, uint32_t* d_inter, float* d_out32,
                        double* d_out64, cudaStream_t s);
+// gather: the candidate flags of a prefetched n_q x n_r intersection matrix (zeroed here) ...
+int launch_fmh_greedy_flag(const uint32_t* d_x, int n_q, int n_r, uint32_t threshold, uint8_t* d_flags, cudaStream_t s);
+// ... one round's pick of every running query (d_d: the last round's subtraction, unused in round 0) ...
+int launch_fmh_greedy_select(uint32_t* d_u, const uint32_t* d_d, int n_c, const uint32_t* d_x, int n_q, int n_r,
+                             const int* d_cand, const uint64_t* d_q_off, int round, uint32_t threshold, int max_matches,
+                             int* d_pick, uint32_t* d_remaining, unsigned long long* d_s_len, int32_t* d_n_matches,
+                             int32_t* d_ref, uint32_t* d_unique, uint32_t* d_inter, uint32_t* d_rem,
+                             unsigned int* d_n_picked, cudaStream_t s);
+// ... and the hashes each pick takes, as a sorted CSR (d_s_len, d_s_off: n_q + 1 words; d_s_len[n_q] = 0)
+size_t fmh_greedy_scan_temp_bytes(int n_q);
+int launch_fmh_greedy_remove(const uint64_t* d_qh, const uint64_t* d_q_off, int n_q, const uint64_t* d_ch,
+                             const uint64_t* d_c_off, const int* d_pick, const unsigned long long* d_s_len,
+                             unsigned long long* d_s_off, void* temp, size_t temp_bytes, uint8_t* d_assigned,
+                             uint64_t* d_s_hashes, unsigned int* d_bad, cudaStream_t s);
 
 // ---- k{k}.txt text (format.cu) --------------------------------------------------
 size_t format_workspace_bytes(uint64_t n_bins, uint64_t max_lines);

@@ -22,6 +22,11 @@
 //   fmh_gather_kernel       that buffer in genome order, as CSR
 //   fmh_intersect_kernel    exact |Q n R| of every (query, reference) pair of two sets of scaled sketches, and
 //   fmh_metric_kernel       containment, max-containment, Jaccard or containment ANI (Hera et al. 2023) from it.
+// Gather (Irber et al. 2022) splits each query greedily into the references that cover it, in rounds over all queries:
+//   fmh_greedy_flag_kernel    the candidate references, from a prefetched |Q n R| (fmh_intersect_kernel)
+//   fmh_greedy_select_kernel  per query, the candidate with the most still-unassigned hashes (ties: smallest index)
+//   fmh_greedy_remove_kernel  per query, the hashes that pick takes: marked assigned and listed as a sorted CSR, which
+//                             fmh_intersect_kernel then subtracts from every candidate's count.
 #include <cub/cub.cuh>
 
 #include "sparse_walk.cuh"
@@ -491,6 +496,145 @@ int launch_fmh_compare(const uint64_t* d_qh, const uint64_t* d_q_off, int n_q, c
         fmh_metric_kernel<<<(unsigned)blocks, 256, 0, s>>>(d_inter, d_q_off, n_q, d_r_off, n_r, k, metric, d_out32, d_out64);
         KM_CUDA(cudaGetLastError());
     }
+    return KMERML_OK;
+}
+
+// ---- gather: greedy, exact split of each query into the references that cover it ---------------------------------
+// The host loop is fmh_gather_core (api.cu).  u[q, c] = |Q_{t-1} n R_c| over the candidates c (references with
+// |Q n R| >= threshold for some query; u never grows, so no other reference can be picked).
+constexpr int GREEDY_THREADS = 256;
+constexpr int REMOVE_THREADS = 1024;                  // one CTA holds a whole query: many searches in flight
+
+// flags[r] = 1 when some query shares at least `threshold` hashes with reference r (flags zeroed by the caller).
+__global__ void fmh_greedy_flag_kernel(const uint32_t* __restrict__ x, uint64_t n, int n_r, uint32_t threshold,
+                                       uint8_t* flags) {
+    for (uint64_t i = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x; i < n; i += (uint64_t)gridDim.x * blockDim.x)
+        if (x[i] >= threshold) flags[i % n_r] = 1;
+}
+
+// Round `round` (< max_matches) of every query still running (pick[q] >= 0), one CTA per query.  Round 0 reads u from
+// the prefetched x = |Q n R| (n_q x n_r) through the candidate list; later rounds subtract d = |S_{t-1} n R_c| first.
+// The argmax of the key (u << 32) | ~c is the largest u at the smallest candidate index.  The CTA records the match or
+// stops the query (pick = -1), and leaves in s_len[q] how many hashes the remove step will assign (0 when stopped).
+__global__ void __launch_bounds__(GREEDY_THREADS)
+fmh_greedy_select_kernel(uint32_t* u, const uint32_t* __restrict__ d, int n_c, const uint32_t* __restrict__ x, int n_r,
+                         const int* __restrict__ cand, const uint64_t* __restrict__ q_off, int round, uint32_t threshold,
+                         int max_matches, int* pick, uint32_t* remaining, unsigned long long* s_len, int32_t* n_matches,
+                         int32_t* m_ref, uint32_t* m_unique, uint32_t* m_inter, uint32_t* m_rem,
+                         unsigned int* n_picked) {
+    using Reduce = cub::BlockReduce<unsigned long long, GREEDY_THREADS>;
+    __shared__ typename Reduce::TempStorage tmp;
+    const int q = blockIdx.x;
+    if (pick[q] < 0) return;
+    uint32_t* row = u + (uint64_t)q * n_c;
+    unsigned long long best = 0;
+    for (int c = threadIdx.x; c < n_c; c += GREEDY_THREADS) {
+        const uint32_t v = round == 0 ? x[(uint64_t)q * n_r + cand[c]] : row[c] - d[(uint64_t)q * n_c + c];
+        row[c] = v;
+        best = max(best, ((unsigned long long)v << 32) | (uint32_t)~(uint32_t)c);
+    }
+    best = Reduce(tmp).Reduce(best, cub::Max());
+    if (threadIdx.x) return;
+    const uint32_t un = (uint32_t)(best >> 32);
+    if (un < threshold) {
+        pick[q] = -1;
+        s_len[q] = 0;
+        return;
+    }
+    const int c = (int)~(uint32_t)best;
+    const uint32_t before = round == 0 ? (uint32_t)(q_off[q + 1] - q_off[q]) : remaining[q];
+    const uint64_t slot = (uint64_t)q * max_matches + round;
+    m_ref[slot] = cand[c];
+    m_unique[slot] = un;
+    m_inter[slot] = x[(uint64_t)q * n_r + cand[c]];
+    m_rem[slot] = remaining[q] = before - un;
+    n_matches[q] = round + 1;
+    pick[q] = c;
+    s_len[q] = un;
+    atomicAdd(n_picked, 1u);
+}
+
+// S_t of every query that picked candidate c this round: the values of R_c found in Q and not yet assigned, marked
+// assigned and written ascending (R_c's order) at s_off[q].  One CTA per query; each value of R_c is a binary search
+// in Q.  A count that differs from the select step's u sets *bad.
+__global__ void __launch_bounds__(REMOVE_THREADS)
+fmh_greedy_remove_kernel(const uint64_t* __restrict__ qh, const uint64_t* __restrict__ q_off,
+                         const uint64_t* __restrict__ ch, const uint64_t* __restrict__ c_off, const int* __restrict__ pick,
+                         const unsigned long long* __restrict__ s_off, uint8_t* assigned, uint64_t* s_hashes,
+                         unsigned int* bad) {
+    using Scan = cub::BlockScan<int, REMOVE_THREADS>;
+    __shared__ typename Scan::TempStorage tmp;
+    const int q = blockIdx.x;
+    const int c = pick[q];
+    if (c < 0) return;
+    const uint64_t* Q = qh + q_off[q];
+    const uint64_t nq = q_off[q + 1] - q_off[q];
+    uint8_t* taken = assigned + q_off[q];
+    const uint64_t* R = ch + c_off[c];
+    const uint64_t nr = c_off[c + 1] - c_off[c];
+    uint64_t* out = s_hashes + s_off[q];
+    uint64_t written = 0;
+    for (uint64_t base = 0; base < nr; base += REMOVE_THREADS) {
+        const uint64_t i = base + threadIdx.x;
+        int take = 0;
+        uint64_t v = 0;
+        if (i < nr) {
+            v = R[i];
+            uint64_t lo = 0, hi = nq;
+            while (lo < hi) {
+                const uint64_t mid = (lo + hi) >> 1;
+                if (Q[mid] < v) lo = mid + 1; else hi = mid;
+            }
+            if (lo < nq && Q[lo] == v && !taken[lo]) {
+                taken[lo] = 1;
+                take = 1;
+            }
+        }
+        int pos, total;
+        Scan(tmp).ExclusiveSum(take, pos, total);
+        if (take) out[written + pos] = v;
+        written += total;
+        __syncthreads();
+    }
+    if (threadIdx.x == 0 && written != s_off[q + 1] - s_off[q]) atomicOr(bad, 1u);
+}
+
+int launch_fmh_greedy_flag(const uint32_t* d_x, int n_q, int n_r, uint32_t threshold, uint8_t* d_flags, cudaStream_t s) {
+    const uint64_t n = (uint64_t)n_q * n_r;
+    KM_CUDA(cudaMemsetAsync(d_flags, 0, (size_t)n_r, s));
+    const uint64_t blocks = std::min<uint64_t>((n + 255) / 256, 1ull << 16);
+    fmh_greedy_flag_kernel<<<(unsigned)blocks, 256, 0, s>>>(d_x, n, n_r, threshold, d_flags);
+    KM_CUDA(cudaGetLastError());
+    return KMERML_OK;
+}
+
+int launch_fmh_greedy_select(uint32_t* d_u, const uint32_t* d_d, int n_c, const uint32_t* d_x, int n_q, int n_r,
+                             const int* d_cand, const uint64_t* d_q_off, int round, uint32_t threshold, int max_matches,
+                             int* d_pick, uint32_t* d_remaining, unsigned long long* d_s_len, int32_t* d_n_matches,
+                             int32_t* d_ref, uint32_t* d_unique, uint32_t* d_inter, uint32_t* d_rem,
+                             unsigned int* d_n_picked, cudaStream_t s) {
+    fmh_greedy_select_kernel<<<n_q, GREEDY_THREADS, 0, s>>>(d_u, d_d, n_c, d_x, n_r, d_cand, d_q_off, round, threshold,
+                                                           max_matches, d_pick, d_remaining, d_s_len, d_n_matches,
+                                                           d_ref, d_unique, d_inter, d_rem, d_n_picked);
+    KM_CUDA(cudaGetLastError());
+    return KMERML_OK;
+}
+
+size_t fmh_greedy_scan_temp_bytes(int n_q) {
+    size_t t = 0;
+    cub::DeviceScan::ExclusiveSum(nullptr, t, (const unsigned long long*)nullptr, (unsigned long long*)nullptr, n_q + 1);
+    return t;
+}
+
+int launch_fmh_greedy_remove(const uint64_t* d_qh, const uint64_t* d_q_off, int n_q, const uint64_t* d_ch,
+                             const uint64_t* d_c_off, const int* d_pick, const unsigned long long* d_s_len,
+                             unsigned long long* d_s_off, void* temp, size_t temp_bytes, uint8_t* d_assigned,
+                             uint64_t* d_s_hashes, unsigned int* d_bad, cudaStream_t s) {
+    size_t tb = temp_bytes;
+    KM_CUDA(cub::DeviceScan::ExclusiveSum(temp, tb, d_s_len, d_s_off, n_q + 1, s));
+    fmh_greedy_remove_kernel<<<n_q, REMOVE_THREADS, 0, s>>>(d_qh, d_q_off, d_ch, d_c_off, d_pick, d_s_off, d_assigned,
+                                                           d_s_hashes, d_bad);
+    KM_CUDA(cudaGetLastError());
     return KMERML_OK;
 }
 

@@ -770,6 +770,50 @@ def fmh_compare_device(queries, references=None, metric="containment", *, out_dt
     return out
 
 
+@dataclass
+class GatherResult:
+    """Gather of each query sketch into the reference sketches that cover it (kmerml_fmh_gather): row q lists its
+    matches in pick order, n_matches[q] of them; the columns past that hold -1 (reference) and 0 (counts)."""
+    n_matches: torch.Tensor   # [n_q] int32
+    reference: torch.Tensor   # [n_q, m] int32: reference index of each match
+    unique: torch.Tensor      # [n_q, m] int64: query hashes first assigned to that reference
+    intersect: torch.Tensor   # [n_q, m] int64: |Q n R| of the whole query
+    remaining: torch.Tensor   # [n_q, m] int64: query hashes still unassigned after the match
+
+
+def fmh_gather_device(queries, references, *, threshold=1, max_matches=None):
+    """Greedy, exact gather of every query into the references: repeatedly pick the reference that shares the most
+    still-unassigned query hashes (ties: the smallest reference index) while that number is >= `threshold`, and
+    assign those hashes to it.  The default `max_matches`, min(n_r, max_q |Q| // threshold), never truncates."""
+    if not (isinstance(queries, ScaledSketches) and isinstance(references, ScaledSketches)):
+        raise ValueError("queries and references must be ScaledSketches")
+    _check_sketches(queries, references)
+    threshold = int(threshold)
+    if threshold < 1:
+        raise ValueError("threshold must be >= 1")
+    dev = queries.hashes.device
+    n_q, n_r = len(queries), len(references)
+    if max_matches is None:
+        largest = int(queries.sizes().max()) if n_q else 0
+        max_matches = min(n_r, largest // threshold)
+    max_matches = int(max_matches)
+    if max_matches < 0:
+        raise ValueError("max_matches must be >= 0")
+    n_matches = torch.zeros(n_q, dtype=torch.int32, device=dev)
+    m = max(max_matches, 1)
+    ref = torch.full((n_q, m), -1, dtype=torch.int32, device=dev)
+    counts = torch.zeros((3, n_q, m), dtype=torch.int32, device=dev)       # uint32 unique | intersect | remaining
+    if n_q and max_matches:
+        ctx = _lib.context(dev.index)
+        stream = ctypes.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
+        _retry_after_cache_release(lambda: _lib.check(_lib.load().kmerml_fmh_gather(
+            ctx.handle, queries.hashes.data_ptr(), queries.offsets.data_ptr(), n_q, references.hashes.data_ptr(),
+            references.offsets.data_ptr(), n_r, threshold, m, n_matches.data_ptr(), ref.data_ptr(),
+            counts[0].data_ptr(), counts[1].data_ptr(), counts[2].data_ptr(), stream)))
+    wide = (counts[:, :, :max_matches].to(torch.int64) & 0xFFFFFFFF)
+    return GatherResult(n_matches, ref[:, :max_matches], wide[0], wide[1], wide[2])
+
+
 def concat_scaled_sketches(*sketches):
     """One ScaledSketches of several batches (same k, scale, seed and canonical flag), genomes in argument order."""
     _check_sketches(*sketches)

@@ -1,7 +1,8 @@
 """Genome x genome Mash / Jaccard distances from MinHash sketches, for any k up to 32 (engine.sketch_batch_device,
 engine.sketch_distance_device).  The matrix feeds `hierarchical_clustering(..., distances=...)` and
 `dbscan_clustering(..., distances=...)` directly.  Query x reference containment, Jaccard and ANI from scaled
-(FracMinHash) sketches (engine.fmh_batch_device, engine.fmh_compare_device): `containment_matrix`."""
+(FracMinHash) sketches (engine.fmh_batch_device, engine.fmh_compare_device): `containment_matrix`.  Which references make up each query,
+and how much of it each explains (engine.fmh_gather_device): `gather`."""
 from pathlib import Path
 
 import numpy as np
@@ -60,3 +61,42 @@ def containment_matrix(query_paths, reference_paths=None, *, k=21, scale=1000, s
     refs = None if reference_paths is None else engine.fmh_batch_device(*_load_batch(r_paths, dev), k, **params)
     d = engine.fmh_compare_device(queries, refs, metric, out_dtype=torch.float64).cpu().numpy()
     return pd.DataFrame(d, index=q_ids, columns=r_ids)
+
+
+def _ids(paths, ids):
+    ids = [p.stem for p in paths] if ids is None else list(ids)
+    if len(ids) != len(paths):
+        raise ValueError("Number of ids must match number of genome paths")
+    return ids
+
+
+def gather(query_paths, reference_paths, *, k=21, scale=1000, seed=42, canonical=True, threshold_bp=50_000,
+           query_ids=None, reference_ids=None, device=None):
+    """Long DataFrame of the gather of every query genome into the reference genomes (one FASTA file each; ids are
+    the file stems unless given): one row per (query, match) in pick order.  A reference is picked while it covers at
+    least max(1, ceil(threshold_bp / scale)) still-unassigned query hashes.  Columns: query, rank (0-based), match,
+    intersect_bp / unique_bp / remaining_bp (hash counts times `scale`), f_orig_query = intersect / |Q|,
+    f_match = intersect / |R|, f_unique_to_query = unique / |Q| and match_containment_ani = (intersect / |R|)^(1/k),
+    all in float64."""
+    q_paths = [Path(p) for p in query_paths]
+    r_paths = [Path(p) for p in reference_paths]
+    q_ids, r_ids = _ids(q_paths, query_ids), _ids(r_paths, reference_ids)
+    dev = torch.device(device if device is not None else "cuda")
+    params = dict(scale=scale, seed=seed, canonical=canonical)
+    queries = engine.fmh_batch_device(*_load_batch(q_paths, dev), k, **params)
+    refs = engine.fmh_batch_device(*_load_batch(r_paths, dev), k, **params)
+    threshold = max(1, -(-int(threshold_bp) // int(scale)))
+    res = engine.fmh_gather_device(queries, refs, threshold=threshold)
+    n = res.n_matches.cpu().numpy()
+    q_of = np.repeat(np.arange(len(q_ids)), n)
+    rank = np.concatenate([np.arange(c) for c in n]) if len(n) else np.zeros(0, np.int64)
+    ref = res.reference.cpu().numpy()[q_of, rank]
+    unique, inter, remaining = (x.cpu().numpy()[q_of, rank].astype(np.float64)
+                                for x in (res.unique, res.intersect, res.remaining))
+    q_size = queries.sizes().cpu().numpy().astype(np.float64)[q_of]
+    r_size = refs.sizes().cpu().numpy().astype(np.float64)[ref]
+    return pd.DataFrame({
+        "query": [q_ids[i] for i in q_of], "rank": rank.astype(np.int64), "match": [r_ids[i] for i in ref],
+        "intersect_bp": inter * scale, "unique_bp": unique * scale, "remaining_bp": remaining * scale,
+        "f_orig_query": inter / q_size, "f_match": inter / r_size, "f_unique_to_query": unique / q_size,
+        "match_containment_ani": (inter / r_size) ** (1.0 / k)})
