@@ -457,6 +457,48 @@ int kmerml_fmh_compare(kmerml_ctx *ctx, const uint64_t *d_q_hashes, const uint64
                        uint32_t *d_intersections, float *d_out32, double *d_out64, void *stream);
 
 /*
+ * k-mer abundance in scaled sketches: how many windows of a genome carry each kept hash, so a metagenome says how much
+ * of each genome it holds, not only which genomes.
+ *
+ * KMERML_FLAG_FMH_ABUNDANCE (flag of kmerml_fmh_batch): also keep, for every value h of every sketch, its abundance
+ * a_g(h) = the number of windows of genome g whose key hashes to h (the windows the sketch counts; with
+ * KMERML_FLAG_CANONICAL both orientations count toward the canonical key), as uint32.  The stored windows of one genome
+ * are at most 2^31 - 1, so every sum below fits uint64 exactly: sum a <= 2^31, sum a_Q a_R <= 2^62, sum a^2 <= 2^62.
+ * The hashes and offsets are those of the call without the flag.  Without the flag nothing extra is kept.
+ *
+ * kmerml_fmh_fetch_abundances: the abundances of the last kmerml_fmh_batch call of this context, in the CSR order of
+ * kmerml_fmh_fetch (d_abundances: out_cap >= its total).  KMERML_ERR_ARG when that call was made without
+ * KMERML_FLAG_FMH_ABUNDANCE or out_cap is short.  Synchronous.
+ *
+ * kmerml_fmh_compare_weighted: two CSR sets of sketches as for kmerml_fmh_compare, with their abundances
+ * (d_r_abundances may be NULL for KMERML_FMH_WEIGHTED_CONTAINMENT).  For every query q and reference r:
+ *   KMERML_FMH_WEIGHTED_CONTAINMENT  x = sum_{h in Q n R} a_Q(h), metric x / sum_{h in Q} a_Q(h): the share of the
+ *                                    query's k-mer mass (reads, coverage) that R explains;
+ *   KMERML_FMH_ANGULAR_SIMILARITY    x = sum_{h in Q n R} a_Q(h) a_R(h), metric 1 - 2 acos(c) / pi with
+ *                                    c = min(1, x / (sqrt(sum_Q a_Q^2) sqrt(sum_R a_R^2))), and c = 1 whenever
+ *                                    x^2 = sum_Q a_Q^2 sum_R a_R^2 exactly (proportional abundances, self-similarity).
+ * Both are 0 when x = 0 or a denominator is 0.  The integer x goes to d_numerators (uint64), the metric in float64 to
+ * d_out64 and rounded to d_out32 (n_q x n_r each, any of them NULL, not all three).  The sums are integers and the
+ * product of the two roots commutes, so Q = R gives an exactly symmetric matrix, and a block of query rows is
+ * bit-identical to the same rows of the whole matrix.  Asynchronous on `stream`.
+ *
+ * kmerml_fmh_gather_abundance: kmerml_fmh_gather with the query abundances d_q_abundances (parallel to d_q_hashes).
+ * The picks are made on the unweighted counts, so the first outputs are those of kmerml_fmh_gather.  For match t of
+ * query q, with S_t the query hashes that match takes, slot q * max_matches + t of d_match_unique_weighted receives
+ * sum_{S_t} a_Q (uint64), of d_match_unique_sumsq sum_{S_t} a_Q^2 (uint64), and of d_match_median_abund the median of
+ * a_Q over S_t (float64; for an even count the mean of the two middle values, exact).  Extra device workspace:
+ * 8 (total query hashes) + 16 n_q bytes and a segmented sort's temporary storage.  Synchronous.
+ */
+#define KMERML_FLAG_FMH_ABUNDANCE 64u
+#define KMERML_FMH_WEIGHTED_CONTAINMENT 5
+#define KMERML_FMH_ANGULAR_SIMILARITY 6
+int kmerml_fmh_fetch_abundances(kmerml_ctx *ctx, uint32_t *d_abundances, uint64_t out_cap, void *stream);
+int kmerml_fmh_compare_weighted(kmerml_ctx *ctx, const uint64_t *d_q_hashes, const uint64_t *d_q_offsets,
+                                const uint32_t *d_q_abundances, int n_q, const uint64_t *d_r_hashes,
+                                const uint64_t *d_r_offsets, const uint32_t *d_r_abundances, int n_r, int metric,
+                                uint64_t *d_numerators, float *d_out32, double *d_out64, void *stream);
+
+/*
  * kmerml_fmh_gather: split each query sketch greedily and exactly into the reference sketches that cover it (gather,
  * Irber et al. 2022: a greedy minimum set cover).  The inputs are two CSR sets of sketches as for kmerml_fmh_compare
  * (same k, scale, seed and canonical flag -- not checked here; the two sets may be the same pointers).  For query Q
@@ -478,6 +520,12 @@ int kmerml_fmh_gather(kmerml_ctx *ctx, const uint64_t *d_q_hashes, const uint64_
                       const uint64_t *d_r_hashes, const uint64_t *d_r_offsets, int n_r, uint32_t threshold,
                       int max_matches, int32_t *d_n_matches, int32_t *d_match_ref, uint32_t *d_match_unique,
                       uint32_t *d_match_intersect, uint32_t *d_match_remaining, void *stream);
+int kmerml_fmh_gather_abundance(kmerml_ctx *ctx, const uint64_t *d_q_hashes, const uint64_t *d_q_offsets, int n_q,
+                                const uint64_t *d_r_hashes, const uint64_t *d_r_offsets, int n_r, uint32_t threshold,
+                                int max_matches, int32_t *d_n_matches, int32_t *d_match_ref, uint32_t *d_match_unique,
+                                uint32_t *d_match_intersect, uint32_t *d_match_remaining,
+                                const uint32_t *d_q_abundances, uint64_t *d_match_unique_weighted,
+                                uint64_t *d_match_unique_sumsq, double *d_match_median_abund, void *stream);
 
 /*
  * Measurement hooks (bench.py): with profiling enabled every kernel the library

@@ -16,6 +16,7 @@ FLAG_FREQ_ON_DEVICE = 4
 FLAG_K8_AS_9 = 8
 FLAG_WIDE_D2H = 16
 FLAG_NO_NIBBLES = 32
+FLAG_FMH_ABUNDANCE = 64
 MAX_DENSE_K = 14
 MAX_K = 32
 SKETCH_MAX = 16384
@@ -26,6 +27,8 @@ FMH_MAX_CONTAINMENT = 1
 FMH_JACCARD = 2
 FMH_CONTAINMENT_ANI = 3
 FMH_MAX_CONTAINMENT_ANI = 4
+FMH_WEIGHTED_CONTAINMENT = 5
+FMH_ANGULAR_SIMILARITY = 6
 
 _lib = None
 
@@ -105,6 +108,10 @@ def load():
     L.kmerml_fmh_fetch.argtypes = [vp, vp, u64, vp, vp]
     L.kmerml_fmh_compare.argtypes = [vp, vp, vp, i32, vp, vp, i32, i32, i32, vp, vp, vp, vp]
     L.kmerml_fmh_gather.argtypes = [vp, vp, vp, i32, vp, vp, i32, u32, i32, vp, vp, vp, vp, vp, vp]
+    L.kmerml_fmh_fetch_abundances.argtypes = [vp, vp, u64, vp]
+    L.kmerml_fmh_compare_weighted.argtypes = [vp, vp, vp, vp, i32, vp, vp, vp, i32, i32, vp, vp, vp, vp]
+    L.kmerml_fmh_gather_abundance.argtypes = [vp, vp, vp, i32, vp, vp, i32, u32, i32, vp, vp, vp, vp, vp, vp, vp, vp, vp,
+                                              vp]
     L.kmerml_profile_enable.argtypes = [vp, i32]
     L.kmerml_profile_read.argtypes = [vp, ctypes.POINTER(Profile), i32]
     for name in EXPORTS:
@@ -129,6 +136,7 @@ EXPORTS = [
     "kmerml_emit_sparse_range", "kmerml_reduce_sparse_windows",
     "kmerml_sketch_batch", "kmerml_sketch_distance_rows",
     "kmerml_fmh_batch", "kmerml_fmh_fetch", "kmerml_fmh_compare", "kmerml_fmh_gather",
+    "kmerml_fmh_fetch_abundances", "kmerml_fmh_compare_weighted", "kmerml_fmh_gather_abundance",
 ]
 
 

@@ -118,7 +118,9 @@ struct kmerml_ctx {
     km::SparsePending sparse_pending;             // kmerml_count_sparse -> kmerml_sparse_fetch
     km::DevBuf fmh_kept;                          // kmerml_fmh_batch -> kmerml_fmh_fetch: the kept values of every round,
     km::DevBuf fmh_index;                         // where each genome's begin there | the CSR offsets
+    km::DevBuf fmh_abund;                         // KMERML_FLAG_FMH_ABUNDANCE: the abundances, parallel to fmh_kept
     int fmh_n = -1;                               // genomes of that result (< 0: none)
+    bool fmh_has_abund = false;                   // that result was made with KMERML_FLAG_FMH_ABUNDANCE
     uint64_t fmh_total = 0;
     km::HostPool* host_pool = nullptr;            // host threads that widen the narrow D2H format
     cudaStream_t last_stream = nullptr;           // ws[0] is scratch shared by every device-resident call: a call on
@@ -689,6 +691,7 @@ int kmerml_ctx_destroy(kmerml_ctx* ctx) {
     for (auto& w : ctx->ws) w.release();
     ctx->fmh_kept.release();
     ctx->fmh_index.release();
+    ctx->fmh_abund.release();
     if (ctx->order_ev) cudaEventDestroy(ctx->order_ev);
     if (ctx->host_pool) host_pool_destroy(ctx->host_pool);
     for (auto& r : ctx->recs) { cudaEventDestroy(r.a); cudaEventDestroy(r.b); }
@@ -1731,10 +1734,11 @@ static int grow_keeping(DevBuf& b, size_t used, size_t bytes, cudaStream_t s) {
 
 // Scaled sketches: the rounds of sketch_rounds with tau = T for every genome.  After each round the distinct values of
 // the genomes that did not overflow are appended to ctx->fmh_kept; at the end the CSR offsets and the gather into the
-// caller's buffer put them in genome order.
+// caller's buffer put them in genome order.  With `abundance` each kept value's run length in the sorted round is
+// appended to ctx->fmh_abund in the same places.
 static int fmh_batch_core(kmerml_ctx* ctx, const uint8_t* d_fasta, const uint64_t* h_offsets, int n, int k, int min_rec,
-                          bool canonical, uint64_t scale, uint64_t seed, uint64_t* d_hashes, uint64_t out_cap,
-                          uint64_t* d_offsets, uint64_t* h_total, cudaStream_t s) {
+                          bool canonical, bool abundance, uint64_t scale, uint64_t seed, uint64_t* d_hashes,
+                          uint64_t out_cap, uint64_t* d_offsets, uint64_t* h_total, cudaStream_t s) {
     const uint64_t T = ~0ull / scale;
     const auto too_large = [&](int g) {
         return fail(KMERML_ERR_RANGE, "genome " + std::to_string(g) + ": its k-mers at or below the threshold of scale " +
@@ -1746,6 +1750,7 @@ static int fmh_batch_core(kmerml_ctx* ctx, const uint8_t* d_fasta, const uint64_
         if (cap[g] > 0x7fffffffull) return too_large(g);
     }
     ctx->fmh_n = -1;
+    ctx->fmh_has_abund = false;
     uint64_t kept = 0;                                 // values in ctx->fmh_kept
     auto scratch = [](uint64_t slots, int n_active) {
         return 2 * align_up(std::max<uint64_t>(slots, 1) * 4, 256) + align_up(fmh_scan_temp_bytes((int)slots), 256) +
@@ -1782,9 +1787,13 @@ static int fmh_batch_core(kmerml_ctx* ctx, const uint8_t* d_fasta, const uint64_
         }
         if (!round_kept) return KMERML_OK;
         int rc = grow_keeping(ctx->fmh_kept, kept * 8, (kept + round_kept) * 8, s);
+        if (!rc && abundance) rc = grow_keeping(ctx->fmh_abund, kept * 4, (kept + round_kept) * 4, s);
         if (!rc) {
-            Prof pr(ctx, s, 3, 1);
+            Prof pr(ctx, s, 3, abundance ? 2 : 1);
             rc = launch_fmh_scatter(r.d_sorted, d_flags, d_pos, (int)r.slots, (uint64_t*)ctx->fmh_kept.p + kept, s);
+            if (!rc && abundance)
+                rc = launch_fmh_abundance(d_flags, d_pos, r.d_seg, r.n_active, (int)r.slots,
+                                          (uint32_t*)ctx->fmh_abund.p + kept, s);
         }
         kept += round_kept;
         return rc;
@@ -1801,6 +1810,7 @@ static int fmh_batch_core(kmerml_ctx* ctx, const uint8_t* d_fasta, const uint64_
     KM_CUDA(cudaMemcpyAsync(ctx->fmh_index.p, index.data(), index.size() * 8, cudaMemcpyHostToDevice, s));
     KM_CUDA(cudaStreamSynchronize(s));
     ctx->fmh_n = n;
+    ctx->fmh_has_abund = abundance;
     ctx->fmh_total = index[2 * (size_t)n];
     *h_total = ctx->fmh_total;
     KM_CUDA(cudaMemcpyAsync(d_offsets, (uint64_t*)ctx->fmh_index.p + n, (size_t)(n + 1) * 8, cudaMemcpyDeviceToDevice, s));
@@ -1868,8 +1878,9 @@ int kmerml_fmh_batch(kmerml_ctx* ctx, const uint8_t* d_fasta, const uint64_t* h_
     DeviceGuard guard(ctx->device);
     if (!guard.ok) return fail(KMERML_ERR_CUDA, "cudaSetDevice failed");
     if (int orc = order_stream(ctx, (cudaStream_t)stream)) return orc;
-    return fmh_batch_core(ctx, d_fasta, h_offsets, n_genomes, k, min_rec, (flags & KMERML_FLAG_CANONICAL) != 0, scale, seed,
-                          d_hashes, out_cap, d_sketch_offsets, h_total, (cudaStream_t)stream);
+    return fmh_batch_core(ctx, d_fasta, h_offsets, n_genomes, k, min_rec, (flags & KMERML_FLAG_CANONICAL) != 0,
+                          (flags & KMERML_FLAG_FMH_ABUNDANCE) != 0, scale, seed, d_hashes, out_cap, d_sketch_offsets,
+                          h_total, (cudaStream_t)stream);
 }
 
 int kmerml_fmh_fetch(kmerml_ctx* ctx, uint64_t* d_hashes, uint64_t out_cap, uint64_t* d_sketch_offsets, void* stream) {
@@ -1914,14 +1925,62 @@ int kmerml_fmh_compare(kmerml_ctx* ctx, const uint64_t* d_q_hashes, const uint64
                               inter, d_out32, d_out64, (cudaStream_t)stream);
 }
 
+int kmerml_fmh_fetch_abundances(kmerml_ctx* ctx, uint32_t* d_abundances, uint64_t out_cap, void* stream) {
+    if (!ctx || (out_cap && !d_abundances)) return fail(KMERML_ERR_ARG, "null pointer argument");
+    if (ctx->fmh_n < 0 || !ctx->fmh_has_abund)
+        return fail(KMERML_ERR_ARG, "no scaled-sketch result made with KMERML_FLAG_FMH_ABUNDANCE to fetch");
+    if (out_cap < ctx->fmh_total) return fail(KMERML_ERR_ARG, "out_cap is smaller than the total of the sketches");
+    DeviceGuard guard(ctx->device);
+    if (!guard.ok) return fail(KMERML_ERR_CUDA, "cudaSetDevice failed");
+    if (int orc = order_stream(ctx, (cudaStream_t)stream)) return orc;
+    cudaStream_t s = (cudaStream_t)stream;
+    const int n = ctx->fmh_n;
+    const uint64_t* index = (const uint64_t*)ctx->fmh_index.p;
+    ctx->launches += 1;
+    int rc = launch_fmh_gather((const uint32_t*)ctx->fmh_abund.p, index, index + n, n, ctx->fmh_total, d_abundances, s);
+    if (!rc) KM_CUDA(cudaStreamSynchronize(s));
+    return rc;
+}
+
+int kmerml_fmh_compare_weighted(kmerml_ctx* ctx, const uint64_t* d_q_hashes, const uint64_t* d_q_offsets,
+                                const uint32_t* d_q_abundances, int n_q, const uint64_t* d_r_hashes,
+                                const uint64_t* d_r_offsets, const uint32_t* d_r_abundances, int n_r, int metric,
+                                uint64_t* d_numerators, float* d_out32, double* d_out64, void* stream) {
+    if (!ctx) return fail(KMERML_ERR_ARG, "ctx is null");
+    if (metric != KMERML_FMH_WEIGHTED_CONTAINMENT && metric != KMERML_FMH_ANGULAR_SIMILARITY)
+        return fail(KMERML_ERR_ARG, "unknown weighted scaled-sketch metric");
+    if (n_q < 0 || n_r < 0) return fail(KMERML_ERR_ARG, "n_q and n_r must be >= 0");
+    if (!n_q || !n_r) return KMERML_OK;
+    if (!d_q_hashes || !d_q_offsets || !d_q_abundances || !d_r_hashes || !d_r_offsets ||
+        (metric == KMERML_FMH_ANGULAR_SIMILARITY && !d_r_abundances) || (!d_numerators && !d_out32 && !d_out64))
+        return fail(KMERML_ERR_ARG, "null pointer argument");
+    DeviceGuard guard(ctx->device);
+    if (!guard.ok) return fail(KMERML_ERR_CUDA, "cudaSetDevice failed");
+    Workspace& ws = ctx->ws[0];
+    if (int orc = order_stream(ctx, (cudaStream_t)stream)) return orc;
+    // workspace: the reference chunk table and the per-sketch sums | the numerators when the caller does not want them
+    const size_t table = align_up(fmh_compare_weighted_workspace(n_q, n_r), 256);
+    int rc = ws.misc.ensure(table + (d_numerators ? 0 : (size_t)n_q * n_r * 8));
+    if (rc) return rc;
+    unsigned long long* num = d_numerators ? (unsigned long long*)d_numerators
+                                           : (unsigned long long*)((uint8_t*)ws.misc.p + table);
+    ctx->launches += 2 + ((d_out32 || d_out64) ? (metric == KMERML_FMH_ANGULAR_SIMILARITY ? 3 : 2) : 0);
+    return launch_fmh_compare_weighted(d_q_hashes, d_q_offsets, d_q_abundances, n_q, d_r_hashes, d_r_offsets,
+                                       d_r_abundances, n_r, metric, ctx->sm_count, ws.misc.p, num, d_out32, d_out64,
+                                       (cudaStream_t)stream);
+}
+
 // Gather: x = |Q n R| for every pair (launch_fmh_compare), the candidate references (x >= threshold for some query)
 // copied into a compact CSR in reference order, then rounds in lockstep over every running query: select (with the
 // last round's subtraction fused), remove (the hashes the pick takes, as a sorted CSR S_t) and subtract
 // (launch_fmh_compare of S_t against the candidates).  The host reads the number of picks after each select and
-// stops when there were none or max_matches rounds have run.
+// stops when there were none or max_matches rounds have run.  With query abundances (d_qa; NULL for
+// kmerml_fmh_gather) the remove step also sums S_t's abundances and a segmented sort gives their median; it then runs
+// in the last round too, so the last recorded match gets its statistics.
 static int fmh_gather_core(kmerml_ctx* ctx, const uint64_t* d_qh, const uint64_t* d_q_off, int n_q, const uint64_t* d_rh,
                            const uint64_t* d_r_off, int n_r, uint32_t threshold, int max_matches, int32_t* d_n_matches,
-                           int32_t* d_ref, uint32_t* d_unique, uint32_t* d_inter, uint32_t* d_rem, cudaStream_t s) {
+                           int32_t* d_ref, uint32_t* d_unique, uint32_t* d_inter, uint32_t* d_rem, const uint32_t* d_qa,
+                           uint64_t* d_uw, uint64_t* d_usq, double* d_med, cudaStream_t s) {
     Workspace& ws = ctx->ws[0];
     KM_CUDA(cudaMemsetAsync(d_n_matches, 0, (size_t)n_q * 4, s));
     if (!n_r) {
@@ -1962,9 +2021,12 @@ static int fmh_gather_core(kmerml_ctx* ctx, const uint64_t* d_qh, const uint64_t
         index[n_c + c + 1] = index[n_c + c] + (r_off[cand[c] + 1] - r_off[cand[c]]);
     }
     const uint64_t c_total = index[2 * (size_t)n_c];
+    if (d_qa && q_total > 0x7fffffffull)
+        return fail(KMERML_ERR_RANGE, "fmh gather with abundances: more than 2^31 - 1 query hashes in one call");
 
     // ws.scratch: candidate hashes | index | candidate list | u | d | pick | remaining | s_len | s_off | scan temp |
     // assigned flags (one byte per query hash) | S_t (at most every query hash) | pick count, inconsistency flag
+    // [| with abundances: S_t's abundances | the same sorted | the sort's temp storage]
     size_t at = 0;
     auto take = [&](size_t bytes) { const size_t a = at; at += align_up(bytes, 256); return a; };
     const size_t uq = (size_t)n_q * n_c * 4;
@@ -1973,6 +2035,9 @@ static int fmh_gather_core(kmerml_ctx* ctx, const uint64_t* d_qh, const uint64_t
     const size_t at_u = take(uq), at_d = take(uq), at_pick = take((size_t)n_q * 4), at_remaining = take((size_t)n_q * 4);
     const size_t at_s_len = take((size_t)(n_q + 1) * 8), at_s_off = take((size_t)(n_q + 1) * 8), at_temp = take(temp_bytes);
     const size_t at_assigned = take(q_total), at_s = take(q_total * 8), at_cnt = take(8);
+    const size_t med_temp = d_qa ? align_up(fmh_greedy_median_temp_bytes(n_q, (int)q_total), 256) : 0;
+    const size_t at_sa = d_qa ? take(q_total * 4) : 0, at_ss = d_qa ? take(q_total * 4) : 0;
+    const size_t at_med_temp = d_qa ? take(med_temp) : 0;
     if ((rc = ws.scratch.ensure(at))) return rc;
     uint8_t* base = (uint8_t*)ws.scratch.p;
     uint64_t* d_ch = (uint64_t*)(base + at_ch);
@@ -2004,6 +2069,7 @@ static int fmh_gather_core(kmerml_ctx* ctx, const uint64_t* d_qh, const uint64_t
         Prof pr(ctx, s, 3, 1);
         if ((rc = launch_fmh_gather(d_rh, d_index, d_c_off, n_c, c_total, d_ch, s))) return rc;
     }
+    GatherAbund ab{d_qa, (uint32_t*)(base + at_sa), (unsigned long long*)d_uw, (unsigned long long*)d_usq, 0, max_matches};
     for (int round = 0; round < max_matches; round++) {
         KM_CUDA(cudaMemsetAsync(d_cnt, 0, 4, s));
         {
@@ -2017,12 +2083,24 @@ static int fmh_gather_core(kmerml_ctx* ctx, const uint64_t* d_qh, const uint64_t
         // the last round's remove assigned other counts than its select recorded: only unsorted or repeated input
         // values do that (a round always ends in a select, so every remove is checked)
         if (h_cnt[1]) return fail(KMERML_ERR_ARG, "fmh gather: the sketches must hold ascending, distinct values");
-        if (!h_cnt[0] || round + 1 == max_matches) break;
-        Prof pr(ctx, s, 3, 5);
+        const bool last = round + 1 == max_matches;
+        if (!h_cnt[0] || (last && !d_qa)) break;
+        Prof pr(ctx, s, 3, (d_qa ? 3 : 0) + (last ? 2 : 5));
+        ab.round = round;
         rc = launch_fmh_greedy_remove(d_qh, d_q_off, n_q, d_ch, d_c_off, d_pick, d_s_len, d_s_off, base + at_temp,
-                                      temp_bytes, d_assigned, d_s, d_cnt + 1, s);
-        if (!rc) rc = launch_fmh_compare(d_s, (const uint64_t*)d_s_off, n_q, d_ch, d_c_off, n_c, 1, KMERML_FMH_CONTAINMENT,
-                                         ctx->sm_count, d_table, d_d, nullptr, nullptr, s);
+                                      temp_bytes, d_assigned, d_s, d_cnt + 1, d_qa ? &ab : nullptr, s);
+        if (!rc && d_qa)
+            rc = launch_fmh_greedy_median(ab, d_s_off, d_pick, n_q, (int)q_total, (uint32_t*)(base + at_ss),
+                                          base + at_med_temp, med_temp, d_med, s);
+        if (rc) return rc;
+        if (last) {                                   // no select follows: check this remove here
+            KM_CUDA(cudaMemcpyAsync(h_cnt, d_cnt, 8, cudaMemcpyDeviceToHost, s));
+            KM_CUDA(cudaStreamSynchronize(s));
+            if (h_cnt[1]) return fail(KMERML_ERR_ARG, "fmh gather: the sketches must hold ascending, distinct values");
+            break;
+        }
+        rc = launch_fmh_compare(d_s, (const uint64_t*)d_s_off, n_q, d_ch, d_c_off, n_c, 1, KMERML_FMH_CONTAINMENT,
+                                ctx->sm_count, d_table, d_d, nullptr, nullptr, s);
         if (rc) return rc;
     }
     return KMERML_OK;
@@ -2044,8 +2122,31 @@ int kmerml_fmh_gather(kmerml_ctx* ctx, const uint64_t* d_q_hashes, const uint64_
     if (!guard.ok) return fail(KMERML_ERR_CUDA, "cudaSetDevice failed");
     if (int orc = order_stream(ctx, (cudaStream_t)stream)) return orc;
     return fmh_gather_core(ctx, d_q_hashes, d_q_offsets, n_q, d_r_hashes, d_r_offsets, n_r, threshold, max_matches,
-                           d_n_matches, d_match_ref, d_match_unique, d_match_intersect, d_match_remaining,
-                           (cudaStream_t)stream);
+                           d_n_matches, d_match_ref, d_match_unique, d_match_intersect, d_match_remaining, nullptr,
+                           nullptr, nullptr, nullptr, (cudaStream_t)stream);
+}
+
+int kmerml_fmh_gather_abundance(kmerml_ctx* ctx, const uint64_t* d_q_hashes, const uint64_t* d_q_offsets, int n_q,
+                                const uint64_t* d_r_hashes, const uint64_t* d_r_offsets, int n_r, uint32_t threshold,
+                                int max_matches, int32_t* d_n_matches, int32_t* d_match_ref, uint32_t* d_match_unique,
+                                uint32_t* d_match_intersect, uint32_t* d_match_remaining, const uint32_t* d_q_abundances,
+                                uint64_t* d_match_unique_weighted, uint64_t* d_match_unique_sumsq,
+                                double* d_match_median_abund, void* stream) {
+    if (!ctx) return fail(KMERML_ERR_ARG, "ctx is null");
+    if (threshold < 1) return fail(KMERML_ERR_ARG, "threshold must be >= 1");
+    if (max_matches < 1) return fail(KMERML_ERR_ARG, "max_matches must be >= 1");
+    if (n_q < 0 || n_r < 0) return fail(KMERML_ERR_ARG, "n_q and n_r must be >= 0");
+    if (!n_q) return KMERML_OK;
+    if (!d_q_offsets || !d_r_offsets || !d_n_matches || !d_match_ref || !d_match_unique || !d_match_intersect ||
+        !d_match_remaining || !d_q_abundances || !d_match_unique_weighted || !d_match_unique_sumsq ||
+        !d_match_median_abund)
+        return fail(KMERML_ERR_ARG, "null pointer argument");
+    DeviceGuard guard(ctx->device);
+    if (!guard.ok) return fail(KMERML_ERR_CUDA, "cudaSetDevice failed");
+    if (int orc = order_stream(ctx, (cudaStream_t)stream)) return orc;
+    return fmh_gather_core(ctx, d_q_hashes, d_q_offsets, n_q, d_r_hashes, d_r_offsets, n_r, threshold, max_matches,
+                           d_n_matches, d_match_ref, d_match_unique, d_match_intersect, d_match_remaining, d_q_abundances,
+                           d_match_unique_weighted, d_match_unique_sumsq, d_match_median_abund, (cudaStream_t)stream);
 }
 
 // NCCL through the process that called us (no link-time dependency): the four entry points the exchange needs.

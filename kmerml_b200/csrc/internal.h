@@ -221,12 +221,23 @@ int launch_fmh_distinct(const SketchGenome* d_sg, const int* d_active, int n_act
                         FmhRoundGenome* d_out, cudaStream_t s);
 int launch_fmh_scatter(const uint64_t* d_sorted, const uint32_t* d_flags, const uint32_t* d_pos, int n_items, uint64_t* d_out,
                        cudaStream_t s);
-int launch_fmh_gather(const uint64_t* d_kept, const uint64_t* d_begin, const uint64_t* d_offsets, int n, uint64_t total,
-                      uint64_t* d_out, cudaStream_t s);
+// the run length of every kept slot of a round (KMERML_FLAG_FMH_ABUNDANCE), at d_out[d_pos[slot]] like the scatter
+int launch_fmh_abundance(const uint32_t* d_flags, const uint32_t* d_pos, const int* d_seg, int n_active, int n_items,
+                         uint32_t* d_out, cudaStream_t s);
+// T = uint64_t (values) or uint32_t (abundances)
+template <typename T>
+int launch_fmh_gather(const T* d_kept, const uint64_t* d_begin, const uint64_t* d_offsets, int n, uint64_t total, T* d_out,
+                      cudaStream_t s);
 size_t fmh_compare_workspace(int n_r);
 int launch_fmh_compare(const uint64_t* d_qh, const uint64_t* d_q_off, int n_q, const uint64_t* d_rh, const uint64_t* d_r_off,
                        int n_r, int k, int metric, int sm_count, void* workspace, uint32_t* d_inter, float* d_out32,
                        double* d_out64, cudaStream_t s);
+// weighted metrics: d_num (n_q x n_r) = sum_{Q n R} a_Q (weighted containment) or a_Q a_R (angular similarity)
+size_t fmh_compare_weighted_workspace(int n_q, int n_r);
+int launch_fmh_compare_weighted(const uint64_t* d_qh, const uint64_t* d_q_off, const uint32_t* d_qa, int n_q,
+                                const uint64_t* d_rh, const uint64_t* d_r_off, const uint32_t* d_ra, int n_r, int metric,
+                                int sm_count, void* workspace, unsigned long long* d_num, float* d_out32, double* d_out64,
+                                cudaStream_t s);
 // gather: the candidate flags of a prefetched n_q x n_r intersection matrix (zeroed here) ...
 int launch_fmh_greedy_flag(const uint32_t* d_x, int n_q, int n_r, uint32_t threshold, uint8_t* d_flags, cudaStream_t s);
 // ... one round's pick of every running query (d_d: the last round's subtraction, unused in round 0) ...
@@ -235,12 +246,25 @@ int launch_fmh_greedy_select(uint32_t* d_u, const uint32_t* d_d, int n_c, const 
                              int* d_pick, uint32_t* d_remaining, unsigned long long* d_s_len, int32_t* d_n_matches,
                              int32_t* d_ref, uint32_t* d_unique, uint32_t* d_inter, uint32_t* d_rem,
                              unsigned int* d_n_picked, cudaStream_t s);
-// ... and the hashes each pick takes, as a sorted CSR (d_s_len, d_s_off: n_q + 1 words; d_s_len[n_q] = 0)
+// ... and the hashes each pick takes, as a sorted CSR (d_s_len, d_s_off: n_q + 1 words; d_s_len[n_q] = 0); with `ab`,
+// also their query abundances beside them (ab->s_abund) and the sum and sum of squares of those per recorded match
+struct GatherAbund {
+    const uint32_t* qa;               // query abundances, parallel to the query hashes
+    uint32_t* s_abund;                // S_t's abundances, parallel to S_t
+    unsigned long long* sum;          // per match slot q * max_matches + round
+    unsigned long long* sumsq;
+    int round, max_matches;
+};
 size_t fmh_greedy_scan_temp_bytes(int n_q);
 int launch_fmh_greedy_remove(const uint64_t* d_qh, const uint64_t* d_q_off, int n_q, const uint64_t* d_ch,
                              const uint64_t* d_c_off, const int* d_pick, const unsigned long long* d_s_len,
                              unsigned long long* d_s_off, void* temp, size_t temp_bytes, uint8_t* d_assigned,
-                             uint64_t* d_s_hashes, unsigned int* d_bad, cudaStream_t s);
+                             uint64_t* d_s_hashes, unsigned int* d_bad, const GatherAbund* ab, cudaStream_t s);
+// ... and the median of S_t's abundances of every query that recorded a match this round (total = |S_t| summed)
+size_t fmh_greedy_median_temp_bytes(int n_q, int total);
+int launch_fmh_greedy_median(const GatherAbund& ab, const unsigned long long* d_s_off, const int* d_pick, int n_q,
+                             int total, uint32_t* d_sorted, void* temp, size_t temp_bytes, double* d_median,
+                             cudaStream_t s);
 
 // ---- k{k}.txt text (format.cu) --------------------------------------------------
 size_t format_workspace_bytes(uint64_t n_bins, uint64_t max_lines);

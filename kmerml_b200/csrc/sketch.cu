@@ -27,6 +27,10 @@
 //   fmh_greedy_select_kernel  per query, the candidate with the most still-unassigned hashes (ties: smallest index)
 //   fmh_greedy_remove_kernel  per query, the hashes that pick takes: marked assigned and listed as a sorted CSR, which
 //                             fmh_intersect_kernel then subtracts from every candidate's count.
+// Abundances (KMERML_FLAG_FMH_ABUNDANCE): fmh_abundance_kernel writes each kept value's run length in the sorted round
+// beside it; fmh_intersect_kernel<true> + fmh_abund_sums_kernel + fmh_weighted_metric_kernel give weighted containment
+// and angular similarity; fmh_greedy_remove_kernel<true> sums S_t's query abundances, and a CUB segmented sort +
+// fmh_greedy_median_kernel give their median.
 #include <cub/cub.cuh>
 
 #include "sparse_walk.cuh"
@@ -287,9 +291,34 @@ __global__ void fmh_scatter_kernel(const uint64_t* __restrict__ sorted, const ui
     if (i < n_items && flags[i]) out[pos[i]] = sorted[i];
 }
 
-// out[offsets[g] + t] = kept[begin[g] + t] for t < offsets[g + 1] - offsets[g]: the kept values in genome order.
-__global__ void fmh_gather_kernel(const uint64_t* __restrict__ kept, const uint64_t* __restrict__ begin,
-                                  const uint64_t* __restrict__ offsets, int n, uint64_t total, uint64_t* out) {
+// Abundance of kept slot i (KMERML_FLAG_FMH_ABUNDANCE): the length of its run of equal sorted survivors, i.e. the next
+// kept slot of its segment (or the segment end) minus i, written beside the value fmh_scatter_kernel writes.  Kept slots
+// after i carry pos + flag > pos[i] + 1, so the run end is a binary search over the inclusive scan pos + flags.
+__global__ void fmh_abundance_kernel(const uint32_t* __restrict__ flags, const uint32_t* __restrict__ pos,
+                                     const int* __restrict__ seg_begin, const int* __restrict__ seg_end, int n_active,
+                                     int n_items, uint32_t* out) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n_items || !flags[i]) return;
+    int lo = 0, hi = n_active;
+    while (lo < hi) {
+        const int mid = (lo + hi) >> 1;
+        if (seg_begin[mid] <= i) lo = mid + 1; else hi = mid;
+    }
+    const int end = seg_end[lo - 1];
+    const uint32_t next = pos[i] + 1;
+    int a = i + 1, b = end;                           // the first slot in [i + 1, end) that is kept, else end
+    while (a < b) {
+        const int mid = (a + b) >> 1;
+        if (pos[mid] + flags[mid] > next) b = mid; else a = mid + 1;
+    }
+    out[pos[i]] = (uint32_t)(a - i);
+}
+
+// out[offsets[g] + t] = kept[begin[g] + t] for t < offsets[g + 1] - offsets[g]: the kept values (or their abundances)
+// in genome order.
+template <typename T>
+__global__ void fmh_gather_kernel(const T* __restrict__ kept, const uint64_t* __restrict__ begin,
+                                  const uint64_t* __restrict__ offsets, int n, uint64_t total, T* out) {
     for (uint64_t i = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x; i < total; i += (uint64_t)gridDim.x * blockDim.x) {
         int lo = 0, hi = n;                           // the last genome whose output begins at or before i
         while (lo < hi) {
@@ -332,14 +361,28 @@ int launch_fmh_scatter(const uint64_t* d_sorted, const uint32_t* d_flags, const 
     return KMERML_OK;
 }
 
-int launch_fmh_gather(const uint64_t* d_kept, const uint64_t* d_begin, const uint64_t* d_offsets, int n, uint64_t total,
-                      uint64_t* d_out, cudaStream_t s) {
-    if (!total) return KMERML_OK;
-    const uint64_t blocks = std::min<uint64_t>((total + 255) / 256, 1ull << 16);
-    fmh_gather_kernel<<<(unsigned)blocks, 256, 0, s>>>(d_kept, d_begin, d_offsets, n, total, d_out);
+int launch_fmh_abundance(const uint32_t* d_flags, const uint32_t* d_pos, const int* d_seg, int n_active, int n_items,
+                         uint32_t* d_out, cudaStream_t s) {
+    if (n_items <= 0) return KMERML_OK;
+    fmh_abundance_kernel<<<(n_items + 255) / 256, 256, 0, s>>>(d_flags, d_pos, d_seg, d_seg + n_active, n_active, n_items,
+                                                               d_out);
     KM_CUDA(cudaGetLastError());
     return KMERML_OK;
 }
+
+template <typename T>
+int launch_fmh_gather(const T* d_kept, const uint64_t* d_begin, const uint64_t* d_offsets, int n, uint64_t total, T* d_out,
+                      cudaStream_t s) {
+    if (!total) return KMERML_OK;
+    const uint64_t blocks = std::min<uint64_t>((total + 255) / 256, 1ull << 16);
+    fmh_gather_kernel<T><<<(unsigned)blocks, 256, 0, s>>>(d_kept, d_begin, d_offsets, n, total, d_out);
+    KM_CUDA(cudaGetLastError());
+    return KMERML_OK;
+}
+template int launch_fmh_gather<uint64_t>(const uint64_t*, const uint64_t*, const uint64_t*, int, uint64_t, uint64_t*,
+                                         cudaStream_t);
+template int launch_fmh_gather<uint32_t>(const uint32_t*, const uint64_t*, const uint64_t*, int, uint64_t, uint32_t*,
+                                         cudaStream_t);
 
 // ---- |Q n R| of two sets of scaled sketches ----------------------------------------------------------------------
 constexpr int FMH_THREADS = 256;
@@ -388,10 +431,16 @@ __device__ __forceinline__ uint64_t warp_lower_bound(const uint64_t* __restrict_
 // of its sketch inside [chunk min, chunk max] with two warp-wide searches in global memory, then looks up 32 values at
 // a time (index, then a binary search inside the bucket) and counts the hits with a ballot.  The chunks of a reference
 // split its values, so their partial counts add up to |Q n R| exactly (one atomic per query and chunk).
-__global__ void __launch_bounds__(FMH_THREADS)
+// WEIGHTED: a hit adds a_Q (ra NULL) or a_Q a_R instead of 1, in uint64 (the sums fit: see kmerml_fmh_compare_weighted);
+// a_R is read from global memory at the hit's chunk position.  Three CTAs share an SM (shared memory), which lets the
+// weighted instantiation keep its 64-bit sums in registers; the unweighted one keeps the register choice it had.
+template <bool WEIGHTED>
+__global__ void __launch_bounds__(FMH_THREADS, WEIGHTED ? 3 : 0)
 fmh_intersect_kernel(const uint64_t* __restrict__ qh, const uint64_t* __restrict__ q_off, int n_q,
                      const uint64_t* __restrict__ rh, const uint64_t* __restrict__ r_off, int n_r,
-                     const unsigned long long* __restrict__ prefix, uint32_t* inter) {
+                     const unsigned long long* __restrict__ prefix,
+                     std::conditional_t<WEIGHTED, unsigned long long, uint32_t>* inter,
+                     const uint32_t* __restrict__ qa, const uint32_t* __restrict__ ra) {
     extern __shared__ uint64_t s_r[];
     uint32_t* s_idx = (uint32_t*)(s_r + FMH_CHUNK);
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -429,6 +478,7 @@ fmh_intersect_kernel(const uint64_t* __restrict__ qh, const uint64_t* __restrict
             const uint64_t a = warp_lower_bound(Q, 0, nq, cmin, lane);
             const uint64_t e = cmax == ~0ull ? nq : warp_lower_bound(Q, a, nq, cmax + 1, lane);
             uint32_t hits = 0;
+            unsigned long long mass = 0;              // WEIGHTED: this lane's share of the weighted count
             for (uint64_t t0 = a; t0 < e; t0 += 32) {
                 const uint64_t t = t0 + lane;
                 bool found = false;
@@ -442,10 +492,18 @@ fmh_intersect_kernel(const uint64_t* __restrict__ qh, const uint64_t* __restrict
                         if (s_r[mid] < v) l = mid + 1; else h = mid;
                     }
                     found = l < h0 && s_r[l] == v;
+                    if constexpr (WEIGHTED) {
+                        if (found) mass += (unsigned long long)qa[q_off[q] + t] * (ra ? ra[c_lo + l] : 1u);
+                    }
                 }
-                hits += __popc(__ballot_sync(0xffffffffu, found));
+                if constexpr (!WEIGHTED) hits += __popc(__ballot_sync(0xffffffffu, found));
             }
-            if (lane == 0 && hits) atomicAdd(inter + (uint64_t)q * n_r + r, hits);
+            if constexpr (WEIGHTED) {
+                for (int o = 16; o; o >>= 1) mass += __shfl_xor_sync(0xffffffffu, mass, o);
+                if (lane == 0 && mass) atomicAdd(inter + (uint64_t)q * n_r + r, mass);
+            } else {
+                if (lane == 0 && hits) atomicAdd(inter + (uint64_t)q * n_r + r, hits);
+            }
         }
     }
 }
@@ -475,21 +533,113 @@ __global__ void fmh_metric_kernel(const uint32_t* __restrict__ inter, const uint
     }
 }
 
+// Per sketch (a warp each): sum[i] = sum of its abundances, sumsq[i] = sum of their squares (either may be NULL).
+__global__ void fmh_abund_sums_kernel(const uint32_t* __restrict__ abund, const uint64_t* __restrict__ off, int n,
+                                      unsigned long long* sum, unsigned long long* sumsq) {
+    const int lane = threadIdx.x & 31;
+    const uint64_t warps = (uint64_t)gridDim.x * (blockDim.x / 32);
+    for (uint64_t i = blockIdx.x * (uint64_t)(blockDim.x / 32) + threadIdx.x / 32; i < (uint64_t)n; i += warps) {
+        unsigned long long s1 = 0, s2 = 0;
+        for (uint64_t t = off[i] + lane; t < off[i + 1]; t += 32) {
+            const unsigned long long a = abund[t];
+            s1 += a;
+            s2 += a * a;
+        }
+        for (int o = 16; o; o >>= 1) {
+            s1 += __shfl_xor_sync(0xffffffffu, s1, o);
+            s2 += __shfl_xor_sync(0xffffffffu, s2, o);
+        }
+        if (lane == 0) {
+            if (sum) sum[i] = s1;
+            if (sumsq) sumsq[i] = s2;
+        }
+    }
+}
+
+// Weighted containment x / sum_Q a_Q, or angular similarity 1 - 2 acos(c) / pi with c = min(1, x / (sqrt(qn) sqrt(rn)))
+// (x = sum_{Q n R} a_Q a_R, qn and rn the squared norms); 0 when x = 0 or a denominator is 0.  c is 1 whenever
+// x^2 = qn rn in integers (Cauchy-Schwarz equality), so proportional abundance vectors give exactly 1 however the
+// square roots round.
+__global__ void fmh_weighted_metric_kernel(const unsigned long long* __restrict__ num, int n_q, int n_r, int metric,
+                                           const unsigned long long* __restrict__ q_den,
+                                           const unsigned long long* __restrict__ r_den, float* out32, double* out64) {
+    const uint64_t n = (uint64_t)n_q * n_r;
+    for (uint64_t i = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x; i < n; i += (uint64_t)gridDim.x * blockDim.x) {
+        const unsigned long long x = num[i], qd = q_den[i / n_r];
+        double d = 0.0;
+        if (x && qd) {
+            if (metric == KMERML_FMH_WEIGHTED_CONTAINMENT) {
+                d = (double)x / (double)qd;
+            } else {
+                const unsigned long long rd = r_den[i % n_r];
+                const bool one = x * x == qd * rd && __umul64hi(x, x) == __umul64hi(qd, rd);
+                const double c = one ? 1.0 : fmin(1.0, (double)x / (sqrt((double)qd) * sqrt((double)rd)));
+                d = 1.0 - 2.0 * acos(c) / 3.141592653589793;
+            }
+        }
+        if (out64) out64[i] = d;
+        if (out32) out32[i] = (float)d;
+    }
+}
+
 size_t fmh_compare_workspace(int n_r) { return (size_t)(n_r + 1) * 8; }
+
+template <bool WEIGHTED>
+static int launch_fmh_intersect(const uint64_t* d_qh, const uint64_t* d_q_off, int n_q, const uint64_t* d_rh,
+                                const uint64_t* d_r_off, int n_r, int sm_count, void* workspace,
+                                std::conditional_t<WEIGHTED, unsigned long long, uint32_t>* d_inter, const uint32_t* d_qa,
+                                const uint32_t* d_ra, cudaStream_t s) {
+    unsigned long long* prefix = (unsigned long long*)workspace;
+    KM_CUDA(cudaMemsetAsync(d_inter, 0, (size_t)n_q * n_r * sizeof(*d_inter), s));
+    fmh_chunk_prefix_kernel<<<1, SELECT_THREADS, 0, s>>>(d_r_off, n_r, prefix);
+    KM_CUDA(cudaGetLastError());
+    KM_CUDA(cudaFuncSetAttribute(fmh_intersect_kernel<WEIGHTED>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                 (int)FMH_SMEM));
+    // three CTAs fit an SM's shared memory; eight rounds of them let the CTAs of long items be balanced by the rest
+    fmh_intersect_kernel<WEIGHTED><<<sm_count * 3 * 8, FMH_THREADS, FMH_SMEM, s>>>(d_qh, d_q_off, n_q, d_rh, d_r_off, n_r,
+                                                                                prefix, d_inter, d_qa, d_ra);
+    KM_CUDA(cudaGetLastError());
+    return KMERML_OK;
+}
+
+size_t fmh_compare_weighted_workspace(int n_q, int n_r) {
+    return fmh_compare_workspace(n_r) + (size_t)(2 * n_q + n_r) * 8;
+}
+
+int launch_fmh_compare_weighted(const uint64_t* d_qh, const uint64_t* d_q_off, const uint32_t* d_qa, int n_q,
+                                const uint64_t* d_rh, const uint64_t* d_r_off, const uint32_t* d_ra, int n_r, int metric,
+                                int sm_count, void* workspace, unsigned long long* d_num, float* d_out32, double* d_out64,
+                                cudaStream_t s) {
+    if (n_q <= 0 || n_r <= 0) return KMERML_OK;
+    const bool angular = metric == KMERML_FMH_ANGULAR_SIMILARITY;
+    int rc = launch_fmh_intersect<true>(d_qh, d_q_off, n_q, d_rh, d_r_off, n_r, sm_count, workspace, d_num, d_qa,
+                                        angular ? d_ra : nullptr, s);
+    if (rc || (!d_out32 && !d_out64)) return rc;
+    // workspace: the chunk table | sum (weighted containment) or squared norm (angular) of each query | of each reference
+    unsigned long long* q_den = (unsigned long long*)workspace + (n_r + 1);
+    unsigned long long* r_den = q_den + n_q;
+    fmh_abund_sums_kernel<<<(unsigned)std::min<uint64_t>((n_q + 7) / 8, 1ull << 16), 256, 0, s>>>(
+        d_qa, d_q_off, n_q, angular ? nullptr : q_den, angular ? q_den : nullptr);
+    KM_CUDA(cudaGetLastError());
+    if (angular) {
+        fmh_abund_sums_kernel<<<(unsigned)std::min<uint64_t>((n_r + 7) / 8, 1ull << 16), 256, 0, s>>>(d_ra, d_r_off, n_r,
+                                                                                                  nullptr, r_den);
+        KM_CUDA(cudaGetLastError());
+    }
+    const uint64_t n = (uint64_t)n_q * n_r;
+    const uint64_t blocks = std::min<uint64_t>((n + 255) / 256, 1ull << 16);
+    fmh_weighted_metric_kernel<<<(unsigned)blocks, 256, 0, s>>>(d_num, n_q, n_r, metric, q_den, r_den, d_out32, d_out64);
+    KM_CUDA(cudaGetLastError());
+    return KMERML_OK;
+}
 
 int launch_fmh_compare(const uint64_t* d_qh, const uint64_t* d_q_off, int n_q, const uint64_t* d_rh, const uint64_t* d_r_off,
                        int n_r, int k, int metric, int sm_count, void* workspace, uint32_t* d_inter, float* d_out32,
                        double* d_out64, cudaStream_t s) {
     if (n_q <= 0 || n_r <= 0) return KMERML_OK;
-    unsigned long long* prefix = (unsigned long long*)workspace;
-    KM_CUDA(cudaMemsetAsync(d_inter, 0, (size_t)n_q * n_r * 4, s));
-    fmh_chunk_prefix_kernel<<<1, SELECT_THREADS, 0, s>>>(d_r_off, n_r, prefix);
-    KM_CUDA(cudaGetLastError());
-    KM_CUDA(cudaFuncSetAttribute(fmh_intersect_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)FMH_SMEM));
-    // three CTAs fit an SM's shared memory; eight rounds of them let the CTAs of long items be balanced by the rest
-    fmh_intersect_kernel<<<sm_count * 3 * 8, FMH_THREADS, FMH_SMEM, s>>>(d_qh, d_q_off, n_q, d_rh, d_r_off, n_r, prefix,
-                                                                      d_inter);
-    KM_CUDA(cudaGetLastError());
+    int rc = launch_fmh_intersect<false>(d_qh, d_q_off, n_q, d_rh, d_r_off, n_r, sm_count, workspace, d_inter, nullptr,
+                                         nullptr, s);
+    if (rc) return rc;
     if (d_out32 || d_out64) {
         const uint64_t n = (uint64_t)n_q * n_r;
         const uint64_t blocks = std::min<uint64_t>((n + 255) / 256, 1ull << 16);
@@ -556,12 +706,14 @@ fmh_greedy_select_kernel(uint32_t* u, const uint32_t* __restrict__ d, int n_c, c
 
 // S_t of every query that picked candidate c this round: the values of R_c found in Q and not yet assigned, marked
 // assigned and written ascending (R_c's order) at s_off[q].  One CTA per query; each value of R_c is a binary search
-// in Q.  A count that differs from the select step's u sets *bad.
+// in Q.  A count that differs from the select step's u sets *bad.  ABUND: also the query abundances of S_t, written
+// beside it, and their sum and sum of squares in slot q * max_matches + round of ab.sum / ab.sumsq.
+template <bool ABUND>
 __global__ void __launch_bounds__(REMOVE_THREADS)
 fmh_greedy_remove_kernel(const uint64_t* __restrict__ qh, const uint64_t* __restrict__ q_off,
                          const uint64_t* __restrict__ ch, const uint64_t* __restrict__ c_off, const int* __restrict__ pick,
                          const unsigned long long* __restrict__ s_off, uint8_t* assigned, uint64_t* s_hashes,
-                         unsigned int* bad) {
+                         unsigned int* bad, GatherAbund ab) {
     using Scan = cub::BlockScan<int, REMOVE_THREADS>;
     __shared__ typename Scan::TempStorage tmp;
     const int q = blockIdx.x;
@@ -574,10 +726,12 @@ fmh_greedy_remove_kernel(const uint64_t* __restrict__ qh, const uint64_t* __rest
     const uint64_t nr = c_off[c + 1] - c_off[c];
     uint64_t* out = s_hashes + s_off[q];
     uint64_t written = 0;
+    unsigned long long sum = 0, sumsq = 0;            // ABUND: this thread's share
     for (uint64_t base = 0; base < nr; base += REMOVE_THREADS) {
         const uint64_t i = base + threadIdx.x;
         int take = 0;
         uint64_t v = 0;
+        uint32_t a = 0;
         if (i < nr) {
             v = R[i];
             uint64_t lo = 0, hi = nq;
@@ -588,15 +742,46 @@ fmh_greedy_remove_kernel(const uint64_t* __restrict__ qh, const uint64_t* __rest
             if (lo < nq && Q[lo] == v && !taken[lo]) {
                 taken[lo] = 1;
                 take = 1;
+                if constexpr (ABUND) {
+                    a = ab.qa[q_off[q] + lo];
+                    sum += a;
+                    sumsq += (unsigned long long)a * a;
+                }
             }
         }
         int pos, total;
         Scan(tmp).ExclusiveSum(take, pos, total);
-        if (take) out[written + pos] = v;
+        if (take) {
+            out[written + pos] = v;
+            if constexpr (ABUND) ab.s_abund[s_off[q] + written + pos] = a;
+        }
         written += total;
         __syncthreads();
     }
     if (threadIdx.x == 0 && written != s_off[q + 1] - s_off[q]) atomicOr(bad, 1u);
+    if constexpr (ABUND) {
+        using Reduce = cub::BlockReduce<unsigned long long, REMOVE_THREADS>;
+        __shared__ typename Reduce::TempStorage rtmp;
+        sum = Reduce(rtmp).Sum(sum);
+        __syncthreads();
+        sumsq = Reduce(rtmp).Sum(sumsq);
+        if (threadIdx.x == 0) {
+            const uint64_t slot = (uint64_t)q * ab.max_matches + ab.round;
+            ab.sum[slot] = sum;
+            ab.sumsq[slot] = sumsq;
+        }
+    }
+}
+
+// The median of the abundances of S_t (sorted per query), for every query that recorded a match this round: the middle
+// value, or the mean of the two middle values (exact in float64).
+__global__ void fmh_greedy_median_kernel(const uint32_t* __restrict__ sorted, const unsigned long long* __restrict__ s_off,
+                                         const int* __restrict__ pick, int n_q, int round, int max_matches, double* median) {
+    const int q = blockIdx.x * blockDim.x + threadIdx.x;
+    if (q >= n_q || pick[q] < 0) return;
+    const uint32_t* a = sorted + s_off[q];
+    const uint64_t n = s_off[q + 1] - s_off[q];
+    median[(uint64_t)q * max_matches + round] = n & 1 ? (double)a[n / 2] : ((double)a[n / 2 - 1] + (double)a[n / 2]) / 2.0;
 }
 
 int launch_fmh_greedy_flag(const uint32_t* d_x, int n_q, int n_r, uint32_t threshold, uint8_t* d_flags, cudaStream_t s) {
@@ -629,11 +814,34 @@ size_t fmh_greedy_scan_temp_bytes(int n_q) {
 int launch_fmh_greedy_remove(const uint64_t* d_qh, const uint64_t* d_q_off, int n_q, const uint64_t* d_ch,
                              const uint64_t* d_c_off, const int* d_pick, const unsigned long long* d_s_len,
                              unsigned long long* d_s_off, void* temp, size_t temp_bytes, uint8_t* d_assigned,
-                             uint64_t* d_s_hashes, unsigned int* d_bad, cudaStream_t s) {
+                             uint64_t* d_s_hashes, unsigned int* d_bad, const GatherAbund* ab, cudaStream_t s) {
     size_t tb = temp_bytes;
     KM_CUDA(cub::DeviceScan::ExclusiveSum(temp, tb, d_s_len, d_s_off, n_q + 1, s));
-    fmh_greedy_remove_kernel<<<n_q, REMOVE_THREADS, 0, s>>>(d_qh, d_q_off, d_ch, d_c_off, d_pick, d_s_off, d_assigned,
-                                                           d_s_hashes, d_bad);
+    if (ab)
+        fmh_greedy_remove_kernel<true><<<n_q, REMOVE_THREADS, 0, s>>>(d_qh, d_q_off, d_ch, d_c_off, d_pick, d_s_off,
+                                                                      d_assigned, d_s_hashes, d_bad, *ab);
+    else
+        fmh_greedy_remove_kernel<false><<<n_q, REMOVE_THREADS, 0, s>>>(d_qh, d_q_off, d_ch, d_c_off, d_pick, d_s_off,
+                                                                       d_assigned, d_s_hashes, d_bad, GatherAbund{});
+    KM_CUDA(cudaGetLastError());
+    return KMERML_OK;
+}
+
+size_t fmh_greedy_median_temp_bytes(int n_q, int total) {
+    size_t t = 0;
+    cub::DeviceSegmentedSort::SortKeys(nullptr, t, (const uint32_t*)nullptr, (uint32_t*)nullptr, total, n_q,
+                                       (const unsigned long long*)nullptr, (const unsigned long long*)nullptr);
+    return t;
+}
+
+int launch_fmh_greedy_median(const GatherAbund& ab, const unsigned long long* d_s_off, const int* d_pick, int n_q,
+                             int total, uint32_t* d_sorted, void* temp, size_t temp_bytes, double* d_median,
+                             cudaStream_t s) {
+    size_t tb = temp_bytes;
+    KM_CUDA(cub::DeviceSegmentedSort::SortKeys(temp, tb, (const uint32_t*)ab.s_abund, d_sorted, total, n_q, d_s_off,
+                                               d_s_off + 1, s));
+    fmh_greedy_median_kernel<<<(n_q + 255) / 256, 256, 0, s>>>(d_sorted, d_s_off, d_pick, n_q, ab.round, ab.max_matches,
+                                                               d_median);
     KM_CUDA(cudaGetLastError());
     return KMERML_OK;
 }

@@ -6,6 +6,7 @@ frequency rows the reference only gestures at (tests/test_ml.py:8).
 """
 import ctypes
 from dataclasses import dataclass
+from typing import Optional
 
 import numpy as np
 import torch
@@ -689,13 +690,15 @@ def concat_sketches(*sketches):
 @dataclass
 class ScaledSketches:
     """Scaled (FracMinHash) sketches of a batch of genomes (kmerml_fmh_batch): genome g's sketch is
-    hashes[offsets[g]:offsets[g + 1]], every distinct hash <= (2^64 - 1) // scale of its k-mers, ascending."""
+    hashes[offsets[g]:offsets[g + 1]], every distinct hash <= (2^64 - 1) // scale of its k-mers, ascending.  With
+    abundance tracking, abundances[i] is the number of windows of that genome whose k-mer hashes to hashes[i]."""
     hashes: torch.Tensor      # [total] int64 storage of uint64
     offsets: torch.Tensor     # [n + 1] int64
     k: int
     scale: int
     seed: int
     canonical: bool
+    abundances: Optional[torch.Tensor] = None     # [total] int32, or None
 
     def __len__(self):
         return self.offsets.shape[0] - 1
@@ -711,12 +714,16 @@ class ScaledSketches:
 _FMH_METRIC = {"containment": _lib.FMH_CONTAINMENT, "max_containment": _lib.FMH_MAX_CONTAINMENT,
                "jaccard": _lib.FMH_JACCARD, "containment_ani": _lib.FMH_CONTAINMENT_ANI,
                "max_containment_ani": _lib.FMH_MAX_CONTAINMENT_ANI}
+_FMH_WEIGHTED_METRIC = {"weighted_containment": _lib.FMH_WEIGHTED_CONTAINMENT,
+                        "angular_similarity": _lib.FMH_ANGULAR_SIMILARITY}
 
 
-def fmh_batch_device(fasta, offsets, k, *, scale=1000, seed=42, canonical=True, min_record_len=None):
+def fmh_batch_device(fasta, offsets, k, *, scale=1000, seed=42, canonical=True, min_record_len=None,
+                     track_abundance=False):
     """Scaled sketches of genomes already resident in HBM (laid out as for count_dense_device), any k <= 32.  The
     output is sized from a guess (1.25 hashes per `scale` bytes, + 256 per genome); a batch with more hashes than that
-    is copied out of the library's workspace once its size is known (kmerml_fmh_fetch), never sketched twice."""
+    is copied out of the library's workspace once its size is known (kmerml_fmh_fetch), never sketched twice.  With
+    track_abundance, also the abundance of every hash (kmerml_fmh_fetch_abundances)."""
     if not (fasta.is_cuda and fasta.dtype == torch.uint8 and fasta.is_contiguous()):
         raise ValueError("fasta must be a contiguous uint8 CUDA tensor")
     ctx = _lib.context(fasta.device.index)
@@ -731,12 +738,17 @@ def fmh_batch_device(fasta, offsets, k, *, scale=1000, seed=42, canonical=True, 
     stream = ctypes.c_void_p(torch.cuda.current_stream(fasta.device).cuda_stream)
     _retry_after_cache_release(lambda: _lib.check(L.kmerml_fmh_batch(
         ctx.handle, fasta.data_ptr() if fasta.numel() else None, offs.ctypes.data, n, int(k), int(min_record_len or 0),
-        _lib.FLAG_CANONICAL if canonical else 0, scale, int(seed) & 0xFFFFFFFFFFFFFFFF, hashes.data_ptr(), guess,
-        sk_offsets.data_ptr(), ctypes.byref(total), stream)))
+        (_lib.FLAG_CANONICAL if canonical else 0) | (_lib.FLAG_FMH_ABUNDANCE if track_abundance else 0), scale,
+        int(seed) & 0xFFFFFFFFFFFFFFFF, hashes.data_ptr(), guess, sk_offsets.data_ptr(), ctypes.byref(total), stream)))
     if total.value > guess:
         hashes = torch.empty(int(total.value), dtype=torch.int64, device=fasta.device)
         _lib.check(L.kmerml_fmh_fetch(ctx.handle, hashes.data_ptr(), total.value, sk_offsets.data_ptr(), stream))
-    return ScaledSketches(hashes[:int(total.value)], sk_offsets, int(k), scale, int(seed), bool(canonical))
+    abundances = None
+    if track_abundance:
+        abundances = torch.empty(max(int(total.value), 1), dtype=torch.int32, device=fasta.device)
+        _lib.check(L.kmerml_fmh_fetch_abundances(ctx.handle, abundances.data_ptr(), total.value, stream))
+        abundances = abundances[:int(total.value)]
+    return ScaledSketches(hashes[:int(total.value)], sk_offsets, int(k), scale, int(seed), bool(canonical), abundances)
 
 
 def fmh_compare_device(queries, references=None, metric="containment", *, out_dtype=torch.float32,
@@ -744,15 +756,21 @@ def fmh_compare_device(queries, references=None, metric="containment", *, out_dt
     """[n_q, n_r] similarity of every query sketch to every reference sketch (the queries themselves when
     `references` is None): "containment" |Q n R| / |Q|, "max_containment" |Q n R| / min(|Q|, |R|), "jaccard",
     "containment_ani" and "max_containment_ani" (the containment to the power 1/k); 0 when |Q n R| = 0.
-    With want_intersections, also the exact [n_q, n_r] int64 |Q n R|."""
-    if metric not in _FMH_METRIC:
-        raise ValueError(f"metric must be one of {sorted(_FMH_METRIC)}")
+    With want_intersections, also the exact [n_q, n_r] int64 |Q n R|.
+    Sketches with abundances (track_abundance) also give "weighted_containment", sum_{Q n R} a_Q / sum_Q a_Q (the
+    share of the query's k-mer mass that R explains; needs the query abundances), and "angular_similarity",
+    1 - 2 acos(cos) / pi of the abundance vectors (needs both); want_intersections then returns the exact integer
+    numerators sum_{Q n R} a_Q and sum_{Q n R} a_Q a_R instead of |Q n R|."""
+    if metric not in _FMH_METRIC and metric not in _FMH_WEIGHTED_METRIC:
+        raise ValueError(f"metric must be one of {sorted(_FMH_METRIC) + sorted(_FMH_WEIGHTED_METRIC)}")
     if out_dtype not in (torch.float32, torch.float64):
         raise ValueError("out_dtype must be torch.float32 or torch.float64")
     refs = queries if references is None else references
     if not (isinstance(queries, ScaledSketches) and isinstance(refs, ScaledSketches)):
         raise ValueError("queries and references must be ScaledSketches")
     _check_sketches(queries, refs)
+    if metric in _FMH_WEIGHTED_METRIC:
+        return _fmh_compare_weighted(queries, refs, metric, out_dtype, want_intersections)
     dev = queries.hashes.device
     n_q, n_r = len(queries), len(refs)
     out = torch.empty((n_q, n_r), dtype=out_dtype, device=dev)
@@ -770,6 +788,28 @@ def fmh_compare_device(queries, references=None, metric="containment", *, out_dt
     return out
 
 
+def _fmh_compare_weighted(queries, refs, metric, out_dtype, want_numerators):
+    if queries.abundances is None or (metric == "angular_similarity" and refs.abundances is None):
+        raise ValueError(f"{metric} needs sketches made with track_abundance=True "
+                         f"({'queries' if metric == 'weighted_containment' else 'queries and references'})")
+    dev = queries.hashes.device
+    n_q, n_r = len(queries), len(refs)
+    out = torch.empty((n_q, n_r), dtype=out_dtype, device=dev)
+    num = torch.empty((n_q, n_r), dtype=torch.int64, device=dev) if want_numerators else None
+    if out.numel():
+        ctx = _lib.context(dev.index)
+        stream = torch.cuda.current_stream(dev).cuda_stream
+        _lib.check(_lib.load().kmerml_fmh_compare_weighted(
+            ctx.handle, queries.hashes.data_ptr(), queries.offsets.data_ptr(), queries.abundances.data_ptr(), n_q,
+            refs.hashes.data_ptr(), refs.offsets.data_ptr(),
+            refs.abundances.data_ptr() if refs.abundances is not None else None, n_r, _FMH_WEIGHTED_METRIC[metric],
+            num.data_ptr() if num is not None else None, out.data_ptr() if out_dtype == torch.float32 else None,
+            out.data_ptr() if out_dtype == torch.float64 else None, ctypes.c_void_p(stream)))
+    if want_numerators:
+        return out, num
+    return out
+
+
 @dataclass
 class GatherResult:
     """Gather of each query sketch into the reference sketches that cover it (kmerml_fmh_gather): row q lists its
@@ -779,12 +819,18 @@ class GatherResult:
     unique: torch.Tensor      # [n_q, m] int64: query hashes first assigned to that reference
     intersect: torch.Tensor   # [n_q, m] int64: |Q n R| of the whole query
     remaining: torch.Tensor   # [n_q, m] int64: query hashes still unassigned after the match
+    # queries with abundances only (else None): over the hashes the match takes,
+    unique_weighted: Optional[torch.Tensor] = None    # [n_q, m] int64: the sum of their query abundances
+    unique_sumsq: Optional[torch.Tensor] = None       # [n_q, m] int64: the sum of their squares
+    median_abund: Optional[torch.Tensor] = None       # [n_q, m] float64: their median
 
 
 def fmh_gather_device(queries, references, *, threshold=1, max_matches=None):
     """Greedy, exact gather of every query into the references: repeatedly pick the reference that shares the most
     still-unassigned query hashes (ties: the smallest reference index) while that number is >= `threshold`, and
-    assign those hashes to it.  The default `max_matches`, min(n_r, max_q |Q| // threshold), never truncates."""
+    assign those hashes to it.  The default `max_matches`, min(n_r, max_q |Q| // threshold), never truncates.  When
+    the queries carry abundances, the picks are the same and each match also gets the sum, sum of squares and median
+    of the query abundances of the hashes it takes (kmerml_fmh_gather_abundance)."""
     if not (isinstance(queries, ScaledSketches) and isinstance(references, ScaledSketches)):
         raise ValueError("queries and references must be ScaledSketches")
     _check_sketches(queries, references)
@@ -803,24 +849,42 @@ def fmh_gather_device(queries, references, *, threshold=1, max_matches=None):
     m = max(max_matches, 1)
     ref = torch.full((n_q, m), -1, dtype=torch.int32, device=dev)
     counts = torch.zeros((3, n_q, m), dtype=torch.int32, device=dev)       # uint32 unique | intersect | remaining
+    weighted = queries.abundances is not None
+    if weighted:
+        sums = torch.zeros((2, n_q, m), dtype=torch.int64, device=dev)     # uint64 (< 2^63) unique_weighted | sumsq
+        median = torch.zeros((n_q, m), dtype=torch.float64, device=dev)
     if n_q and max_matches:
         ctx = _lib.context(dev.index)
         stream = ctypes.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
-        _retry_after_cache_release(lambda: _lib.check(_lib.load().kmerml_fmh_gather(
-            ctx.handle, queries.hashes.data_ptr(), queries.offsets.data_ptr(), n_q, references.hashes.data_ptr(),
-            references.offsets.data_ptr(), n_r, threshold, m, n_matches.data_ptr(), ref.data_ptr(),
-            counts[0].data_ptr(), counts[1].data_ptr(), counts[2].data_ptr(), stream)))
+        args = (ctx.handle, queries.hashes.data_ptr(), queries.offsets.data_ptr(), n_q, references.hashes.data_ptr(),
+                references.offsets.data_ptr(), n_r, threshold, m, n_matches.data_ptr(), ref.data_ptr(),
+                counts[0].data_ptr(), counts[1].data_ptr(), counts[2].data_ptr())
+        if weighted:
+            _retry_after_cache_release(lambda: _lib.check(_lib.load().kmerml_fmh_gather_abundance(
+                *args, queries.abundances.data_ptr(), sums[0].data_ptr(), sums[1].data_ptr(), median.data_ptr(),
+                stream)))
+        else:
+            _retry_after_cache_release(lambda: _lib.check(_lib.load().kmerml_fmh_gather(*args, stream)))
     wide = (counts[:, :, :max_matches].to(torch.int64) & 0xFFFFFFFF)
-    return GatherResult(n_matches, ref[:, :max_matches], wide[0], wide[1], wide[2])
+    res = GatherResult(n_matches, ref[:, :max_matches], wide[0], wide[1], wide[2])
+    if weighted:
+        res.unique_weighted, res.unique_sumsq = sums[0, :, :max_matches], sums[1, :, :max_matches]
+        res.median_abund = median[:, :max_matches]
+    return res
 
 
 def concat_scaled_sketches(*sketches):
-    """One ScaledSketches of several batches (same k, scale, seed and canonical flag), genomes in argument order."""
+    """One ScaledSketches of several batches (same k, scale, seed and canonical flag), genomes in argument order.
+    Abundances are kept when every batch has them; a mix of batches with and without them raises ValueError."""
     _check_sketches(*sketches)
+    has = [sk.abundances is not None for sk in sketches]
+    if any(has) and not all(has):
+        raise ValueError("some sketches carry abundances and some do not")
     first = sketches[0]
     offs, base = [first.offsets[:1]], 0
     for sk in sketches:
         offs.append(sk.offsets[1:] + base)
         base += int(sk.offsets[-1])
+    abundances = torch.cat([sk.abundances for sk in sketches]) if all(has) else None
     return ScaledSketches(torch.cat([sk.hashes for sk in sketches]), torch.cat(offs), first.k, first.scale, first.seed,
-                          first.canonical)
+                          first.canonical, abundances)

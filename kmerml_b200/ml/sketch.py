@@ -45,7 +45,9 @@ def containment_matrix(query_paths, reference_paths=None, *, k=21, scale=1000, s
     """DataFrame of a similarity of every query genome to every reference genome (one FASTA file each) from scaled
     sketches: index = query ids, columns = reference ids (file stems unless given).  Without `reference_paths` the
     queries are compared with each other.  `metric` is one of engine.fmh_compare_device's; all are similarities, so
-    with "max_containment_ani" (symmetric) `1 - df` goes straight into `hierarchical_clustering(..., distances=...)`."""
+    with "max_containment_ani" or "angular_similarity" (symmetric) `1 - df` goes straight into
+    `hierarchical_clustering(..., distances=...)`.  The abundance-weighted metrics ("weighted_containment",
+    "angular_similarity") sketch with abundance tracking."""
     q_paths = [Path(p) for p in query_paths]
     r_paths = q_paths if reference_paths is None else [Path(p) for p in reference_paths]
     q_ids = [p.stem for p in q_paths] if query_ids is None else list(query_ids)
@@ -56,7 +58,8 @@ def containment_matrix(query_paths, reference_paths=None, *, k=21, scale=1000, s
     if len(q_ids) != len(q_paths) or len(r_ids) != len(r_paths):
         raise ValueError("Number of ids must match number of genome paths")
     dev = torch.device(device if device is not None else "cuda")
-    params = dict(scale=scale, seed=seed, canonical=canonical)
+    params = dict(scale=scale, seed=seed, canonical=canonical,
+                  track_abundance=metric in ("weighted_containment", "angular_similarity"))
     queries = engine.fmh_batch_device(*_load_batch(q_paths, dev), k, **params)
     refs = None if reference_paths is None else engine.fmh_batch_device(*_load_batch(r_paths, dev), k, **params)
     d = engine.fmh_compare_device(queries, refs, metric, out_dtype=torch.float64).cpu().numpy()
@@ -71,19 +74,22 @@ def _ids(paths, ids):
 
 
 def gather(query_paths, reference_paths, *, k=21, scale=1000, seed=42, canonical=True, threshold_bp=50_000,
-           query_ids=None, reference_ids=None, device=None):
+           query_ids=None, reference_ids=None, device=None, track_abundance=False):
     """Long DataFrame of the gather of every query genome into the reference genomes (one FASTA file each; ids are
     the file stems unless given): one row per (query, match) in pick order.  A reference is picked while it covers at
     least max(1, ceil(threshold_bp / scale)) still-unassigned query hashes.  Columns: query, rank (0-based), match,
     intersect_bp / unique_bp / remaining_bp (hash counts times `scale`), f_orig_query = intersect / |Q|,
     f_match = intersect / |R|, f_unique_to_query = unique / |Q| and match_containment_ani = (intersect / |R|)^(1/k),
-    all in float64."""
+    all in float64.  With track_abundance the queries are sketched with k-mer abundances and, over the hashes each
+    match takes, the columns n_unique_weighted_found (the sum of their abundances), f_unique_weighted (that over the
+    query's total abundance: the match's share of the query's k-mers, e.g. of a metagenome's reads),
+    average_abund, median_abund and std_abund (population standard deviation) are added."""
     q_paths = [Path(p) for p in query_paths]
     r_paths = [Path(p) for p in reference_paths]
     q_ids, r_ids = _ids(q_paths, query_ids), _ids(r_paths, reference_ids)
     dev = torch.device(device if device is not None else "cuda")
     params = dict(scale=scale, seed=seed, canonical=canonical)
-    queries = engine.fmh_batch_device(*_load_batch(q_paths, dev), k, **params)
+    queries = engine.fmh_batch_device(*_load_batch(q_paths, dev), k, track_abundance=track_abundance, **params)
     refs = engine.fmh_batch_device(*_load_batch(r_paths, dev), k, **params)
     threshold = max(1, -(-int(threshold_bp) // int(scale)))
     res = engine.fmh_gather_device(queries, refs, threshold=threshold)
@@ -95,8 +101,21 @@ def gather(query_paths, reference_paths, *, k=21, scale=1000, seed=42, canonical
                                 for x in (res.unique, res.intersect, res.remaining))
     q_size = queries.sizes().cpu().numpy().astype(np.float64)[q_of]
     r_size = refs.sizes().cpu().numpy().astype(np.float64)[ref]
-    return pd.DataFrame({
+    df = pd.DataFrame({
         "query": [q_ids[i] for i in q_of], "rank": rank.astype(np.int64), "match": [r_ids[i] for i in ref],
         "intersect_bp": inter * scale, "unique_bp": unique * scale, "remaining_bp": remaining * scale,
         "f_orig_query": inter / q_size, "f_match": inter / r_size, "f_unique_to_query": unique / q_size,
         "match_containment_ani": (inter / r_size) ** (1.0 / k)})
+    if track_abundance:
+        weighted = res.unique_weighted.cpu().numpy()[q_of, rank]
+        sumsq = res.unique_sumsq.cpu().numpy()[q_of, rank].astype(np.float64)
+        q_mass = torch.zeros(len(queries), dtype=torch.int64, device=dev).index_add_(
+            0, torch.repeat_interleave(torch.arange(len(queries), device=dev), queries.sizes()),
+            queries.abundances.to(torch.int64)).cpu().numpy().astype(np.float64)[q_of]
+        avg = weighted / unique
+        df["n_unique_weighted_found"] = weighted.astype(np.int64)
+        df["f_unique_weighted"] = weighted / q_mass
+        df["average_abund"] = avg
+        df["median_abund"] = res.median_abund.cpu().numpy()[q_of, rank]
+        df["std_abund"] = np.sqrt(np.maximum(sumsq / unique - avg * avg, 0.0))
+    return df
